@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- luma Mpixel/s of the QVRCNN int8 pass (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--kernel auto|fused|layered]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--kernel auto|fused|layered] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic luma: BASELINE config 3,
 QP=32, 64 frames of 1920x1080 per GPU (weak scaling: every rank processes its own 64 frames,
@@ -296,6 +296,22 @@ def run_config5(torch, dist, api, rank, world, local, steps=20, warmup=3):
     return block
 
 
+DUMP_SEED, DUMP_FRAMES, DUMP_PIXELS = 20261020, 4, 1 << 22
+
+
+def dump_outputs(out_dir: str, d_out) -> None:
+    """What the timed step hands its caller, the reconstructed luma d_out (uint8 [FRAMES, H, W], 133 MB), as float32 .npy
+    files of 50 MB: recon_frames.npy = DUMP_FRAMES whole frames, recon_pixels.npy = DUMP_PIXELS pixels over the whole batch.
+    Which frames and pixels depends on DUMP_SEED alone, so two builds of the project can be compared file for file."""
+    import torch
+    rng = np.random.default_rng(DUMP_SEED)
+    frames = np.sort(rng.choice(FRAMES, DUMP_FRAMES, replace=False))
+    pixels = np.sort(rng.integers(0, FRAMES * H * W, DUMP_PIXELS))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "recon_frames.npy"), d_out[torch.from_numpy(frames).cuda()].cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "recon_pixels.npy"), d_out.view(-1)[torch.from_numpy(pixels).cuda()].cpu().numpy().astype(np.float32))
+
+
 REF_BIN = os.path.join(ROOT, "oracle", "_ref", "qcnn_ref_witness")
 
 
@@ -329,9 +345,9 @@ def run_reference(args, rank: int, world: int):
     _, _, anchor, _ = build_inputs(0)
     anchor = anchor[:sample_frames]
     om = oracle.OracleModel(image)
-    # CPU port: one frame per step, bounded
+    # CPU port: one frame per step
     om.forward_blu(anchor[:1, :270])
-    cpu_steps = max(1, min(args.steps, 4))
+    cpu_steps = args.steps
     t0 = time.perf_counter()
     for i in range(cpu_steps):
         cpu_out = om.forward_blu(anchor[i % sample_frames:i % sample_frames + 1])
@@ -347,7 +363,8 @@ def run_reference(args, rank: int, world: int):
             open(mf, "wb").write(image)
             anchor.tofile(fi)
             reps = args.warmup + args.steps
-            p = subprocess.run([REF_BIN, mf, str(H), str(W), str(sample_frames), fi, fo, str(reps)], capture_output=True, text=True, timeout=1500)
+            p = subprocess.run([REF_BIN, mf, str(H), str(W), str(sample_frames), fi, fo, str(reps)], capture_output=True, text=True,
+                               timeout=300 + 30 * reps)     # a step of the reference takes ~3 s on a B200
             times = [int(l.split(":")[1]) for l in p.stdout.splitlines() if l.startswith("time_us:")]
             if p.returncode == 0 and len(times) == reps:
                 timed = times[args.warmup:]
@@ -386,12 +403,17 @@ def main():
     ap.add_argument("--no-extra-configs", action="store_true", help="skip the config4 / config5 blocks")
     ap.add_argument("--reference-kind", default="auto", choices=["auto", "cpu"],
                     help="--impl reference: auto = the real reference (cuDNN) when it can run, cpu = the CPU port only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a fixed, seeded sample of what the last one computed (rank 0) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.impl == "reference":
-        args.steps = max(1, min(args.steps, 20))
         run_reference(args, rank, world)
         return
 
@@ -452,6 +474,8 @@ def main():
     barrier()
     launches = net.launch_count() - l0
     sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_out)
     total_ms = evs[0].elapsed_time(evs[-1])
     step_ms = [evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)]
 
