@@ -116,11 +116,26 @@ QV_API int qv_forward_frames_host(qv_net *net, const uint8_t *h_in, uint8_t *h_o
    vrcnn_data::psnr, inference/yuv_data.cpp:87-97).  ori_yuv, recon_yuv, sse_before, sse_after may be NULL. */
 QV_API int qv_stream_yuv(qv_net *net, const char *anchor_yuv, const char *ori_yuv, const char *recon_yuv,
                          int first_frame, int n_frames, int64_t *sse_before, int64_t *sse_after);
+/* qv_stream_yuv with the SSEs per frame, the integer core of vrcnn_data::psnr_pf (inference/yuv_data.cpp:98-112):
+   sse_before_pf[j] / sse_after_pf[j] = SSE of the anchor / the reconstruction against the original for frame
+   first_frame + j.  Both are host arrays of n_frames (either may be NULL; both need ori_yuv).  qv_stream_yuv returns
+   their sums. */
+QV_API int qv_stream_yuv_pf(qv_net *net, const char *anchor_yuv, const char *ori_yuv, const char *recon_yuv,
+                            int first_frame, int n_frames, int64_t *sse_before_pf, int64_t *sse_after_pf);
 /* Same pass on frames already resident in device memory (n_frames may exceed `batch`);
    asynchronous on `cuda_stream` (a cudaStream_t, NULL = the handle's own stream, in which
    case the call synchronises before returning). */
 QV_API int qv_forward_frames_device(qv_net *net, const uint8_t *d_in, uint8_t *d_out, int n_frames,
                                     void *cuda_stream);
+/* qv_forward_frames_device plus the per-frame quality report of vrcnn_data::psnr_pf (inference/yuv_data.cpp:98-112):
+   for every frame f the exact sum of (anchor - ori)^2 is ADDED to d_sse[2f] and the sum of (out - ori)^2 to
+   d_sse[2f + 1] (device int64, [n_frames][2]; incremented like qv_sse_device, so chunks and repeated calls add up).
+   d_ori holds the original luma of the same n_frames frames.  The output is byte-identical to qv_forward_frames_device.
+   The fused path computes the sums in the kernel's output stage (one extra byte read per pixel; there is no SSE form of
+   the opt-in QV_FUSED_TMA input ring, so with it set this call runs the kernel without TMA); the layered path runs a
+   separate SSE pass per frame.  Null d_ori / d_sse: QV_ERR_ARG; frame heights above 66051 are refused (QV_ERR_ARG). */
+QV_API int qv_forward_frames_device_sse(qv_net *net, const uint8_t *d_in, const uint8_t *d_ori, uint8_t *d_out,
+                                        int n_frames, int64_t *d_sse, void *cuda_stream);
 /* Spatially partitioned pass for one very large frame (multi-GPU strips): the frame has
    img_height x width pixels (width = the handle's); d_in points at image row `in_row0` and holds
    `in_rows` rows (the strip plus up to 6 halo rows each side); rows [out_row0, out_row1) are
@@ -169,6 +184,12 @@ QV_API int qv_strip_acquire(qv_net *net, int slot, void *cuda_stream);
 QV_API int qv_strip_load(qv_net *net, int slot, const uint8_t *host_rows, void *cuda_stream);
 /* forward_blu on this GPU's rows of the frame in `slot`; rows [row0, row1) of the reconstruction go to d_out. */
 QV_API int qv_strip_forward(qv_net *net, int slot, uint8_t *d_out, void *cuda_stream);
+/* qv_strip_forward plus this GPU's share of vrcnn_data::psnr_pf (inference/yuv_data.cpp:98-112) for the frame: d_ori_rows
+   holds the original's rows [row0, row1) (device memory of this GPU), and the SSEs of the anchor and of the reconstruction
+   over those rows are ADDED to d_sse2[0] and d_sse2[1] (device int64).  The caller adds the strips' values together.
+   Null d_ori_rows / d_sse2: QV_ERR_ARG; not the fused path: QV_ERR_STATE, as qv_strip_forward. */
+QV_API int qv_strip_forward_sse(qv_net *net, int slot, const uint8_t *d_ori_rows, uint8_t *d_out, int64_t *d_sse2,
+                                void *cuda_stream);
 /* Unmaps the neighbours and frees the block (all GPUs must be idle). */
 QV_API int qv_strip_release(qv_net *net);
 

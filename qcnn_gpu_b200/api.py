@@ -26,14 +26,14 @@ ABI_SYMBOLS = (
     "qv_last_error", "qv_version", "qv_create", "qv_destroy", "qv_load_static_para",
     "qv_load_static_para_mem", "qv_load_static_para_hwcn", "qv_load_quant_params", "qv_read_quant_params",
     "qv_set_weights", "qv_get_quant_params", "qv_load_data", "qv_forward_blu", "qv_get_recon",
-    "qv_forward_frames_host", "qv_stream_yuv", "qv_forward_frames_device", "qv_forward_rows_device", "qv_device_buffers",
+    "qv_forward_frames_host", "qv_stream_yuv", "qv_stream_yuv_pf", "qv_forward_frames_device", "qv_forward_frames_device_sse", "qv_forward_rows_device", "qv_device_buffers",
     "qv_sse_device", "qv_host_alloc", "qv_host_free",
     "qv_set_impl", "qv_get_impl", "qv_launch_count", "qv_get_activation",
     "qv_convert_model_hwcn_to_vect_c", "qv_yuv_read_luma", "qv_yuv_read_frame", "qv_yuv_write_recon",
     "qv_psnr", "qv_psnr_from_sse", "qv_solve_quant_params", "qv_write_quant_params_cpp", "qv_quantize_layer",
     "qv_debug_fused_tables", "qv_debug_fused_units", "qv_synchronize",
     "qv_strip_setup", "qv_strip_export", "qv_strip_attach", "qv_strip_input", "qv_strip_acquire", "qv_strip_load",
-    "qv_strip_forward", "qv_strip_release",
+    "qv_strip_forward", "qv_strip_forward_sse", "qv_strip_release",
 )
 
 CUDA_STREAM_LEGACY = 1      # cudaStreamLegacy: names the legacy default stream explicitly (NULL = "the handle's own stream")
@@ -81,11 +81,13 @@ def lib():
         L.qv_get_recon.argtypes = [vp, vp]
         L.qv_forward_frames_host.argtypes = [vp, vp, vp, i32]
         L.qv_forward_frames_device.argtypes = [vp, vp, vp, i32, vp]
+        L.qv_forward_frames_device_sse.argtypes = [vp, vp, vp, vp, i32, vp, vp]
         L.qv_host_alloc.argtypes = [C.c_size_t]
         L.qv_host_alloc.restype = vp
         L.qv_host_free.argtypes = [vp]
         L.qv_host_free.restype = None
         L.qv_stream_yuv.argtypes = [vp, cp, cp, cp, i32, i32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+        L.qv_stream_yuv_pf.argtypes = [vp, cp, cp, cp, i32, i32, vp, vp]
         L.qv_forward_rows_device.argtypes = [vp, vp, i32, i32, i32, vp, i32, i32, vp]
         L.qv_sse_device.argtypes = [vp, vp, C.c_size_t, vp, vp]
         L.qv_set_impl.argtypes = [vp, i32]
@@ -112,6 +114,7 @@ def lib():
         L.qv_strip_acquire.argtypes = [vp, i32, vp]
         L.qv_strip_load.argtypes = [vp, i32, vp, vp]
         L.qv_strip_forward.argtypes = [vp, i32, vp, vp]
+        L.qv_strip_forward_sse.argtypes = [vp, i32, vp, vp, vp, vp]
         L.qv_strip_release.argtypes = [vp]
         _lib = L
     return _lib
@@ -202,11 +205,26 @@ class QVRCNN:
                                    C.byref(b) if ori_yuv else None, C.byref(a) if ori_yuv else None))
         return int(b.value), int(a.value)
 
+    def stream_yuv_pf(self, anchor_yuv: str, ori_yuv: str, recon_yuv: Optional[str], first_frame: int, n_frames: int):
+        """qv_stream_yuv_pf: returns (sse_before, sse_after), two np.int64 arrays of n_frames -- the per-frame SSEs of the
+        anchor and of the reconstruction against the original (vrcnn_data::psnr_pf, inference/yuv_data.cpp:98-112)."""
+        before = np.zeros(max(n_frames, 0), np.int64)
+        after = np.zeros(max(n_frames, 0), np.int64)
+        enc = lambda p: os.fsencode(p) if p else None
+        _check(lib().qv_stream_yuv_pf(self._h, enc(anchor_yuv), enc(ori_yuv), enc(recon_yuv), first_frame, n_frames,
+                                      before.ctypes.data, after.ctypes.data))
+        return before, after
+
     def forward_frames_host_ptr(self, in_ptr: int, out_ptr: int, n: int) -> None:
         _check(lib().qv_forward_frames_host(self._h, in_ptr, out_ptr, n))
 
     def forward_frames_device(self, d_in: int, d_out: int, n: int, stream: int = 0) -> None:
         _check(lib().qv_forward_frames_device(self._h, d_in, d_out, n, stream or None))
+
+    def forward_frames_device_sse(self, d_in: int, d_ori: int, d_out: int, n: int, d_sse: int, stream: int = 0) -> None:
+        """forward_frames_device, and per frame f the SSEs of the input / the output against d_ori ADDED to the device int64
+        pair d_sse[2f], d_sse[2f + 1]."""
+        _check(lib().qv_forward_frames_device_sse(self._h, d_in, d_ori, d_out, n, d_sse, stream or None))
 
     def forward_rows_device(self, d_in: int, img_height: int, in_row0: int, in_rows: int, d_out: int,
                             out_row0: int, out_row1: int, stream: int = 0) -> None:
@@ -246,6 +264,11 @@ class QVRCNN:
 
     def strip_forward(self, slot: int, d_out: int, stream: int = 0) -> None:
         _check(lib().qv_strip_forward(self._h, slot, d_out, stream or None))
+
+    def strip_forward_sse(self, slot: int, d_ori_rows: int, d_out: int, d_sse2: int, stream: int = 0) -> None:
+        """strip_forward, and the SSEs of this handle's rows (anchor, reconstruction against d_ori_rows) ADDED to the device
+        int64 pair d_sse2[0], d_sse2[1]; the strips' values add up to the frame's."""
+        _check(lib().qv_strip_forward_sse(self._h, slot, d_ori_rows, d_out, d_sse2, stream or None))
 
     def strip_release(self) -> None:
         _check(lib().qv_strip_release(self._h))

@@ -14,11 +14,16 @@
 //                and no collective between frames
 //   --stream     files in, file out through qv_stream_yuv: the sequence is never held in host memory (reader thread,
 //                GPU stage and writer thread overlap); PSNR from the exact on-device SSE
+//   --psnr-pf    after the report, the per-frame PSNR of vrcnn_data::psnr_pf (inference/yuv_data.cpp:98-112), one line
+//                "PSNR of Frame %d:%f" per frame, then the mean of the per-frame PSNR before and after the net.  Default mode
+//                and --gpus: from the host buffers; --stream: qv_stream_yuv_pf; --strips: qv_strip_forward_sse, every strip
+//                uploads its rows of the original and the host adds the strips' SSEs
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <ctime>
+#include <mutex>
 #include <string>
 #include <thread>
 #include <vector>
@@ -34,8 +39,23 @@ struct Options {
     std::vector<int> qps{22};
     int frames = 1, gpus = 1, strips = 0;
     std::string save_recon;
-    bool stream = false;
+    bool stream = false, psnr_pf = false;
 };
+
+// --psnr-pf: the lines of vrcnn_data::psnr_pf (inference/yuv_data.cpp:98-112, format of yuv_data.h) from per-frame SSEs of the
+// anchor (before) and of the reconstruction (after), then the means of the per-frame PSNR
+static void print_psnr_pf(const std::vector<int64_t> &before, const std::vector<int64_t> &after, size_t fpx)
+{
+    double mb = 0, ma = 0;
+    for (size_t n = 0; n < after.size(); ++n) {
+        const double pa = qv_psnr_from_sse(after[n], fpx);
+        printf("PSNR of Frame %d:%f\n", (int)n, pa);
+        ma += pa;
+        mb += qv_psnr_from_sse(before[n], fpx);
+    }
+    const double k = after.empty() ? 1.0 : (double)after.size();
+    printf("mean per-frame PSNR: before net:%f after quantized net:%f\n", mb / k, ma / k);
+}
 
 static void report(const char *input_fn, int frame, int height, int width, double psnr1, double psnr2, long long us)
 {
@@ -81,6 +101,8 @@ static void testqvrcnn_strips(const char *ori_fn, const char *input_fn, const ch
     // hosts several strips (more strips than GPUs: a test layout) drives all of them on ONE stream, frame by frame, all
     // loads before the forwards: strips on one GPU are ordered by stream order, never by kernels waiting for each other.
     std::vector<std::string> errs(G);
+    std::vector<int64_t> sse_b(opt.psnr_pf ? frame : 0, 0), sse_a(opt.psnr_pf ? frame : 0, 0);      // summed over the strips
+    std::mutex sse_mu;
     auto t0 = std::chrono::steady_clock::now();
     {
         std::vector<std::thread> th;
@@ -92,12 +114,16 @@ static void testqvrcnn_strips(const char *ori_fn, const char *input_fn, const ch
                 const bool solo = mine.size() == 1;
                 cudaStream_t st[2] = {nullptr, nullptr};
                 cudaEvent_t ev = nullptr;
-                std::vector<uint8_t *> d_out(mine.size() * 2, nullptr);
+                std::vector<uint8_t *> d_out(mine.size() * 2, nullptr), d_ori(opt.psnr_pf ? mine.size() * 2 : 0, nullptr);
+                int64_t *d_sse = nullptr;                          // --psnr-pf: [strip j][frame][2]
                 bool ok = cudaSetDevice(g) == cudaSuccess && cudaEventCreateWithFlags(&ev, cudaEventDisableTiming) == cudaSuccess;
                 for (int s = 0; s < 2 && ok; ++s) ok = cudaStreamCreateWithFlags(&st[s], cudaStreamNonBlocking) == cudaSuccess;
                 for (size_t j = 0; j < mine.size() && ok; ++j)
                     for (int s = 0; s < 2 && ok; ++s)
                         ok = cudaMalloc(&d_out[j * 2 + s], (size_t)(r1[mine[j]] - r0[mine[j]]) * W) == cudaSuccess;
+                for (size_t j = 0; j < d_ori.size() && ok; ++j) ok = cudaMalloc(&d_ori[j], (size_t)(r1[mine[j / 2]] - r0[mine[j / 2]]) * W) == cudaSuccess;
+                const size_t sse_bytes = mine.size() * (size_t)frame * 2 * sizeof(int64_t);
+                if (opt.psnr_pf && ok) ok = cudaMalloc(&d_sse, sse_bytes) == cudaSuccess && cudaMemset(d_sse, 0, sse_bytes) == cudaSuccess;
                 if (!ok) errs[g] = "CUDA setup failed";
                 for (int k = 0; k < frame && ok; ++k) {
                     const int s = k & 1;
@@ -105,8 +131,13 @@ static void testqvrcnn_strips(const char *ori_fn, const char *input_fn, const ch
                     for (size_t j = 0; j < mine.size() && ok; ++j)
                         ok = qv_strip_load(nets[mine[j]], s, test_data.input + (size_t)k * fpx + (size_t)r0[mine[j]] * W, q) == QV_OK;
                     if (ok && solo && k > 0) ok = cudaStreamWaitEvent(q, ev, 0) == cudaSuccess;
+                    for (size_t j = 0; j < d_ori.size() / 2 && ok; ++j)      // this strip's rows of the original, same slot scheme
+                        ok = cudaMemcpyAsync(d_ori[j * 2 + s], test_data.ori + (size_t)k * fpx + (size_t)r0[mine[j]] * W,
+                                             (size_t)(r1[mine[j]] - r0[mine[j]]) * W, cudaMemcpyHostToDevice, q) == cudaSuccess;
                     for (size_t j = 0; j < mine.size() && ok; ++j)
-                        ok = qv_strip_forward(nets[mine[j]], s, d_out[j * 2 + s], q) == QV_OK;
+                        ok = (opt.psnr_pf ? qv_strip_forward_sse(nets[mine[j]], s, d_ori[j * 2 + s], d_out[j * 2 + s],
+                                                                 d_sse + (j * (size_t)frame + k) * 2, q)
+                                          : qv_strip_forward(nets[mine[j]], s, d_out[j * 2 + s], q)) == QV_OK;
                     if (ok && solo) ok = cudaEventRecord(ev, q) == cudaSuccess;
                     for (size_t j = 0; j < mine.size() && ok; ++j) {
                         const int i = mine[j];
@@ -119,6 +150,15 @@ static void testqvrcnn_strips(const char *ori_fn, const char *input_fn, const ch
                     if (st[s] && qv_synchronize(nets[mine[0]], st[s]) != QV_OK && errs[g].empty()) errs[g] = qv_last_error();
                 for (size_t j = 1; j < mine.size(); ++j)
                     if (qv_synchronize(nets[mine[j]], st[0]) != QV_OK && errs[g].empty()) errs[g] = qv_last_error();
+                if (d_sse && errs[g].empty()) {
+                    std::vector<int64_t> h(mine.size() * (size_t)frame * 2);
+                    if (cudaMemcpy(h.data(), d_sse, sse_bytes, cudaMemcpyDeviceToHost) != cudaSuccess) errs[g] = "copy of the SSEs failed";
+                    std::lock_guard<std::mutex> l(sse_mu);
+                    for (size_t j = 0; j < mine.size(); ++j)
+                        for (int k = 0; k < frame; ++k) { sse_b[k] += h[(j * frame + k) * 2]; sse_a[k] += h[(j * frame + k) * 2 + 1]; }
+                }
+                cudaFree(d_sse);
+                for (uint8_t *p : d_ori) cudaFree(p);
                 for (uint8_t *p : d_out) cudaFree(p);
                 for (int s = 0; s < 2; ++s) if (st[s]) cudaStreamDestroy(st[s]);
                 if (ev) cudaEventDestroy(ev);
@@ -136,6 +176,7 @@ static void testqvrcnn_strips(const char *ori_fn, const char *input_fn, const ch
     printf("throughput:%.1f Mpixel/s (%d frame(s) of %dx%d in %d strip(s) on %d GPU(s), halo rows over peer-mapped memory, copies included)\n",
            (double)frame * fpx / (double)us, frame, width, height, S, G);
     report(input_fn, frame, height, width, psnr1, psnr2, us);
+    if (opt.psnr_pf) print_psnr_pf(sse_b, sse_a, fpx);
 }
 
 static void testqvrcnn(const char *ori_fn, const char *input_fn, const char *model_fn, int frame, int channel, int height,
@@ -179,6 +220,14 @@ static void testqvrcnn(const char *ori_fn, const char *input_fn, const char *mod
     printf("throughput:%.1f Mpixel/s (%d frame(s) of %dx%d on %d GPU(s), host buffers, copies included)\n",
            (double)frame * fpx / (double)us, frame, width, height, G);
     report(input_fn, frame, height, width, psnr1, psnr2, us);
+    if (opt.psnr_pf) {
+        std::vector<int64_t> b(frame), a(frame);
+        for (int n = 0; n < frame; ++n) {
+            qv_psnr(test_data.input + (size_t)n * fpx, test_data.ori + (size_t)n * fpx, fpx, &b[n]);
+            qv_psnr(test_data.recon + (size_t)n * fpx, test_data.ori + (size_t)n * fpx, fpx, &a[n]);
+        }
+        print_psnr_pf(b, a, fpx);
+    }
 }
 
 // --stream: the same report from the streaming pipeline.  Each GPU takes a contiguous frame range and fills its own part
@@ -195,7 +244,7 @@ static void testqvrcnn_stream(const char *ori_fn, const char *input_fn, const ch
             exit(1);
         }
     }
-    std::vector<long long> sb(G, 0), sa(G, 0);
+    std::vector<int64_t> pf_b(frame, 0), pf_a(frame, 0);              // per frame; GPU g fills its own frame range
     std::vector<int> rcs(G, 0);
     std::vector<std::string> errs(G);
     if (!opt.save_recon.empty()) {
@@ -215,9 +264,8 @@ static void testqvrcnn_stream(const char *ori_fn, const char *input_fn, const ch
         for (int g = 0; g < G; ++g) {
             const int nf = frame / G + (g < frame % G ? 1 : 0);
             th.emplace_back([&, g, f0, nf] {
-                int64_t b = 0, a = 0;
-                rcs[g] = qv_stream_yuv(nets[g], input_fn, ori_fn, opt.save_recon.empty() ? nullptr : opt.save_recon.c_str(), f0, nf, &b, &a);
-                sb[g] = b; sa[g] = a;
+                rcs[g] = qv_stream_yuv_pf(nets[g], input_fn, ori_fn, opt.save_recon.empty() ? nullptr : opt.save_recon.c_str(), f0, nf,
+                                          pf_b.data() + f0, pf_a.data() + f0);
                 if (rcs[g]) errs[g] = qv_last_error();                      // thread-local: copy it in this thread
             });
             f0 += nf;
@@ -229,14 +277,15 @@ static void testqvrcnn_stream(const char *ori_fn, const char *input_fn, const ch
     long long b = 0, a = 0;
     for (int g = 0; g < G; ++g) {
         if (rcs[g]) { printf("%s\n", errs[g].c_str()); exit(1); }
-        b += sb[g]; a += sa[g];
         qv_destroy(nets[g]);
     }
+    for (int n = 0; n < frame; ++n) { b += pf_b[n]; a += pf_a[n]; }
     const double psnr1 = qv_psnr_from_sse(b, (size_t)frame * fpx), psnr2 = qv_psnr_from_sse(a, (size_t)frame * fpx);
     printf("\nbefore net:PSNR=%.3f\nafter quantized net:PSNR=%.3f\ntime:%lldus\n", psnr1, psnr2, us);
     printf("throughput:%.1f Mpixel/s (%d frame(s) of %dx%d on %d GPU(s), streamed from and to files)\n",
            (double)frame * fpx / (double)us, frame, width, height, G);
     report(input_fn, frame, height, width, psnr1, psnr2, us);
+    if (opt.psnr_pf) print_psnr_pf(pf_b, pf_a, fpx);
 }
 
 static int run_all(const char *oriname, const char *inputname, int height, int width, const Options &opt)
@@ -255,7 +304,7 @@ static int run_all(const char *oriname, const char *inputname, int height, int w
 int main(int argc, char **argv)
 {
     if (argc < 5) {
-        fprintf(stderr, "usage: %s <ori.yuv> <anchor_prefix> <H> <W> [--model tmpl%%d] [--qp 22,27,..] [--frames n] [--gpus n] [--save-recon f] [--stream] [--strips n]\n", argv[0]);
+        fprintf(stderr, "usage: %s <ori.yuv> <anchor_prefix> <H> <W> [--model tmpl%%d] [--qp 22,27,..] [--frames n] [--gpus n] [--save-recon f] [--stream] [--strips n] [--psnr-pf]\n", argv[0]);
         return 2;
     }
     Options opt;
@@ -267,6 +316,7 @@ int main(int argc, char **argv)
         else if (a == "--save-recon" && i + 1 < argc) opt.save_recon = argv[++i];
         else if (a == "--strips" && i + 1 < argc) opt.strips = atoi(argv[++i]);
         else if (a == "--stream") opt.stream = true;
+        else if (a == "--psnr-pf") opt.psnr_pf = true;
         else if (a == "--qp" && i + 1 < argc) {
             opt.qps.clear();
             for (char *t = strtok(argv[++i], ","); t; t = strtok(nullptr, ",")) opt.qps.push_back(atoi(t));

@@ -218,7 +218,11 @@ static int ensure_acts(qv_net *net)
     return QV_OK;
 }
 
-static int run_forward(qv_net *net, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W, cudaStream_t st)
+// With d_ori / d_sse: also adds, per frame f, the SSE of the input and of the output against d_ori to d_sse[2f], d_sse[2f + 1]
+// (the integer core of vrcnn_data::psnr_pf, inference/yuv_data.cpp:98-112).  The fused path computes them in the kernel's
+// output stage; the layered path, the independent cross-check, runs sse_accumulate once per frame on (in, ori) and (out, ori).
+static int run_forward(qv_net *net, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W, cudaStream_t st,
+                       const uint8_t *d_ori = nullptr, int64_t *d_sse = nullptr)
 {
     if (!net->uploaded) {
         set_error("forward called before a complete model (weights + quant params) was loaded");
@@ -228,7 +232,8 @@ static int run_forward(qv_net *net, const uint8_t *d_in, uint8_t *d_out, int n, 
     if (impl == QV_IMPL_AUTO) impl = net->fm ? QV_IMPL_FUSED : QV_IMPL_LAYERED;
     if (impl == QV_IMPL_FUSED) {
         if (!net->fm) { set_error("fused tcgen05 path is not available in this build"); return QV_ERR_STATE; }
-        QV_CUDA(fused_forward(net->fm, d_in, d_out, n, H, W, st, &net->launches));
+        if (d_sse && H > FUSED_SSE_MAX_H) { set_error("per-frame SSE: frame height %d exceeds %d", H, FUSED_SSE_MAX_H); return QV_ERR_ARG; }
+        QV_CUDA(fused_forward(net->fm, d_in, d_out, n, H, W, st, &net->launches, nullptr, d_ori, d_sse));
         return QV_OK;
     }
     int rc = ensure_acts(net);
@@ -242,6 +247,14 @@ static int run_forward(qv_net *net, const uint8_t *d_in, uint8_t *d_out, int n, 
         const int c = std::min(chunk, n - f0);
         QV_CUDA(layered_forward(net->lm, d_in + (size_t)f0 * fpx, d_out + (size_t)f0 * fpx, c, H, W, net->d_a1,
                                 net->d_a2, net->d_a3, st, &net->launches));
+    }
+    if (d_sse) {
+        for (int f = 0; f < n; ++f) {
+            const size_t o = (size_t)f * fpx;
+            QV_CUDA(sse_accumulate(d_in + o, d_ori + o, fpx, d_sse + 2 * f, st));
+            QV_CUDA(sse_accumulate(d_out + o, d_ori + o, fpx, d_sse + 2 * f + 1, st));
+        }
+        net->launches += 2 * n;
     }
     return QV_OK;
 }
@@ -449,6 +462,22 @@ int qv_forward_frames_device(qv_net *net, const uint8_t *d_in, uint8_t *d_out, i
     cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : net->st;
     if (n_frames > 0) {
         rc = run_forward(net, d_in, d_out, n_frames, net->H, net->W, st);
+        if (rc) return rc;
+    }
+    if (!cuda_stream) { QV_CUDA(cudaStreamSynchronize(st)); return kernel_report(net); }
+    return QV_OK;
+}
+
+int qv_forward_frames_device_sse(qv_net *net, const uint8_t *d_in, const uint8_t *d_ori, uint8_t *d_out, int n_frames,
+                                 int64_t *d_sse, void *cuda_stream)
+{
+    // per-frame form of vrcnn_data::psnr_pf (inference/yuv_data.cpp:98-112): exact integer SSEs, incremented
+    if (!net || !d_in || !d_ori || !d_out || !d_sse || n_frames < 0) { set_error("qv_forward_frames_device_sse: bad argument"); return QV_ERR_ARG; }
+    int rc = set_device(net);
+    if (rc) return rc;
+    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : net->st;
+    if (n_frames > 0) {
+        rc = run_forward(net, d_in, d_out, n_frames, net->H, net->W, st, d_ori, d_sse);
         if (rc) return rc;
     }
     if (!cuda_stream) { QV_CUDA(cudaStreamSynchronize(st)); return kernel_report(net); }
@@ -699,23 +728,23 @@ int qv_strip_load(qv_net *net, int slot, const uint8_t *host_rows, void *cuda_st
     return QV_OK;
 }
 
-int qv_strip_forward(qv_net *net, int slot, uint8_t *d_out, void *cuda_stream)
+static int strip_forward(qv_net *net, int slot, const uint8_t *d_ori, uint8_t *d_out, int64_t *d_sse, void *cuda_stream, const char *who)
 {
-    if (!net || !d_out || slot < 0 || slot > 1) { set_error("qv_strip_forward: bad argument"); return QV_ERR_ARG; }
     StripState &S = net->strip;
-    if (!S.on) { set_error("qv_strip_forward: qv_strip_setup has not been called"); return QV_ERR_STATE; }
+    if (!S.on) { set_error("%s: qv_strip_setup has not been called", who); return QV_ERR_STATE; }
     if (!net->uploaded || !net->fm || net->impl == QV_IMPL_LAYERED) {
-        set_error("qv_strip_forward: needs a loaded model and the fused path (peer-mapped halo rows are read by the fused kernel)");
+        set_error("%s: needs a loaded model and the fused path (peer-mapped halo rows are read by the fused kernel)", who);
         return QV_ERR_STATE;
     }
     if ((S.row0 > 0 && !S.peer[QV_STRIP_ABOVE].attached) || (S.row1 < S.img_h && !S.peer[QV_STRIP_BELOW].attached)) {
-        set_error("qv_strip_forward: rows [%d, %d) of %d have an interior edge with no neighbour attached", S.row0, S.row1, S.img_h);
+        set_error("%s: rows [%d, %d) of %d have an interior edge with no neighbour attached", who, S.row0, S.row1, S.img_h);
         return QV_ERR_STATE;
     }
+    if (d_sse && S.img_h > FUSED_SSE_MAX_H) { set_error("%s: frame height %d exceeds %d", who, S.img_h, FUSED_SSE_MAX_H); return QV_ERR_ARG; }
     int rc = set_device(net);
     if (rc) return rc;
     cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : net->st;
-    if ((rc = check_shared_device_stream(net, st, "qv_strip_forward"))) return rc;
+    if ((rc = check_shared_device_stream(net, st, who))) return rc;
     const size_t W = net->W;
     FusedRows fr;
     fr.own0 = fr.out0 = S.row0; fr.own1 = fr.out1 = S.row1;
@@ -731,7 +760,7 @@ int qv_strip_forward(qv_net *net, int slot, uint8_t *d_out, void *cuda_stream)
             // a neighbour on this very GPU: no kernel may wait for it -- its rows are ordered before this launch by the shared
             // stream, provided its slot was filled for this frame already (checked here, on the host)
             if (P.net->strip.fills[slot] == 0) {
-                set_error("qv_strip_forward: the neighbour strip on the same GPU has not filled slot %d yet (strips that share a GPU: all loads of a frame, then its forwards, on one stream)", slot);
+                set_error("%s: the neighbour strip on the same GPU has not filled slot %d yet (strips that share a GPU: all loads of a frame, then its forwards, on one stream)", who, slot);
                 return QV_ERR_STATE;
             }
             flag = nullptr;
@@ -745,9 +774,22 @@ int qv_strip_forward(qv_net *net, int slot, uint8_t *d_out, void *cuda_stream)
     S.last_stream = st; S.used = true;
     fr.seq = seq;
     const uint8_t *own = S.block + STRIP_HDR + (size_t)slot * S.slot_stride;
-    QV_CUDA(fused_forward(net->fm, own, d_out, 1, S.img_h, net->W, st, &net->launches, &fr));
+    QV_CUDA(fused_forward(net->fm, own, d_out, 1, S.img_h, net->W, st, &net->launches, &fr, d_ori, d_sse));
     if (!cuda_stream) { QV_CUDA(cudaStreamSynchronize(st)); return kernel_report(net); }
     return QV_OK;
+}
+
+int qv_strip_forward(qv_net *net, int slot, uint8_t *d_out, void *cuda_stream)
+{
+    if (!net || !d_out || slot < 0 || slot > 1) { set_error("qv_strip_forward: bad argument"); return QV_ERR_ARG; }
+    return strip_forward(net, slot, nullptr, d_out, nullptr, cuda_stream, "qv_strip_forward");
+}
+
+int qv_strip_forward_sse(qv_net *net, int slot, const uint8_t *d_ori_rows, uint8_t *d_out, int64_t *d_sse2, void *cuda_stream)
+{
+    // this GPU's share of vrcnn_data::psnr_pf (inference/yuv_data.cpp:98-112) for one frame; the strips' values add up
+    if (!net || !d_ori_rows || !d_out || !d_sse2 || slot < 0 || slot > 1) { set_error("qv_strip_forward_sse: bad argument"); return QV_ERR_ARG; }
+    return strip_forward(net, slot, d_ori_rows, d_out, d_sse2, cuda_stream, "qv_strip_forward_sse");
 }
 
 int qv_forward_frames_host(qv_net *net, const uint8_t *h_in, uint8_t *h_out, int n_frames)
@@ -861,15 +903,20 @@ bool read_luma(FILE *f, long long frame, size_t fpx, uint8_t *dst)
 }
 }  // namespace
 
-int qv_stream_yuv(qv_net *net, const char *anchor_yuv, const char *ori_yuv, const char *recon_yuv, int first_frame, int n_frames,
-                  int64_t *sse_before, int64_t *sse_after)
+// Per-frame SSEs of the anchor and of the reconstruction against the original (vrcnn_data::psnr_pf, inference/yuv_data.cpp:98-112)
+// for frames [first_frame, first_frame + n_frames): they are computed with the reconstruction (in the fused kernel, or per frame
+// on the layered path) into a device array of n_frames pairs and copied out once at the end.
+int qv_stream_yuv_pf(qv_net *net, const char *anchor_yuv, const char *ori_yuv, const char *recon_yuv, int first_frame, int n_frames,
+                     int64_t *sse_before_pf, int64_t *sse_after_pf)
 {
-    if (!net || !anchor_yuv || first_frame < 0 || n_frames < 0) { set_error("qv_stream_yuv: bad argument"); return QV_ERR_ARG; }
-    if ((sse_before || sse_after) && !ori_yuv) { set_error("qv_stream_yuv: an SSE was asked for but no original file given"); return QV_ERR_ARG; }
+    if (!net || !anchor_yuv || first_frame < 0 || n_frames < 0) { set_error("qv_stream_yuv_pf: bad argument"); return QV_ERR_ARG; }
+    if ((sse_before_pf || sse_after_pf) && !ori_yuv) { set_error("qv_stream_yuv_pf: an SSE was asked for but no original file given"); return QV_ERR_ARG; }
     int rc = set_device(net);
     if (rc) return rc;
-    if (sse_before) *sse_before = 0;
-    if (sse_after) *sse_after = 0;
+    for (int j = 0; j < n_frames; ++j) {
+        if (sse_before_pf) sse_before_pf[j] = 0;
+        if (sse_after_pf) sse_after_pf[j] = 0;
+    }
     if (n_frames == 0) return QV_OK;
     const size_t fpx = (size_t)net->H * net->W;
     const int C = net->batch, NS = 3;
@@ -886,9 +933,10 @@ int qv_stream_yuv(qv_net *net, const char *anchor_yuv, const char *ori_yuv, cons
     }
     StreamSlot slot[3];
     StreamShared sh;
-    int64_t *d_sse = nullptr;
-    cudaError_t e = cudaMalloc(&d_sse, 2 * sizeof(int64_t));
-    if (e == cudaSuccess) e = cudaMemset(d_sse, 0, 2 * sizeof(int64_t));
+    int64_t *d_sse = nullptr;                                   // [n_frames][2]
+    const size_t sse_bytes = (size_t)n_frames * 2 * sizeof(int64_t);
+    cudaError_t e = cudaMalloc(&d_sse, sse_bytes);
+    if (e == cudaSuccess) e = cudaMemset(d_sse, 0, sse_bytes);
     for (int s = 0; s < NS && e == cudaSuccess; ++s) {
         StreamSlot &S = slot[s];
         e = cudaMallocHost(&S.h_in, C * fpx);
@@ -979,12 +1027,8 @@ int qv_stream_yuv(qv_net *net, const char *anchor_yuv, const char *ori_yuv, cons
         // the layered path's launches share the handle's activation scratch: keep them in order across the slots' streams
         if (e == cudaSuccess && !fused_path && k > 0) e = cudaStreamWaitEvent(S.st, ev_compute, 0);
         if (e == cudaSuccess) {
-            rc = run_forward(net, S.d_in, S.d_out, S.c, net->H, net->W, S.st);
+            rc = run_forward(net, S.d_in, S.d_out, S.c, net->H, net->W, S.st, fo ? S.d_ori : nullptr, fo ? d_sse + 2 * (size_t)S.f0 : nullptr);
             if (rc == QV_OK && !fused_path) e = cudaEventRecord(ev_compute, S.st);
-            if (rc == QV_OK && fo) {
-                e = sse_accumulate(S.d_in, S.d_ori, bytes, d_sse + 0, S.st);
-                if (e == cudaSuccess) e = sse_accumulate(S.d_out, S.d_ori, bytes, d_sse + 1, S.st);
-            }
         }
         if (e == cudaSuccess && rc == QV_OK) e = cudaMemcpyAsync(S.h_out, S.d_out, bytes, cudaMemcpyDeviceToHost, S.st);
         if (e == cudaSuccess && rc == QV_OK) e = cudaEventRecord(S.done, S.st);
@@ -996,17 +1040,41 @@ int qv_stream_yuv(qv_net *net, const char *anchor_yuv, const char *ori_yuv, cons
     reader.join();
     writer.join();
     if (ev_compute) { for (int s = 0; s < NS; ++s) cudaStreamSynchronize(slot[s].st); cudaEventDestroy(ev_compute); }
-    int64_t h_sse[2] = {0, 0};
+    std::vector<int64_t> h_sse(fo ? (size_t)n_frames * 2 : 0);
     if (rc == QV_OK && !sh.failed) {
         for (int s = 0; s < NS; ++s) cudaStreamSynchronize(slot[s].st);
-        if (cudaMemcpy(h_sse, d_sse, sizeof(h_sse), cudaMemcpyDeviceToHost) != cudaSuccess) rc = QV_ERR_CUDA;
+        if (fo && cudaMemcpy(h_sse.data(), d_sse, sse_bytes, cudaMemcpyDeviceToHost) != cudaSuccess) {
+            set_error("qv_stream_yuv_pf: copy of the SSEs failed");
+            rc = QV_ERR_CUDA;
+        }
     }
     cleanup();
     if (rc == QV_OK && sh.failed) { set_error("%s", sh.msg); rc = strstr(sh.msg, "GPU") ? QV_ERR_CUDA : QV_ERR_IO; }
     if (rc != QV_OK) return rc;
-    if (sse_before) *sse_before = h_sse[0];
-    if (sse_after) *sse_after = h_sse[1];
+    for (int j = 0; fo && j < n_frames; ++j) {
+        if (sse_before_pf) sse_before_pf[j] = h_sse[2 * (size_t)j];
+        if (sse_after_pf) sse_after_pf[j] = h_sse[2 * (size_t)j + 1];
+    }
     return kernel_report(net);
+}
+
+int qv_stream_yuv(qv_net *net, const char *anchor_yuv, const char *ori_yuv, const char *recon_yuv, int first_frame, int n_frames,
+                  int64_t *sse_before, int64_t *sse_after)
+{
+    // the pooled SSEs of vrcnn_data::psnr (inference/yuv_data.cpp:87-97) are the sums of the per-frame ones
+    if (!net || !anchor_yuv || first_frame < 0 || n_frames < 0) { set_error("qv_stream_yuv: bad argument"); return QV_ERR_ARG; }
+    if ((sse_before || sse_after) && !ori_yuv) { set_error("qv_stream_yuv: an SSE was asked for but no original file given"); return QV_ERR_ARG; }
+    std::vector<int64_t> before(ori_yuv ? n_frames : 0), after(ori_yuv ? n_frames : 0);
+    const int rc = qv_stream_yuv_pf(net, anchor_yuv, ori_yuv, recon_yuv, first_frame, n_frames, ori_yuv ? before.data() : nullptr,
+                                    ori_yuv ? after.data() : nullptr);
+    if (sse_before) *sse_before = 0;
+    if (sse_after) *sse_after = 0;
+    if (rc != QV_OK) return rc;
+    for (size_t j = 0; j < before.size(); ++j) {
+        if (sse_before) *sse_before += before[j];
+        if (sse_after) *sse_after += after[j];
+    }
+    return QV_OK;
 }
 
 void *qv_host_alloc(size_t bytes)

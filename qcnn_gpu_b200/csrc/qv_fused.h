@@ -25,8 +25,15 @@ struct FusedRows {
     uint32_t seq = 0;
 };
 // Whole net on n frames of HxW luma resident in device memory, one launch.  With `rows`: n = 1, H = image height.
+// With d_ori and d_sse (both or neither): k_enh_sse instead of k_fused, the same reconstruction, and for every frame f of the
+// launch the exact sum (anchor - ori)^2 is ADDED to d_sse[2f] and sum (out - ori)^2 to d_sse[2f + 1] (device int64; the
+// integer core of vrcnn_data::psnr_pf, inference/yuv_data.cpp:98-112).  d_ori holds the same pixels as d_out (with `rows`:
+// rows [out0, out1)).  There is no SSE form of the profiling build or of the opt-in TMA input ring: with QV_FUSED_TMA=1 an
+// SSE launch runs the kernel without TMA.  H > FUSED_SSE_MAX_H is refused (cudaErrorInvalidValue).
+constexpr int FUSED_SSE_MAX_H = 66051;     // per-thread column sums are 32-bit: 255^2 * H < 2^32
 cudaError_t fused_forward(const FusedModel *fm, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W,
-                          cudaStream_t st, long long *launches, const FusedRows *rows = nullptr);
+                          cudaStream_t st, long long *launches, const FusedRows *rows = nullptr,
+                          const uint8_t *d_ori = nullptr, int64_t *d_sse = nullptr);
 // Stream-ordered helper of the strip protocol: spin (bounded) until *a >= va and *b >= vb (either pointer may be null; the
 // words live on OTHER GPUs), reporting a timeout through the model's failure word (code 3).
 cudaError_t fused_wait_words(const FusedModel *fm, const uint32_t *a, uint32_t va, const uint32_t *b, uint32_t vb, cudaStream_t st);

@@ -13,6 +13,10 @@
 --check additionally computes the whole job on rank 0 alone and asserts the N-GPU result is bit-identical; in strips mode
 every step of the check uploads a DIFFERENT frame (alternating the two input slots), so a halo row read too early or too
 late shows up as a mismatch.
+
+--per-frame adds the per-frame PSNR before and after the net (vrcnn_data::psnr_pf, inference/yuv_data.cpp:98-112): every rank
+fills its part of a zeroed [frames, 2] int64 tensor of exact SSEs -- its frame range (forward_frames_device_sse) or its rows of
+the frame (strip_forward_sse) -- and one all-reduce adds them up, so the result is the one-GPU result bit for bit.
 """
 from __future__ import annotations
 
@@ -63,6 +67,7 @@ def main():
     ap.add_argument("--width", type=int, default=3840)
     ap.add_argument("--steps", type=int, default=3)
     ap.add_argument("--check", action="store_true")
+    ap.add_argument("--per-frame", action="store_true", help="per-frame PSNR before / after the net in the JSON line")
     ap.add_argument("--uniq", type=int, default=4, help="distinct synthetic frames per rank (repeated)")
     args = ap.parse_args()
     rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
@@ -85,14 +90,20 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    check_outs = []
-    if args.mode == "frames":
-        f0, nf = shard.split(args.frames, rank, world)
+    def rank_frames(r):
+        """frames mode: the anchor and original frames of rank r (`uniq` distinct synthetic frames, repeated)"""
+        f0, nf = shard.split(args.frames, r, world)
         uniq = max(1, min(args.uniq, nf))
         a, o = synth.make_frames(0xC0FFEE + 4, uniq, h, w, first_frame=f0 % 1024)
         reps = (nf + uniq - 1) // uniq
-        d_in = torch.from_numpy(np.tile(a, (reps, 1, 1))[:nf]).cuda()
-        d_ori = torch.from_numpy(np.tile(o, (reps, 1, 1))[:nf]).cuda()
+        return np.tile(a, (reps, 1, 1))[:nf], np.tile(o, (reps, 1, 1))[:nf]
+
+    check_outs = []
+    if args.mode == "frames":
+        f0, nf = shard.split(args.frames, rank, world)
+        a, o = rank_frames(rank)
+        d_in = torch.from_numpy(a).cuda()
+        d_ori = torch.from_numpy(o).cuda()
         d_out = torch.empty_like(d_in)
         net = api.QVRCNN(local, max(1, min(nf, 8)), 1, h, w)
         net.load_static_para_mem(image)
@@ -148,6 +159,21 @@ def main():
               "frames": args.frames if args.mode == "frames" else 1,
               "Mpixel_per_s": n * args.steps / (float(ms.item()) * 1e-3) / 1e6, "ms_per_step": float(ms.item()) / args.steps,
               "after_quantized_net_PSNR": psnr, "sse": sse, "halo": halo}
+    if args.per_frame:
+        n_frames = args.frames if args.mode == "frames" else 1
+        pf = torch.zeros((n_frames, 2), dtype=torch.int64, device="cuda")
+        if args.mode == "frames":
+            net.forward_frames_device_sse(d_in.data_ptr(), d_ori.data_ptr(), d_out.data_ptr(), nf, pf[f0:].data_ptr(), sp)
+        else:                                    # slot 0 holds this rank's rows of the frame d_ori belongs to
+            net.strip_forward_sse(0, d_ori.data_ptr(), d_out.data_ptr(), pf.data_ptr(), sp)
+        net.synchronize(sp)
+        if world > 1:
+            dist.all_reduce(pf, op=dist.ReduceOp.SUM)
+        pf_host = pf.cpu().numpy()
+        before = [api.psnr_from_sse(int(v), h * w) for v in pf_host[:, 0]]
+        after = [api.psnr_from_sse(int(v), h * w) for v in pf_host[:, 1]]
+        result.update({"psnr_per_frame_before": before, "psnr_per_frame_after": after,
+                       "psnr_per_frame_mean_before": float(np.mean(before)), "psnr_per_frame_mean_after": float(np.mean(after))})
     if args.check:
         # gather every rank's output on rank 0 and compare with rank 0 computing everything alone
         mine = d_out.cpu().numpy() if args.mode == "frames" else np.stack([t.cpu().numpy() for t in check_outs])
@@ -158,10 +184,7 @@ def main():
         if rank == 0:
             if args.mode == "frames":
                 got = np.concatenate(outs)
-                full = np.concatenate([np.tile(synth.make_frames(0xC0FFEE + 4, max(1, min(args.uniq, shard.split(args.frames, r, world)[1])), h, w,
-                                                first_frame=shard.split(args.frames, r, world)[0] % 1024)[0],
-                                               ((shard.split(args.frames, r, world)[1] + args.uniq - 1) // max(1, args.uniq) + 1, 1, 1))[:shard.split(args.frames, r, world)[1]]
-                                       for r in range(world)])
+                full = np.concatenate([rank_frames(r)[0] for r in range(world)])
                 solo = api.QVRCNN(local, 4, 1, h, w)
             else:
                 got = np.concatenate(outs, axis=1)                      # [steps, h, w]
@@ -171,6 +194,16 @@ def main():
             want = solo.forward_frames_host(full)
             result["bit_identical_to_1gpu"] = bool(np.array_equal(got.reshape(want.shape), want))
             result["distinct_frames_checked"] = int(want.shape[0])
+            if args.per_frame:
+                # the all-reduced per-frame SSEs against rank 0's own computation of the frames of the report
+                if args.mode == "frames":
+                    anc, ori = full, np.concatenate([rank_frames(r)[1] for r in range(world)])
+                    rec = want
+                else:
+                    anc, ori = synth.make_frames(0xC0FFEE + 5, 1, h, w)
+                    rec = solo.forward_frames_host(anc)
+                sse = lambda x: ((x.astype(np.int64) - ori.astype(np.int64)) ** 2).reshape(len(ori), -1).sum(axis=1)
+                result["per_frame_sse_identical_to_1gpu"] = bool(np.array_equal(pf_host, np.stack([sse(anc), sse(rec)], axis=1)))
     if rank == 0:
         print(json.dumps(result))
     if world > 1:
