@@ -133,7 +133,8 @@ QV_API int qv_forward_frames_device(qv_net *net, const uint8_t *d_in, uint8_t *d
    d_ori holds the original luma of the same n_frames frames.  The output is byte-identical to qv_forward_frames_device.
    The fused path computes the sums in the kernel's output stage (one extra byte read per pixel; there is no SSE form of
    the opt-in QV_FUSED_TMA input ring, so with it set this call runs the kernel without TMA); the layered path runs a
-   separate SSE pass per frame.  Null d_ori / d_sse: QV_ERR_ARG; frame heights above 66051 are refused (QV_ERR_ARG). */
+   separate SSE pass per frame.  Null d_ori / d_sse: QV_ERR_ARG; on the fused path frame heights above 66051 are refused
+   (QV_ERR_ARG), the layered path takes any height. */
 QV_API int qv_forward_frames_device_sse(qv_net *net, const uint8_t *d_in, const uint8_t *d_ori, uint8_t *d_out,
                                         int n_frames, int64_t *d_sse, void *cuda_stream);
 /* Spatially partitioned pass for one very large frame (multi-GPU strips): the frame has

@@ -51,7 +51,6 @@ class Emu:
     def __init__(self, model_bytes, rng):
         self.k, wimg, self.ops, self.groups, self.bias, c4w = fused_tables(model_bytes)
         k = self.k
-        assert k["fast"] == 1
         self.sm = np.zeros(k["SMEM_BYTES"], np.uint8)
         self.sm[:k["WIMG_BYTES"]] = wimg
         self.tmem = rng.integers(-2**31, 2**31 - 1, size=(128, 512), dtype=np.int64).astype(np.int32)     # never initialised
@@ -91,10 +90,16 @@ class Emu:
 
     # ---- workers: TMEM -> requantise -> activation rows ---------------------------------------------------
     def requant_store(self, col, boff, g, valid, dst):
-        hi, M = int(self.groups[g][0]), int(self.groups[g][1]) & 0xFFFFFFFF
+        hi, M, blu, mul, shift, rbias = (int(v) for v in self.groups[g])
         acc = self.tmem[:, col:col + 16].astype(np.int64) + self.bias[boff:boff + 16].astype(np.int64)[None, :]
-        t = np.clip(acc, 0, hi)
-        q = ((t * M) >> 24) & 0xFF
+        if self.k["fast"]:
+            # bias' = b + rbias: t = clamp(acc + bias', 0, blu + rbias), q = byte 3 of t * (mul << (24 - shift))
+            q = ((np.clip(acc, 0, hi) * (M & 0xFFFFFFFF)) >> 24) & 0xFF
+        else:
+            # the reference formula on u = acc + b (mat.cu:286-291): int32 product, arithmetic shift, (char) store
+            p = ((acc + rbias) * mul) & 0xFFFFFFFF
+            p = np.where(p >= 1 << 31, p - (1 << 32), p)
+            q = np.where(acc > blu, 127, np.where(acc < 0, 0, (p >> shift) & 0xFF))
         q = np.where(valid[:, None], q, 0).astype(np.uint8)
         m = np.arange(128)
         self.sm[dst + m[:, None] * 16 + np.arange(16)[None, :]] = q
@@ -212,12 +217,24 @@ def plane_rows(emu, off, row_bytes, R, first_px, nplanes, W):
     return np.concatenate([emu.sm[base + pl * k["PLANE"] + px[:, None] * 16 + np.arange(16)[None, :]] for pl in range(nplanes)], axis=1)
 
 
-@pytest.mark.parametrize("qp,H,W", [(32, 19, 37), (22, 12, 120), (37, 33, 8)])
+EDGE = {e[0]: e[1:] for e in synth.edge_models()}
+CASES = [(32, 19, 37), (22, 12, 120), (37, 33, 8)] + [(mid, 17, 61) for mid in EDGE]
+
+
+def _case_model(qp):
+    if qp in EDGE:
+        return synth.make_edge_model(*EDGE[qp])
+    return synth.make_model(0xC0FFEE + qp, qp)
+
+
+@pytest.mark.parametrize("qp,H,W", CASES)
 def test_kernel_dataflow_on_host_tables_matches_oracle(qp, H, W):
-    rng = np.random.default_rng(1234 + qp)
-    model = synth.make_model(0xC0FFEE + qp, qp)
+    """qp: a calibrated model of that QP, or an edge model (synth.make_edge_model) by its id -- the generic families run the
+    reference-formula requantiser, with the biases the host wrote for it."""
+    rng = np.random.default_rng(1234 + (qp if isinstance(qp, int) else len(qp)))
+    model = _case_model(qp)
     mb = formats.write_model_vect_c(model)
-    img = synth.make_uniform_frames(0xBEEF + qp, 1, H, W)[0]
+    img = synth.make_uniform_frames(0xBEEF + (qp if isinstance(qp, int) else H), 1, H, W)[0]
     rec, a1, a2, a3, _ = oracle.OracleModel(mb).forward_taps(img)
     emu = Emu(mb, rng)
     seen = {"a1": 0, "a2": 0, "a3": 0}
@@ -235,3 +252,22 @@ def test_kernel_dataflow_on_host_tables_matches_oracle(qp, H, W):
     out = emu.run(img, taps)
     assert seen == {"a1": H, "a2": H, "a3": H}
     np.testing.assert_array_equal(out, rec)
+
+
+@pytest.mark.parametrize("mid", [e[0] for e in synth.edge_models()])
+def test_fast_flag_is_all_or_nothing(mid):
+    """qv_debug_fused_tables reports fast == 1 exactly when all five hidden rows pass the fast requantiser's precondition;
+    one failing row sends the whole model to the generic kernels.  The fast path folds rbias into the biases it writes,
+    the generic path writes the layer biases as they are."""
+    model = synth.make_edge_model(*EDGE[mid])
+    k, _, _, groups, bias, _ = fused_tables(formats.write_model_vect_c(model))
+    want = all(synth.fast_row_ok(*q) for q in model.qparams[:5])
+    assert k["fast"] == int(want)
+    layer_of_group = (0, 2, 1, 3, 4)                   # q1, q22, q21, q31, q32 -> C1, C2_2, C2_1, C3_1, C3_2
+    offsets = (0, 64, 80, 112, 128)
+    for g, l in enumerate(layer_of_group):
+        blu, mul, shift = model.qparams[l]
+        rb = (1 << (shift - 1)) // mul
+        assert groups[g][2:].tolist() == [blu, mul, shift, rb]
+        b = model.b[l].astype(np.int64) + (rb if want else 0)
+        assert bias[offsets[g]:offsets[g] + len(b)].tolist() == b.tolist(), l

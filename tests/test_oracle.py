@@ -130,3 +130,18 @@ def test_psnr_matches_reference_formula():
     d = anchor.astype(np.int64) - ori
     assert sse == int((d * d).sum())
     assert p == 10 * np.log10(65025.0 / (sse / anchor.size))
+
+
+@pytest.mark.parametrize("mid,seed,family,variant", synth.edge_models(), ids=[e[0] for e in synth.edge_models()])
+def test_c_oracle_equals_numpy_restatement_on_edge_models(mid, seed, family, variant):
+    """The same cross-check on the corners of the envelope (synth.make_edge_model): -128 taps, channels at exactly
+    128*sum|w| + |b| = 2^24 - 1, rows of every shift, requantiser rows that wrap, C4 rows whose product wraps int32 and
+    whose residual wraps as a short.  Each model is also shown to exercise what its family names."""
+    from oracle import edge_claims
+    m = synth.make_edge_model(seed, family, variant)
+    x = synth.make_uniform_frames(0xED6E + seed, 1, 48, 80)[0]
+    taps = _om(m).forward_taps(x)
+    ref = oracle_np.forward_frame(m, x)
+    for name, got in zip(("rec", "a1", "a2", "a3", "u4"), taps):
+        assert np.array_equal(got, ref[name]), name
+    edge_claims.check_claims(m, seed, family, variant, x, taps)
