@@ -815,16 +815,6 @@ int qv_forward_frames_host(qv_net *net, const uint8_t *h_in, uint8_t *h_out, int
                 }
             }
         }
-        const char *ov = getenv("QV_E2E_CHUNKS");                  // tuning only: explicit chunk sizes, e.g. "4,4,8,16,16,8,4,4"
-        if (ov && *ov) {
-            chunks.clear(); left = n_frames;
-            for (const char *p = ov; *p && left > 0;) {
-                const int c = std::min(std::min(std::max(1, atoi(p)), left), net->batch);
-                chunks.push_back(c); left -= c;
-                while (*p && *p != ',') ++p;
-                if (*p == ',') ++p;
-            }
-        }
         const int uni = std::max(1, std::min(net->batch, (n_frames + 3) / 4));
         while (left > 0) { const int c = std::min(uni, left); chunks.push_back(c); left -= c; }
     }

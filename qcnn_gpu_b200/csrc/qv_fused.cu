@@ -31,8 +31,8 @@
 // and C2_1 shift s-1 read the same a1 tile, C3_1's centre-tap K-steps and C3_2's two K-steps read the same
 // a2 tiles, and the three ring-slot initialisations share the zero tile.
 //
-// Pipeline.  13 warps, three roles; iteration i, R1 = y0-4+i:
-//   warp 8, MMA issue : 27 MMAs per iteration -- C1 for a1 row R1 (im2col operand); the three ring-slot
+// Pipeline.  9 warps, three roles; iteration i, R1 = y0-4+i:
+//   warp 4, MMA issue : 27 MMAs per iteration -- C1 for a1 row R1 (im2col operand); the three ring-slot
 //                initialisations; C3_1 scatter and C3_2 of a2 row R1-6; C2_2 and C2_1 scatter of a1 row R1-2
 //                (the wide MMAs last: they execute slower than they issue, so the tensor pipe still has a
 //                backlog during the handshake).  Both descriptors of every MMA come ready-made from a 12-phase table
@@ -40,11 +40,11 @@
 //                loop executes no ALU-pipe instruction, which matters because the worker warps of the same SM
 //                sub-partition saturate that pipe (profiles/r1_probe3_contention*), and it is this warp's serial
 //                work that bounds the kernel.
-//   warps 0-7, workers: drain what iteration i-1 completed, TMEM -> requantise -> st.shared: a1 row R1-1; a2 row
+//   warps 0-3, workers: drain what iteration i-1 completed, TMEM -> requantise -> st.shared: a1 row R1-1; a2 row
 //                R1-5 plane 2 (C2_2) and a2 row R1-4 planes 0,1 (C2_1); a3 row R1-8 plane 0 (C3_1) and a3 row
-//                R1-7 planes 1,2 (C3_2).  A warp can only read its own TMEM lane quarter, so two warps share a
-//                quarter and split the ten 16-column groups five / five.
-//   warps 9-12, C4    : everything that needs no TMEM -- the input ring (global loads one row ahead), the C1
+//                R1-7 planes 1,2 (C3_2).  A warp can only read its own TMEM lane quarter, so warp q owns quarter q
+//                (pixels 32q .. 32q+31) and drains all ten of its 16-column groups.
+//   warps 5-8, C4     : everything that needs no TMEM -- the input ring (global loads one row ahead), the C1
 //                operand of a1 row R1+1 (im2col, three stages), C4 on a3 row R1-9 (9 LDS.128 + 108 dp4a per
 //                pixel, two running sums carry the partial output rows), applyRes_y and the store of output row
 //                R1-10.
@@ -67,34 +67,18 @@
 #include "qv_tcgen05.cuh"
 
 
-#ifndef QV_EXP
-#define QV_EXP 0
-#endif
 // Code alignment.  The SM's L0 instruction cache works on 128-byte lines (8 instructions) and holds ~6 KB; the three roles' loops
 // are ~13 KB per sub-partition, so every warp keeps refetching, and where the loops start relative to a line boundary is worth
-// up to 2.4 % (profiles/r2_kernel_ab_code_alignment.log: 5.90 ... 6.04 ms for the eight alignments, period 128 bytes).  The
-// shifts below put that many extra instructions (membar.cta, executed once) in front of the code of all roles / the workers and
-// C4 warps / the C4 warps.
+// up to 2.4 % (profiles/r2_kernel_ab_code_alignment.log: 5.90 ... 6.04 ms for the eight alignments, period 128 bytes).
+// QV_CODE_SHIFT puts that many extra instructions (membar.cta, executed once) in front of the code of all roles; re-run the
+// search over its eight values after any edit of the kernel (DESIGN.md section 7).
 #ifndef QV_CODE_SHIFT
 #define QV_CODE_SHIFT 5          // best of the eight positions for this source (profiles/r2_kernel_ab_row_line_decomposition.log)
-#endif
-#ifndef QV_SHIFT_WORK
-#define QV_SHIFT_WORK 0
-#endif
-#ifndef QV_SHIFT_C4
-#define QV_SHIFT_C4 0
-#endif
-#ifndef QV_BULK_WEIGHTS
-#define QV_BULK_WEIGHTS 1        // the weight image goes global -> shared by cp.async.bulk (TMA engine); 0 = per-thread copy loop
-#endif
-#ifndef QV_LIGHT_PROF
-#define QV_LIGHT_PROF 0          // profiling build: 1 = only the timeline of block 0 (no per-MMA stamps, no per-thread counters)
 #endif
 
 namespace qv {
 namespace {
 using namespace tc;
-constexpr int EXP = QV_EXP;   // timing experiments only (tools/build_variants.sh): 1 no a3 requantisation and no C4, 2 no requantiser arithmetic, 4 no im2col
 
 constexpr int WT = 120;                    // output columns per strip
 constexpr int PW = 136;                    // pixel pitch of every activation row buffer
@@ -131,10 +115,7 @@ constexpr int OFF_IN_T = (SMEM_BYTES + 127) / 128 * 128;
 constexpr int SMEM_BYTES_T = OFF_IN_T + IN_SLOTS * IN_PITCH_T;
 static_assert(SMEM_BYTES_T <= 232448, "exceeds the 227 KB of dynamic shared memory per CTA");
 
-#ifndef QV_ONE_WORKER
-#define QV_ONE_WORKER 1          // one worker warp per TMEM lane quarter (ten accumulator groups each); 0 = two (five each), the round-1 arrangement
-#endif
-constexpr int NWORKER = QV_ONE_WORKER ? 128 : 256, NC4 = 128, NTHREADS = NWORKER + 32 + NC4;   // warps 0-7 workers, 8 MMA issue, 9-12 C4
+constexpr int NWORKER = 128, NC4 = 128, NTHREADS = NWORKER + 32 + NC4;   // warps 0-3 workers (one per TMEM lane quarter), 4 MMA issue, 5-8 C4
 constexpr int MMA_WARP = NWORKER / 32;
 constexpr int TR_ITER0 = 300, TR_N = 8;    // profile-mode timeline window
 constexpr int PIPE = 14;                   // pipeline depth in rows: output row y0 appears at iteration 14
@@ -326,8 +307,7 @@ __device__ __forceinline__ void requant_store(const uint32_t (&r)[16], const Fus
                                               uint8_t *dst)
 {
     uint32_t o[4];
-    if (EXP & 2) { o[0] = r[0] & 0x7f7f7f7fu; o[1] = r[5] & 0x7f7f7f7fu; o[2] = r[10] & 0x7f7f7f7fu; o[3] = r[15] & 0x7f7f7f7fu; }
-    else requant<FAST, BOFF>(r, P, g, valid, o);
+    requant<FAST, BOFF>(r, P, g, valid, o);
     *reinterpret_cast<uint4 *>(dst) = make_uint4(o[0], o[1], o[2], o[3]);
 }
 // C4 (48 -> 1, 3x3): the products of one a3 pixel (three 16-channel planes v[pl]) at horizontal tap DX with the three
@@ -466,7 +446,7 @@ struct FusedModel {
     bool fast = true;
     int sm_count = 148;
     // environment switches, read once at upload (never on the per-launch path)
-    bool env_profile = false, env_test_fail = false, env_tma = false, env_linear = true;
+    bool env_profile = false, env_test_fail = false, env_tma = false;
     int env_experiment = 0;
     void *encode_tiled = nullptr;      // cuTensorMapEncodeTiled (driver entry point; the library does not link libcuda)
 };
@@ -670,7 +650,6 @@ FusedModel *fused_upload(const ModelHost &m, cudaStream_t st)
     fm->env_experiment = getenv("QV_FUSED_EXPERIMENT") ? atoi(getenv("QV_FUSED_EXPERIMENT")) : 0;
     fm->env_test_fail = getenv("QV_FUSED_TEST_FAIL") != nullptr;     // tests only: make every CTA report a base mismatch
     fm->env_tma = getenv("QV_FUSED_TMA") != nullptr && atoi(getenv("QV_FUSED_TMA")) != 0;
-    fm->env_linear = !(getenv("QV_FUSED_LINEAR") && atoi(getenv("QV_FUSED_LINEAR")) == 0);      // A/B switch: 0 = equal row segments only
     if (fm->env_tma) {
         cudaDriverEntryPointQueryResult qr;
         if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fm->encode_tiled, cudaEnableDefault, &qr) != cudaSuccess || qr != cudaDriverEntryPointSuccess)
@@ -832,7 +811,7 @@ cudaError_t fused_forward(const FusedModel *fm, const uint8_t *d_in, uint8_t *d_
         P.pub = rows->pub; P.done = rows->done; P.done_ctr = rows->done_ctr; P.seq = rows->seq;
     }
     int grid = 1;
-    if (const cudaError_t e = plan_units(P, fm->sm_count, fm->env_linear, rows != nullptr, grid)) return e;
+    if (const cudaError_t e = plan_units(P, fm->sm_count, true, rows != nullptr, grid)) return e;
     const bool prof = fm->env_profile;
     P.dbg = nullptr;
     P.dbg_flags = fm->env_experiment;
@@ -884,7 +863,7 @@ cudaError_t fused_forward(const FusedModel *fm, const uint8_t *d_in, uint8_t *d_
         if (t0)
             for (int k = 0; k < TR_N; ++k, tr += 16)
                 fprintf(stderr, "[qv fused trace] it %d | mma: start %lld end %lld | w0: commit %lld drained %lld arrived %lld bar %lld | "
-                        "w4: commit %lld drained %lld arrived %lld bar %lld\n", TR_ITER0 + k, tr[0] - t0, tr[1] - t0, tr[2] - t0, tr[3] - t0,
+                        "w2: commit %lld drained %lld arrived %lld bar %lld\n", TR_ITER0 + k, tr[0] - t0, tr[1] - t0, tr[2] - t0, tr[3] - t0,
                         tr[4] - t0, tr[5] - t0, tr[6] - t0, tr[7] - t0, tr[8] - t0, tr[9] - t0);
         tr = h.data() + (size_t)grid * 16;
         if (t0)

@@ -1,4 +1,4 @@
-# builds tools/bin/lib_<name>.so for each "name:flags" argument, e.g.  tools/build_variants.sh "a:-DQV_C4_LATE=0" "b:-DQV_C4_LATE=1"
+# builds tools/bin/lib_<name>.so for each "name:flags" argument, e.g.  tools/build_variants.sh "s4:-DQV_CODE_SHIFT=4" "s5:-DQV_CODE_SHIFT=5"
 set -e
 cd "$(dirname "$0")/../qcnn_gpu_b200/csrc"
 mkdir -p ../../tools/bin
