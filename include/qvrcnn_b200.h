@@ -191,6 +191,30 @@ QV_API int qv_strip_forward(qv_net *net, int slot, uint8_t *d_out, void *cuda_st
    Null d_ori_rows / d_sse2: QV_ERR_ARG; not the fused path: QV_ERR_STATE, as qv_strip_forward. */
 QV_API int qv_strip_forward_sse(qv_net *net, int slot, const uint8_t *d_ori_rows, uint8_t *d_out, int64_t *d_sse2,
                                 void *cuda_stream);
+/* qv_stream_yuv_pf through the strip partition: frames [first_frame, first_frame + n_frames) of a YUV 4:2:0 sequence,
+   enhanced by the strip handles of THIS process (set up, exported and attached; on one device or several).  Each handle
+   reads only its own rows of each frame from the anchor (and original) file with pread -- luma row r of frame f at byte
+   f*H*W*3/2 + r*W -- and writes its rows of the reconstruction at the same offsets with pwrite; the handle that owns the
+   last image row also writes the frame's H*W/2 zero bytes of chroma (save_recon_as' layout).  recon_yuv is opened like
+   qv_stream_yuv's (created if missing, never truncated): frames outside the range and other processes' rows are left as
+   they are.  A reader thread keeps one frame ahead and a writer thread one frame behind, over a ring of three page-locked
+   slots per strip; one GPU thread per device drives that device's strips (one strip: two streams, upload of frame k+1
+   overlapping the compute of frame k; several strips: one stream, all loads of a frame before its forwards).  Host and
+   device memory are O(strip rows x W), whatever n_frames is.  The call waits for the devices of `nets` to be idle before it
+   starts and leaves the handles idle, free to be driven on any stream.
+   With ori_yuv, sse_before_pf[j] / sse_after_pf[j] are the SSEs of the anchor / the reconstruction against the original
+   over this call's rows of frame first_frame + j (qv_strip_forward_sse per strip); with every strip of the frame in one call
+   they are the frame's, as qv_stream_yuv_pf returns them, and across processes the caller adds them up.  Either may be NULL.
+   Every process that holds strips of the frame must make the same call (same first_frame and n_frames): the strips' handles
+   must see the same sequence of forwards.  Checked before any file is opened: QV_ERR_ARG for null or empty nets, a handle
+   given twice, handles of different widths or image heights, a negative first_frame / n_frames, an SSE pointer without
+   ori_yuv, or with ori_yuv an image taller than 66051 rows; QV_ERR_STATE for a handle without qv_strip_setup, without a
+   neighbour on an interior edge or without the fused path, and for a device that also holds a strip handle of this process
+   that is not in nets (strips that share a GPU are driven together).  QV_ERR_IO: open failure, short read, failed write.
+   QV_ERR_CUDA: a CUDA call failed or a CTA reported a failure.  n_frames == 0: QV_OK, no file touched. */
+QV_API int qv_strip_stream_yuv_pf(qv_net *const *nets, int n_nets, const char *anchor_yuv, const char *ori_yuv,
+                                  const char *recon_yuv, int first_frame, int n_frames,
+                                  int64_t *sse_before_pf, int64_t *sse_after_pf);
 /* Unmaps the neighbours and frees the block (all GPUs must be idle). */
 QV_API int qv_strip_release(qv_net *net);
 

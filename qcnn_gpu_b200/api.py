@@ -33,7 +33,7 @@ ABI_SYMBOLS = (
     "qv_psnr", "qv_psnr_from_sse", "qv_solve_quant_params", "qv_write_quant_params_cpp", "qv_quantize_layer",
     "qv_debug_fused_tables", "qv_debug_fused_units", "qv_synchronize",
     "qv_strip_setup", "qv_strip_export", "qv_strip_attach", "qv_strip_input", "qv_strip_acquire", "qv_strip_load",
-    "qv_strip_forward", "qv_strip_forward_sse", "qv_strip_release",
+    "qv_strip_forward", "qv_strip_forward_sse", "qv_strip_stream_yuv_pf", "qv_strip_release",
 )
 
 CUDA_STREAM_LEGACY = 1      # cudaStreamLegacy: names the legacy default stream explicitly (NULL = "the handle's own stream")
@@ -115,6 +115,7 @@ def lib():
         L.qv_strip_load.argtypes = [vp, i32, vp, vp]
         L.qv_strip_forward.argtypes = [vp, i32, vp, vp]
         L.qv_strip_forward_sse.argtypes = [vp, i32, vp, vp, vp, vp]
+        L.qv_strip_stream_yuv_pf.argtypes = [C.POINTER(vp), i32, cp, cp, cp, i32, i32, vp, vp]
         L.qv_strip_release.argtypes = [vp]
         _lib = L
     return _lib
@@ -287,6 +288,20 @@ class QVRCNN:
         out = np.empty((64 if which == 1 else 48, self.height, self.width), np.int8)
         _check(lib().qv_get_activation(self._h, which, out.ctypes.data))
         return out
+
+
+def strip_stream_yuv_pf(nets, anchor_yuv: str, ori_yuv: Optional[str], recon_yuv: Optional[str], first_frame: int, n_frames: int):
+    """qv_strip_stream_yuv_pf: frames [first_frame, first_frame + n_frames) of the anchor file through the strip handles `nets`
+    (QVRCNN objects after strip_setup / strip_export / strip_attach), each reading and writing only its own rows.  Returns
+    (sse_before, sse_after), two np.int64 arrays of n_frames: the SSEs over these handles' rows of each frame (zeros without
+    `ori_yuv`)."""
+    before = np.zeros(max(n_frames, 0), np.int64)
+    after = np.zeros(max(n_frames, 0), np.int64)
+    handles = (C.c_void_p * len(nets))(*[n._h.value for n in nets])
+    enc = lambda p: os.fsencode(p) if p else None
+    _check(lib().qv_strip_stream_yuv_pf(handles, len(nets), enc(anchor_yuv), enc(ori_yuv), enc(recon_yuv), first_frame, n_frames,
+                                        before.ctypes.data if ori_yuv else None, after.ctypes.data if ori_yuv else None))
+    return before, after
 
 
 def sse_device(d_a: int, d_b: int, n: int, d_accum: int, stream: int = 0) -> None:
