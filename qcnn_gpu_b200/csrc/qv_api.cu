@@ -108,6 +108,9 @@ struct qv_net {
 
 static int set_device(const qv_net *net) { QV_CUDA(cudaSetDevice(net->dev)); return QV_OK; }
 
+// Does this handle run the fused kernel?  QV_IMPL_AUTO picks it whenever it is built.
+static bool runs_fused(const qv_net *net) { return net->impl == QV_IMPL_FUSED || (net->impl == QV_IMPL_AUTO && net->fm); }
+
 static void free_layered(qv_net *net)
 {
     for (int l = 0; l < QV_NLAYER; ++l) {
@@ -230,9 +233,7 @@ static int run_forward(qv_net *net, const uint8_t *d_in, uint8_t *d_out, int n, 
         set_error("forward called before a complete model (weights + quant params) was loaded");
         return QV_ERR_STATE;
     }
-    int impl = net->impl;
-    if (impl == QV_IMPL_AUTO) impl = net->fm ? QV_IMPL_FUSED : QV_IMPL_LAYERED;
-    if (impl == QV_IMPL_FUSED) {
+    if (runs_fused(net)) {
         if (!net->fm) { set_error("fused tcgen05 path is not available in this build"); return QV_ERR_STATE; }
         if (d_sse && H > FUSED_SSE_MAX_H) { set_error("per-frame SSE: frame height %d exceeds %d", H, FUSED_SSE_MAX_H); return QV_ERR_ARG; }
         QV_CUDA(fused_forward(net->fm, d_in, d_out, n, H, W, st, &net->launches, nullptr, d_ori, d_sse));
@@ -503,8 +504,7 @@ int qv_forward_rows_device(qv_net *net, const uint8_t *d_in, int img_height, int
     if (rc) return rc;
     cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : net->st;
     const size_t W = net->W;
-    const bool fused_path = net->impl == QV_IMPL_FUSED || (net->impl == QV_IMPL_AUTO && net->fm);
-    if (fused_path) {
+    if (runs_fused(net)) {
         // the fused kernel takes the window as what it is: rows [in_row0, in_row1) of an img_height-row image, of which it
         // computes and writes exactly [out_row0, out_row1) -- no scratch frame, no copy
         if (!net->uploaded || !net->fm) { set_error("forward called before a complete model (weights + quant params) was loaded"); return QV_ERR_STATE; }
@@ -866,8 +866,7 @@ int qv_forward_frames_host(qv_net *net, const uint8_t *h_in, uint8_t *h_out, int
         // The layered path's compute stages must run one after the other (they share the handle's activation scratch).
         // The fused kernel has no scratch: its launches of the two slots are left unordered, so the persistent CTAs of the
         // next chunk move onto the SMs the previous chunk's last wave has already left.
-        const bool fused_path = net->impl == QV_IMPL_FUSED || (net->impl == QV_IMPL_AUTO && net->fm);
-        if (f0 > 0 && !fused_path) QV_CUDA(cudaStreamWaitEvent(net->pst[slot], net->ev_compute, 0));
+        if (f0 > 0 && !runs_fused(net)) QV_CUDA(cudaStreamWaitEvent(net->pst[slot], net->ev_compute, 0));
         rc = run_forward(net, net->d_slot_in[slot], net->d_slot_out[slot], c, net->H, net->W, net->pst[slot]);
         if (rc) return rc;
         QV_CUDA(cudaEventRecord(net->ev_compute, net->pst[slot]));
@@ -881,28 +880,9 @@ int qv_forward_frames_host(qv_net *net, const uint8_t *h_in, uint8_t *h_out, int
 }
 
 // ---- streaming file pipeline (SURVEY 8 f2) -------------------------------------------------------------
+}  // extern "C"
+
 namespace {
-struct StreamSlot {
-    uint8_t *h_in = nullptr, *h_ori = nullptr, *h_out = nullptr;      // pinned
-    uint8_t *d_in = nullptr, *d_ori = nullptr, *d_out = nullptr;
-    cudaStream_t st = nullptr;
-    cudaEvent_t done = nullptr;
-    int state = 0;                       // 0 free -> 1 filled by the reader -> 2 launched -> 0 (written)
-    int f0 = 0, c = 0;
-};
-struct StreamShared {
-    std::mutex mu;
-    std::condition_variable cv;
-    bool failed = false;
-    int rc = QV_OK;                      // the QV_ERR_* code of the first failure
-    char msg[256] = {0};
-    void fail(int code, const char *m)
-    {
-        std::lock_guard<std::mutex> l(mu);
-        if (!failed) { failed = true; rc = code; snprintf(msg, sizeof(msg), "%s", m); }
-        cv.notify_all();
-    }
-};
 // The files of one streaming call (-1: not given).  The reconstruction is opened without truncation and created if missing:
 // several ranks / threads may fill one file, each its own frame range or rows (a caller that lost the race to create it
 // must not wipe what another has written).
@@ -958,7 +938,164 @@ bool write_recon_rows(int fd, long long frame, int img_h, int w, int row0, int r
     return pwrite_all(fd, src, (size_t)(row1 - row0) * w, luma_offset(frame, img_h, w, row0)) &&
            (row1 < img_h || pwrite_all(fd, zeros, (size_t)img_h * w / 2, luma_offset(frame, img_h, w, img_h)));
 }
+
+// What one streaming call holds on one device: streams, events, device and page-locked memory.  The destructor, which also
+// runs on every early return, makes the streams idle before it frees anything they may still read or write.
+struct DeviceHold {
+    int dev = 0;
+    std::vector<cudaStream_t> streams;
+    std::vector<cudaEvent_t> events;
+    std::vector<void *> mem, pinned;
+    DeviceHold() = default;
+    DeviceHold(const DeviceHold &) = delete;
+    DeviceHold &operator=(const DeviceHold &) = delete;
+    ~DeviceHold()
+    {
+        cudaSetDevice(dev);
+        idle();
+        for (cudaStream_t s : streams) cudaStreamDestroy(s);
+        for (cudaEvent_t e : events) cudaEventDestroy(e);
+        for (void *p : mem) cudaFree(p);
+        for (void *p : pinned) cudaFreeHost(p);
+    }
+    void idle() { for (cudaStream_t s : streams) cudaStreamSynchronize(s); }
+    cudaError_t stream(cudaStream_t *s)
+    {
+        const cudaError_t e = cudaStreamCreateWithFlags(s, cudaStreamNonBlocking);
+        if (e == cudaSuccess) streams.push_back(*s);
+        return e;
+    }
+    cudaError_t event(cudaEvent_t *ev)
+    {
+        const cudaError_t e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
+        if (e == cudaSuccess) events.push_back(*ev);
+        return e;
+    }
+    template <class T> cudaError_t alloc(T **p, size_t bytes)
+    {
+        const cudaError_t e = cudaMalloc(p, bytes);
+        if (e == cudaSuccess) mem.push_back(*p);
+        return e;
+    }
+};
+
+constexpr int RING_NS = 3;                       // ring entries: one being read, one on the GPU, one being written
+// One handle's band of a streaming call: rows [row0, row1) of every frame, on the device of hold[hold].
+struct RingPart {
+    int hold = 0, row0 = 0, row1 = 0;
+    uint8_t *h_in[RING_NS] = {}, *h_ori[RING_NS] = {}, *h_out[RING_NS] = {};   // page-locked, c_max frames of the band each
+    cudaEvent_t done[RING_NS] = {};             // recorded by the GPU stage once the rows of ring entry r are downloaded
+};
+// The GPU stage of device hold[d] for item k (frames [first_frame + f0, first_frame + f0 + c)) in ring entry r: uploads h_in
+// (h_ori) of its parts, runs the forward, downloads h_out and records done[r] of every part.  Returns a QV_ERR_* code.
+using RingLaunch = std::function<int(int d, int k, int f0, int c, int r)>;
+
+// The pipeline behind qv_stream_yuv_pf and qv_strip_stream_yuv_pf.  Frames [first_frame, first_frame + n_frames) pass in items
+// of up to c_max frames, item k through ring entry k % RING_NS of every part: a reader thread reads the parts' rows of the
+// item's frames from the anchor (and original) file, one thread per device of `hold` calls `launch`, and a writer thread
+// waits for every part's done event and writes its rows to the reconstruction file.  An entry goes free -> read -> launched
+// on every device -> free, so the reader is at most one entry ahead of the GPU stage and the writer one behind.  The first
+// failure of any stage wakes them all; its code is returned and its message set on the calling thread.  The ring is
+// allocated in `hold`, which frees it once the streams of the GPU stage are idle.
+int stream_ring(const char *who, const StreamFiles &F, int img_h, int W, int first_frame, int n_frames, int c_max,
+                std::vector<RingPart> &parts, std::vector<DeviceHold> &hold, const RingLaunch &launch)
+{
+    const bool with_ori = F.ori >= 0;
+    for (RingPart &P : parts) {
+        DeviceHold &H = hold[P.hold];
+        QV_CUDA(cudaSetDevice(H.dev));
+        const size_t bytes = (size_t)c_max * (P.row1 - P.row0) * W;
+        for (int r = 0; r < RING_NS; ++r) {
+            for (uint8_t **p : {&P.h_in[r], &P.h_out[r], with_ori ? &P.h_ori[r] : nullptr})
+                if (p) { QV_CUDA(cudaMallocHost(p, bytes)); H.pinned.push_back(*p); }
+            QV_CUDA(H.event(&P.done[r]));
+        }
+    }
+
+    enum { FREE, READ, LAUNCHED };
+    struct Entry { int item = -1, state = FREE, launched = 0; } ring[RING_NS];
+    std::mutex mu;
+    std::condition_variable cv;
+    bool failed = false;
+    int fail_rc = QV_OK;
+    std::string fail_msg;
+    auto fail = [&](int code, const std::string &msg) {
+        std::lock_guard<std::mutex> l(mu);
+        if (!failed) { failed = true; fail_rc = code; fail_msg = msg; }
+        cv.notify_all();
+    };
+    // Waits until entry E holds item k in `state` (a free entry: any item); false once a stage has failed.
+    auto wait = [&](const Entry &E, int state, int k) {
+        std::unique_lock<std::mutex> l(mu);
+        cv.wait(l, [&] { return (E.state == state && (state == FREE || E.item == k)) || failed; });
+        return !failed;
+    };
+    const int items = (n_frames + c_max - 1) / c_max;
+    auto frames = [&](int k) { return std::min(c_max, n_frames - k * c_max); };
+    auto band = [&](const RingPart &P) { return (size_t)(P.row1 - P.row0) * W; };
+
+    std::thread reader([&] {
+        for (int k = 0; k < items; ++k) {
+            Entry &E = ring[k % RING_NS];
+            if (!wait(E, FREE, k)) return;
+            for (RingPart &P : parts)
+                for (int j = 0; j < frames(k); ++j) {
+                    const long long f = (long long)first_frame + k * c_max + j;
+                    if (!read_luma(F.anchor, f, img_h, W, P.row0, P.row1, P.h_in[k % RING_NS] + j * band(P)) ||
+                        (with_ori && !read_luma(F.ori, f, img_h, W, P.row0, P.row1, P.h_ori[k % RING_NS] + j * band(P)))) {
+                        fail(QV_ERR_IO, std::string(who) + ": short read (file smaller than the requested frame range)");
+                        return;
+                    }
+                }
+            { std::lock_guard<std::mutex> l(mu); E.item = k; E.state = READ; }
+            cv.notify_all();
+        }
+    });
+    std::thread writer([&] {
+        const std::vector<uint8_t> zeros((size_t)img_h * W / 2, 0);
+        for (int k = 0; k < items; ++k) {
+            Entry &E = ring[k % RING_NS];
+            if (!wait(E, LAUNCHED, k)) return;
+            for (const RingPart &P : parts) {
+                if (cudaSetDevice(hold[P.hold].dev) != cudaSuccess || cudaEventSynchronize(P.done[k % RING_NS]) != cudaSuccess) {
+                    fail(QV_ERR_CUDA, std::string(who) + ": the GPU stage failed");
+                    return;
+                }
+                for (int j = 0; F.recon >= 0 && j < frames(k); ++j)
+                    if (!write_recon_rows(F.recon, (long long)first_frame + k * c_max + j, img_h, W, P.row0, P.row1,
+                                          P.h_out[k % RING_NS] + j * band(P), zeros.data())) {
+                        fail(QV_ERR_IO, std::string(who) + ": write to the reconstruction file failed");
+                        return;
+                    }
+            }
+            { std::lock_guard<std::mutex> l(mu); E.state = FREE; E.launched = 0; }
+            cv.notify_all();
+        }
+    });
+    auto gpu = [&](int d) {
+        int rc = QV_OK;
+        if (cudaSetDevice(hold[d].dev) != cudaSuccess) { set_error("cudaSetDevice(%d) failed", hold[d].dev); rc = QV_ERR_CUDA; }
+        for (int k = 0; k < items && rc == QV_OK; ++k) {
+            Entry &E = ring[k % RING_NS];
+            if (!wait(E, READ, k)) return;
+            if ((rc = launch(d, k, k * c_max, frames(k), k % RING_NS))) break;
+            { std::lock_guard<std::mutex> l(mu); if (++E.launched == (int)hold.size()) E.state = LAUNCHED; }
+            cv.notify_all();
+        }
+        if (rc) fail(rc, "GPU " + std::to_string(hold[d].dev) + ": " + get_error());   // the message is thread-local
+    };
+    std::vector<std::thread> gpus;
+    for (size_t d = 0; d < hold.size(); ++d) gpus.emplace_back(gpu, (int)d);
+    for (std::thread &t : gpus) t.join();
+    reader.join();
+    writer.join();
+    if (!failed) return QV_OK;
+    set_error("%s", fail_msg.c_str());
+    return fail_rc;
+}
 }  // namespace
+
+extern "C" {
 
 // Per-frame SSEs of the anchor and of the reconstruction against the original (vrcnn_data::psnr_pf, inference/yuv_data.cpp:98-112)
 // for frames [first_frame, first_frame + n_frames): they are computed with the reconstruction (in the fused kernel, or per frame
@@ -975,129 +1112,52 @@ int qv_stream_yuv_pf(qv_net *net, const char *anchor_yuv, const char *ori_yuv, c
         if (sse_after_pf) sse_after_pf[j] = 0;
     }
     if (n_frames == 0) return QV_OK;
-    const size_t fpx = (size_t)net->H * net->W;
-    const int C = net->batch, NS = 3;
     StreamFiles F;
     if ((rc = F.open_all(anchor_yuv, ori_yuv, recon_yuv))) return rc;
-    const bool with_ori = F.ori >= 0;
-    StreamSlot slot[3];
-    StreamShared sh;
+    const bool with_ori = F.ori >= 0, fused_path = runs_fused(net);
+    const size_t fpx = (size_t)net->H * net->W, cbytes = (size_t)net->batch * fpx;
+    std::vector<DeviceHold> hold(1);
+    DeviceHold &H = hold[0];
+    H.dev = net->dev;
+    // one whole-frame part; per ring entry, device buffers of a chunk and a stream for its H2D -> forward -> D2H chain
+    std::vector<RingPart> parts(1);
+    parts[0].row1 = net->H;
+    const RingPart &P = parts[0];
+    struct { uint8_t *d_in = nullptr, *d_ori = nullptr, *d_out = nullptr; cudaStream_t st = nullptr; } slot[RING_NS];
+    for (auto &S : slot) {
+        QV_CUDA(H.alloc(&S.d_in, cbytes));
+        QV_CUDA(H.alloc(&S.d_out, cbytes));
+        if (with_ori) QV_CUDA(H.alloc(&S.d_ori, cbytes));
+        QV_CUDA(H.stream(&S.st));
+    }
     int64_t *d_sse = nullptr;                                   // [n_frames][2]
     const size_t sse_bytes = (size_t)n_frames * 2 * sizeof(int64_t);
-    cudaError_t e = cudaMalloc(&d_sse, sse_bytes);
-    if (e == cudaSuccess) e = cudaMemset(d_sse, 0, sse_bytes);
-    for (int s = 0; s < NS && e == cudaSuccess; ++s) {
-        StreamSlot &S = slot[s];
-        e = cudaMallocHost(&S.h_in, C * fpx);
-        if (e == cudaSuccess) e = cudaMallocHost(&S.h_out, C * fpx);
-        if (e == cudaSuccess && with_ori) e = cudaMallocHost(&S.h_ori, C * fpx);
-        if (e == cudaSuccess) e = cudaMalloc(&S.d_in, C * fpx);
-        if (e == cudaSuccess) e = cudaMalloc(&S.d_out, C * fpx);
-        if (e == cudaSuccess && with_ori) e = cudaMalloc(&S.d_ori, C * fpx);
-        if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&S.st, cudaStreamNonBlocking);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&S.done, cudaEventDisableTiming);
-    }
-    const int nchunk = (n_frames + C - 1) / C;
-    auto cleanup = [&]() {
-        for (int s = 0; s < NS; ++s) {
-            StreamSlot &S = slot[s];
-            if (S.st) cudaStreamSynchronize(S.st);
-            cudaFreeHost(S.h_in); cudaFreeHost(S.h_out); cudaFreeHost(S.h_ori);
-            cudaFree(S.d_in); cudaFree(S.d_out); cudaFree(S.d_ori);
-            if (S.done) cudaEventDestroy(S.done);
-            if (S.st) cudaStreamDestroy(S.st);
-        }
-        cudaFree(d_sse);
-    };
-    if (e != cudaSuccess) { cleanup(); set_error("qv_stream_yuv: %s", cudaGetErrorString(e)); return QV_ERR_CUDA; }
+    QV_CUDA(H.alloc(&d_sse, sse_bytes));
+    QV_CUDA(cudaMemset(d_sse, 0, sse_bytes));
+    cudaEvent_t ev_compute = nullptr;        // the layered path's launches share the handle's activation scratch: keep them in order
+    if (!fused_path) QV_CUDA(H.event(&ev_compute));
 
-    // reader: files -> pinned memory, one chunk ahead of the GPU
-    std::thread reader([&] {
-        for (int k = 0; k < nchunk; ++k) {
-            StreamSlot &S = slot[k % NS];
-            {
-                std::unique_lock<std::mutex> l(sh.mu);
-                sh.cv.wait(l, [&] { return S.state == 0 || sh.failed; });
-                if (sh.failed) return;
-            }
-            const int f0 = k * C, c = std::min(C, n_frames - f0);
-            for (int j = 0; j < c; ++j) {
-                const long long f = (long long)first_frame + f0 + j;
-                if (!read_luma(F.anchor, f, net->H, net->W, 0, net->H, S.h_in + (size_t)j * fpx) ||
-                    (with_ori && !read_luma(F.ori, f, net->H, net->W, 0, net->H, S.h_ori + (size_t)j * fpx))) {
-                    sh.fail(QV_ERR_IO, "qv_stream_yuv: short read (file smaller than the requested frame range)");
-                    return;
-                }
-            }
-            { std::lock_guard<std::mutex> l(sh.mu); S.f0 = f0; S.c = c; S.state = 1; }
-            sh.cv.notify_all();
-        }
+    rc = stream_ring("qv_stream_yuv_pf", F, net->H, net->W, first_frame, n_frames, net->batch, parts, hold,
+                     [&](int, int k, int f0, int c, int r) -> int {
+        const auto &S = slot[r];
+        const size_t bytes = (size_t)c * fpx;
+        QV_CUDA(cudaMemcpyAsync(S.d_in, P.h_in[r], bytes, cudaMemcpyHostToDevice, S.st));
+        if (with_ori) QV_CUDA(cudaMemcpyAsync(S.d_ori, P.h_ori[r], bytes, cudaMemcpyHostToDevice, S.st));
+        if (!fused_path && k > 0) QV_CUDA(cudaStreamWaitEvent(S.st, ev_compute, 0));
+        const int frc = run_forward(net, S.d_in, S.d_out, c, net->H, net->W, S.st, S.d_ori, with_ori ? d_sse + 2 * (size_t)f0 : nullptr);
+        if (frc) return frc;
+        if (!fused_path) QV_CUDA(cudaEventRecord(ev_compute, S.st));
+        QV_CUDA(cudaMemcpyAsync(P.h_out[r], S.d_out, bytes, cudaMemcpyDeviceToHost, S.st));
+        QV_CUDA(cudaEventRecord(P.done[r], S.st));
+        return QV_OK;
     });
-    // writer: pinned memory -> recon file, one chunk behind the GPU
-    const int dev = net->dev;
-    std::thread writer([&] {
-        cudaSetDevice(dev);
-        std::vector<uint8_t> zeros(fpx / 2, 0);
-        for (int k = 0; k < nchunk; ++k) {
-            StreamSlot &S = slot[k % NS];
-            {
-                std::unique_lock<std::mutex> l(sh.mu);
-                sh.cv.wait(l, [&] { return S.state == 2 || sh.failed; });
-                if (sh.failed) return;
-            }
-            if (cudaEventSynchronize(S.done) != cudaSuccess) { sh.fail(QV_ERR_CUDA, "qv_stream_yuv: the GPU stage failed"); return; }
-            bool ok = true;
-            for (int j = 0; F.recon >= 0 && j < S.c && ok; ++j)
-                ok = write_recon_rows(F.recon, (long long)first_frame + S.f0 + j, net->H, net->W, 0, net->H, S.h_out + (size_t)j * fpx, zeros.data());
-            if (!ok) { sh.fail(QV_ERR_IO, "qv_stream_yuv: write to the reconstruction file failed"); return; }
-            { std::lock_guard<std::mutex> l(sh.mu); S.state = 0; }
-            sh.cv.notify_all();
-        }
-    });
-    // GPU stage, in chunk order
-    const bool fused_path = net->impl == QV_IMPL_FUSED || (net->impl == QV_IMPL_AUTO && net->fm);
-    cudaEvent_t ev_compute = nullptr;
-    if (!fused_path && cudaEventCreateWithFlags(&ev_compute, cudaEventDisableTiming) != cudaSuccess) {
-        sh.fail(QV_ERR_CUDA, "qv_stream_yuv: the GPU stage failed");
-        rc = QV_ERR_CUDA;
-    }
-    for (int k = 0; k < nchunk && rc == QV_OK; ++k) {
-        StreamSlot &S = slot[k % NS];
-        {
-            std::unique_lock<std::mutex> l(sh.mu);
-            sh.cv.wait(l, [&] { return S.state == 1 || sh.failed; });
-            if (sh.failed) break;
-        }
-        const size_t bytes = (size_t)S.c * fpx;
-        e = cudaMemcpyAsync(S.d_in, S.h_in, bytes, cudaMemcpyHostToDevice, S.st);
-        if (e == cudaSuccess && with_ori) e = cudaMemcpyAsync(S.d_ori, S.h_ori, bytes, cudaMemcpyHostToDevice, S.st);
-        // the layered path's launches share the handle's activation scratch: keep them in order across the slots' streams
-        if (e == cudaSuccess && !fused_path && k > 0) e = cudaStreamWaitEvent(S.st, ev_compute, 0);
-        if (e == cudaSuccess) {
-            rc = run_forward(net, S.d_in, S.d_out, S.c, net->H, net->W, S.st, with_ori ? S.d_ori : nullptr, with_ori ? d_sse + 2 * (size_t)S.f0 : nullptr);
-            if (rc == QV_OK && !fused_path) e = cudaEventRecord(ev_compute, S.st);
-        }
-        if (e == cudaSuccess && rc == QV_OK) e = cudaMemcpyAsync(S.h_out, S.d_out, bytes, cudaMemcpyDeviceToHost, S.st);
-        if (e == cudaSuccess && rc == QV_OK) e = cudaEventRecord(S.done, S.st);
-        if (e != cudaSuccess) { set_error("qv_stream_yuv: %s", cudaGetErrorString(e)); rc = QV_ERR_CUDA; }
-        if (rc != QV_OK) { sh.fail(rc, "qv_stream_yuv: the GPU stage failed"); break; }
-        { std::lock_guard<std::mutex> l(sh.mu); S.state = 2; }
-        sh.cv.notify_all();
-    }
-    reader.join();
-    writer.join();
-    if (ev_compute) { for (int s = 0; s < NS; ++s) cudaStreamSynchronize(slot[s].st); cudaEventDestroy(ev_compute); }
+    if (rc) return rc;
+    H.idle();
     std::vector<int64_t> h_sse(with_ori ? (size_t)n_frames * 2 : 0);
-    if (rc == QV_OK && !sh.failed) {
-        for (int s = 0; s < NS; ++s) cudaStreamSynchronize(slot[s].st);
-        if (with_ori && cudaMemcpy(h_sse.data(), d_sse, sse_bytes, cudaMemcpyDeviceToHost) != cudaSuccess) {
-            set_error("qv_stream_yuv_pf: copy of the SSEs failed");
-            rc = QV_ERR_CUDA;
-        }
+    if (with_ori && cudaMemcpy(h_sse.data(), d_sse, sse_bytes, cudaMemcpyDeviceToHost) != cudaSuccess) {
+        set_error("qv_stream_yuv_pf: copy of the SSEs failed");
+        return QV_ERR_CUDA;
     }
-    cleanup();
-    if (rc == QV_OK && sh.failed) { set_error("%s", sh.msg); rc = sh.rc; }
-    if (rc != QV_OK) return rc;
     for (int j = 0; with_ori && j < n_frames; ++j) {
         if (sse_before_pf) sse_before_pf[j] = h_sse[2 * (size_t)j];
         if (sse_after_pf) sse_after_pf[j] = h_sse[2 * (size_t)j + 1];
@@ -1124,11 +1184,10 @@ int qv_stream_yuv(qv_net *net, const char *anchor_yuv, const char *ori_yuv, cons
     return QV_OK;
 }
 
-// qv_stream_yuv_pf through the strip partition.  Per frame k every strip's rows pass through ring entry k % NS of page-locked
-// buffers (reader thread: anchor / original rows in; writer thread: reconstruction rows out) and through the strip's input
-// slot k & 1 on the GPU.  One GPU thread per device drives that device's strips the way qcnn_gpu --strips does: a device with
-// one strip alternates two streams and an event keeps the forwards in frame order; a device with several strips drives them
-// all on one stream, all loads of a frame before its forwards.
+// qv_stream_yuv_pf through the strip partition, on the same ring: one part per strip handle (its own rows of each frame), one
+// frame per ring entry, and per frame k the strip's input slot k & 1 on the GPU.  The GPU stage of a device drives its strips
+// the way qcnn_gpu --strips does: a device with one strip alternates two streams and an event keeps the forwards in frame
+// order; a device with several strips drives them all on one stream, all loads of a frame before its forwards.
 int qv_strip_stream_yuv_pf(qv_net *const *nets, int n_nets, const char *anchor_yuv, const char *ori_yuv, const char *recon_yuv,
                            int first_frame, int n_frames, int64_t *sse_before_pf, int64_t *sse_after_pf)
 {
@@ -1170,198 +1229,98 @@ int qv_strip_stream_yuv_pf(qv_net *const *nets, int n_nets, const char *anchor_y
     if ((rc = F.open_all(anchor_yuv, ori_yuv, recon_yuv))) return rc;
     const bool with_ori = F.ori >= 0;
 
-    constexpr int NS = 3;
-    struct StripIO {
-        qv_net *net = nullptr;
-        size_t bytes = 0;                                           // (row1 - row0) * W
-        uint8_t *h_in[NS] = {}, *h_ori[NS] = {}, *h_out[NS] = {};   // pinned ring
-        uint8_t *d_ori[2] = {}, *d_out[2] = {};                     // per input slot
-        int64_t *d_sse = nullptr;                                   // [n_frames][2]
-        cudaEvent_t done[NS] = {};                                  // rows of ring entry r downloaded
-    };
-    struct DeviceIO {
-        int dev = 0;
+    // the devices in order of first use; per device its strips, and per strip its part of the ring
+    std::vector<int> devices;
+    std::vector<RingPart> parts(n_nets);
+    for (int i = 0; i < n_nets; ++i) {
+        auto d = std::find(devices.begin(), devices.end(), nets[i]->dev);
+        parts[i].hold = (int)(d - devices.begin());
+        if (d == devices.end()) devices.push_back(nets[i]->dev);
+        parts[i].row0 = nets[i]->strip.row0;
+        parts[i].row1 = nets[i]->strip.row1;
+    }
+    struct StripDevice {
         std::vector<int> strips;
         cudaStream_t st[2] = {};
         cudaEvent_t ev = nullptr;                                   // one strip: orders the forwards of the two streams
     };
-    struct RingEntry { int frame = -1, state = 0, launched = 0; };  // state 0 free -> 1 read -> 2 launched on every device -> 0
-    std::vector<StripIO> io(n_nets);
-    std::vector<DeviceIO> devs;
-    for (int i = 0; i < n_nets; ++i) {
-        io[i].net = nets[i];
-        io[i].bytes = (size_t)(nets[i]->strip.row1 - nets[i]->strip.row0) * W;
-        auto d = std::find_if(devs.begin(), devs.end(), [&](const DeviceIO &x) { return x.dev == nets[i]->dev; });
-        if (d == devs.end()) { devs.emplace_back(); d = devs.end() - 1; d->dev = nets[i]->dev; }
-        d->strips.push_back(i);
-    }
-    RingEntry ring[NS];
-    StreamShared sh;
+    struct StripBuffers {
+        uint8_t *d_ori[2] = {}, *d_out[2] = {};                     // per input slot
+        int64_t *d_sse = nullptr;                                   // [n_frames][2]
+    };
+    std::vector<DeviceHold> hold(devices.size());
+    std::vector<StripDevice> sd(devices.size());
+    std::vector<StripBuffers> buf(n_nets);
+    for (int i = 0; i < n_nets; ++i) sd[parts[i].hold].strips.push_back(i);
     const size_t sse_bytes = (size_t)n_frames * 2 * sizeof(int64_t);
-    cudaError_t e = cudaSuccess;
-    for (DeviceIO &D : devs) {
-        // the strips' earlier work, on whatever stream, is complete before this call moves them onto its own streams
-        if (e == cudaSuccess) e = cudaSetDevice(D.dev);
-        if (e == cudaSuccess) e = cudaDeviceSynchronize();
-        for (int s = 0; s < 2 && e == cudaSuccess; ++s) e = cudaStreamCreateWithFlags(&D.st[s], cudaStreamNonBlocking);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&D.ev, cudaEventDisableTiming);
-        for (int i : D.strips) {
-            StripIO &T = io[i];
-            for (int r = 0; r < NS && e == cudaSuccess; ++r) {
-                e = cudaMallocHost(&T.h_in[r], T.bytes);
-                if (e == cudaSuccess) e = cudaMallocHost(&T.h_out[r], T.bytes);
-                if (e == cudaSuccess && with_ori) e = cudaMallocHost(&T.h_ori[r], T.bytes);
-                if (e == cudaSuccess) e = cudaEventCreateWithFlags(&T.done[r], cudaEventDisableTiming);
-            }
-            for (int s = 0; s < 2 && e == cudaSuccess; ++s) {
-                e = cudaMalloc(&T.d_out[s], T.bytes);
-                if (e == cudaSuccess && with_ori) e = cudaMalloc(&T.d_ori[s], T.bytes);
-            }
-            if (e == cudaSuccess && with_ori) e = cudaMalloc(&T.d_sse, sse_bytes);
-            if (e == cudaSuccess && with_ori) e = cudaMemset(T.d_sse, 0, sse_bytes);
-        }
-    }
+    auto bytes = [&](int i) { return (size_t)(parts[i].row1 - parts[i].row0) * W; };
     // the handles' streams are this call's from here on; at the end they are idle and free to be driven on any stream again
     auto unbind = [&]() {
         std::lock_guard<std::mutex> l(g_strip_mu);
         for (int i = 0; i < n_nets; ++i) { nets[i]->strip.used = false; nets[i]->strip.last_stream = nullptr; }
     };
-    auto cleanup = [&]() {
-        for (DeviceIO &D : devs) {
-            cudaSetDevice(D.dev);
-            for (cudaStream_t s : D.st) if (s) { cudaStreamSynchronize(s); cudaStreamDestroy(s); }
-            if (D.ev) cudaEventDestroy(D.ev);
-            for (int i : D.strips) {
-                StripIO &T = io[i];
-                for (int r = 0; r < NS; ++r) {
-                    cudaFreeHost(T.h_in[r]); cudaFreeHost(T.h_ori[r]); cudaFreeHost(T.h_out[r]);
-                    if (T.done[r]) cudaEventDestroy(T.done[r]);
-                }
-                for (int s = 0; s < 2; ++s) { cudaFree(T.d_out[s]); cudaFree(T.d_ori[s]); }
-                cudaFree(T.d_sse);
-            }
-        }
-        unbind();
-    };
-    if (e != cudaSuccess) { cleanup(); set_error("%s: %s", who, cudaGetErrorString(e)); return QV_ERR_CUDA; }
     unbind();
+    for (size_t d = 0; d < devices.size(); ++d) {
+        hold[d].dev = devices[d];
+        // the strips' earlier work, on whatever stream, is complete before this call moves them onto its own streams
+        QV_CUDA(cudaSetDevice(devices[d]));
+        QV_CUDA(cudaDeviceSynchronize());
+        for (int s = 0; s < 2; ++s) QV_CUDA(hold[d].stream(&sd[d].st[s]));
+        QV_CUDA(hold[d].event(&sd[d].ev));
+        for (int i : sd[d].strips) {
+            for (int s = 0; s < 2; ++s) {
+                QV_CUDA(hold[d].alloc(&buf[i].d_out[s], bytes(i)));
+                if (with_ori) QV_CUDA(hold[d].alloc(&buf[i].d_ori[s], bytes(i)));
+            }
+            if (with_ori) {
+                QV_CUDA(hold[d].alloc(&buf[i].d_sse, sse_bytes));
+                QV_CUDA(cudaMemset(buf[i].d_sse, 0, sse_bytes));
+            }
+        }
+    }
 
-    // reader: each strip's rows of the files -> pinned ring, one frame ahead of the GPUs
-    std::thread reader([&] {
-        for (int k = 0; k < n_frames; ++k) {
-            RingEntry &R = ring[k % NS];
-            {
-                std::unique_lock<std::mutex> l(sh.mu);
-                sh.cv.wait(l, [&] { return R.state == 0 || sh.failed; });
-                if (sh.failed) return;
-            }
-            for (StripIO &T : io) {
-                const StripState &S = T.net->strip;
-                if (!read_luma(F.anchor, (long long)first_frame + k, img_h, W, S.row0, S.row1, T.h_in[k % NS]) ||
-                    (with_ori && !read_luma(F.ori, (long long)first_frame + k, img_h, W, S.row0, S.row1, T.h_ori[k % NS]))) {
-                    sh.fail(QV_ERR_IO, "qv_strip_stream_yuv_pf: short read (file smaller than the requested frame range)");
-                    return;
-                }
-            }
-            { std::lock_guard<std::mutex> l(sh.mu); R.frame = k; R.state = 1; }
-            sh.cv.notify_all();
-        }
-    });
-    // writer: pinned ring -> each strip's rows of the reconstruction file, one frame behind the GPUs
-    std::thread writer([&] {
-        std::vector<uint8_t> zeros((size_t)img_h * W / 2, 0);
-        for (int k = 0; k < n_frames; ++k) {
-            RingEntry &R = ring[k % NS];
-            {
-                std::unique_lock<std::mutex> l(sh.mu);
-                sh.cv.wait(l, [&] { return (R.frame == k && R.state == 2) || sh.failed; });
-                if (sh.failed) return;
-            }
-            for (StripIO &T : io) {
-                const StripState &S = T.net->strip;
-                if (cudaSetDevice(T.net->dev) != cudaSuccess || cudaEventSynchronize(T.done[k % NS]) != cudaSuccess) {
-                    sh.fail(QV_ERR_CUDA, "qv_strip_stream_yuv_pf: the GPU stage failed");
-                    return;
-                }
-                if (F.recon >= 0 && !write_recon_rows(F.recon, (long long)first_frame + k, img_h, W, S.row0, S.row1, T.h_out[k % NS], zeros.data())) {
-                    sh.fail(QV_ERR_IO, "qv_strip_stream_yuv_pf: write to the reconstruction file failed");
-                    return;
-                }
-            }
-            { std::lock_guard<std::mutex> l(sh.mu); R.state = 0; R.launched = 0; }
-            sh.cv.notify_all();
-        }
-    });
-    // GPU stage: one thread per device, in frame order
-    auto gpu = [&](DeviceIO &D) {
+    rc = stream_ring(who, F, img_h, W, first_frame, n_frames, 1, parts, hold, [&](int d, int k, int, int, int r) -> int {
+        const StripDevice &D = sd[d];
         const bool solo = D.strips.size() == 1;
-        int grc = QV_OK;
-        if (cudaSetDevice(D.dev) != cudaSuccess) { set_error("%s: cudaSetDevice(%d) failed", who, D.dev); grc = QV_ERR_CUDA; }
-        for (int k = 0; k < n_frames && grc == QV_OK; ++k) {
-            RingEntry &R = ring[k % NS];
-            {
-                std::unique_lock<std::mutex> l(sh.mu);
-                sh.cv.wait(l, [&] { return (R.frame == k && R.state == 1) || sh.failed; });
-                if (sh.failed) return;
-            }
-            const int s = k & 1, r = k % NS;
-            cudaStream_t q = D.st[solo ? s : 0];
-            cudaError_t ce = cudaSuccess;
-            for (size_t j = 0; j < D.strips.size() && grc == QV_OK; ++j)
-                grc = qv_strip_load(io[D.strips[j]].net, s, io[D.strips[j]].h_in[r], q);
-            if (grc == QV_OK && solo && k > 0) ce = cudaStreamWaitEvent(q, D.ev, 0);
-            for (size_t j = 0; j < D.strips.size() && with_ori && grc == QV_OK && ce == cudaSuccess; ++j) {
-                const StripIO &T = io[D.strips[j]];
-                ce = cudaMemcpyAsync(T.d_ori[s], T.h_ori[r], T.bytes, cudaMemcpyHostToDevice, q);
-            }
-            for (size_t j = 0; j < D.strips.size() && grc == QV_OK && ce == cudaSuccess; ++j) {
-                const StripIO &T = io[D.strips[j]];
-                grc = with_ori ? qv_strip_forward_sse(T.net, s, T.d_ori[s], T.d_out[s], T.d_sse + 2 * (size_t)k, q)
-                               : qv_strip_forward(T.net, s, T.d_out[s], q);
-            }
-            if (grc == QV_OK && solo && ce == cudaSuccess) ce = cudaEventRecord(D.ev, q);
-            for (size_t j = 0; j < D.strips.size() && grc == QV_OK && ce == cudaSuccess; ++j) {
-                const StripIO &T = io[D.strips[j]];
-                ce = cudaMemcpyAsync(T.h_out[r], T.d_out[s], T.bytes, cudaMemcpyDeviceToHost, q);
-                if (ce == cudaSuccess) ce = cudaEventRecord(T.done[r], q);
-            }
-            if (grc == QV_OK && ce != cudaSuccess) { set_error("%s: %s", who, cudaGetErrorString(ce)); grc = QV_ERR_CUDA; }
-            if (grc != QV_OK) break;
-            { std::lock_guard<std::mutex> l(sh.mu); if (++R.launched == (int)devs.size()) R.state = 2; }
-            sh.cv.notify_all();
-        }
-        if (grc != QV_OK) {
-            char msg[256];
-            snprintf(msg, sizeof(msg), "GPU %d: %s", D.dev, qv_last_error());      // the message is thread-local: copy it here
-            sh.fail(grc, msg);
-        }
-    };
-    {
-        std::vector<std::thread> th;
-        for (DeviceIO &D : devs) th.emplace_back(gpu, std::ref(D));
-        for (std::thread &t : th) t.join();
-    }
-    reader.join();
-    writer.join();
-    std::vector<int64_t> h_sse(with_ori ? (size_t)n_frames * 2 : 0), sum(h_sse.size(), 0);
-    rc = sh.failed ? sh.rc : QV_OK;
-    for (DeviceIO &D : devs) {
-        if (cudaSetDevice(D.dev) != cudaSuccess) { if (rc == QV_OK) { set_error("%s: cudaSetDevice failed", who); rc = QV_ERR_CUDA; } continue; }
-        for (cudaStream_t s : D.st) cudaStreamSynchronize(s);
+        const int s = k & 1;
+        cudaStream_t q = D.st[solo ? s : 0];
+        int lrc;
+        for (int i : D.strips)
+            if ((lrc = qv_strip_load(nets[i], s, parts[i].h_in[r], q))) return lrc;
+        if (solo && k > 0) QV_CUDA(cudaStreamWaitEvent(q, D.ev, 0));
+        for (int i : D.strips)
+            if (with_ori) QV_CUDA(cudaMemcpyAsync(buf[i].d_ori[s], parts[i].h_ori[r], bytes(i), cudaMemcpyHostToDevice, q));
         for (int i : D.strips) {
-            if (rc == QV_OK && with_ori) {
-                if (cudaMemcpy(h_sse.data(), io[i].d_sse, sse_bytes, cudaMemcpyDeviceToHost) != cudaSuccess) {
-                    set_error("%s: copy of the SSEs failed", who);
-                    rc = QV_ERR_CUDA;
-                }
-                for (size_t x = 0; x < sum.size(); ++x) sum[x] += h_sse[x];
+            const StripBuffers &B = buf[i];
+            lrc = with_ori ? qv_strip_forward_sse(nets[i], s, B.d_ori[s], B.d_out[s], B.d_sse + 2 * (size_t)k, q)
+                           : qv_strip_forward(nets[i], s, B.d_out[s], q);
+            if (lrc) return lrc;
+        }
+        if (solo) QV_CUDA(cudaEventRecord(D.ev, q));
+        for (int i : D.strips) {
+            QV_CUDA(cudaMemcpyAsync(parts[i].h_out[r], buf[i].d_out[s], bytes(i), cudaMemcpyDeviceToHost, q));
+            QV_CUDA(cudaEventRecord(parts[i].done[r], q));
+        }
+        return QV_OK;
+    });
+    std::vector<int64_t> h_sse(with_ori ? (size_t)n_frames * 2 : 0), sum(h_sse.size(), 0);
+    for (size_t d = 0; d < devices.size(); ++d) {
+        if (cudaSetDevice(devices[d]) != cudaSuccess && rc == QV_OK) { set_error("%s: cudaSetDevice failed", who); rc = QV_ERR_CUDA; }
+        hold[d].idle();
+        for (int i : sd[d].strips) {
+            if (rc == QV_OK && with_ori && cudaMemcpy(h_sse.data(), buf[i].d_sse, sse_bytes, cudaMemcpyDeviceToHost) != cudaSuccess) {
+                set_error("%s: copy of the SSEs failed", who);
+                rc = QV_ERR_CUDA;
             }
-            const int krc = kernel_report(nets[i]);                   // on every handle, after the final synchronisation
-            if (rc == QV_OK) rc = krc;
+            for (size_t x = 0; rc == QV_OK && x < sum.size(); ++x) sum[x] += h_sse[x];
         }
     }
-    if (sh.failed) set_error("%s", sh.msg);
-    cleanup();
+    unbind();
+    // every handle's fused-kernel report is taken (and cleared) now that its streams are idle; the first failure's message stands
+    for (int i = 0; i < n_nets; ++i) {
+        if (rc == QV_OK) rc = kernel_report(nets[i]);
+        else if (nets[i]->fm) fused_take_failure(nets[i]->fm);
+    }
     if (rc != QV_OK) return rc;
     for (int j = 0; with_ori && j < n_frames; ++j) {
         if (sse_before_pf) sse_before_pf[j] = sum[2 * (size_t)j];
@@ -1415,8 +1374,7 @@ int qv_set_impl(qv_net *net, int impl)
 int qv_get_impl(const qv_net *net)
 {
     if (!net) return QV_ERR_ARG;
-    if (net->impl != QV_IMPL_AUTO) return net->impl;
-    return net->fm ? QV_IMPL_FUSED : QV_IMPL_LAYERED;
+    return runs_fused(net) ? QV_IMPL_FUSED : QV_IMPL_LAYERED;
 }
 
 long long qv_launch_count(const qv_net *net) { return net ? net->launches : 0; }

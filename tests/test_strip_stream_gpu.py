@@ -1,8 +1,8 @@
 """Streaming a YUV sequence through the strip partition (qv_strip_stream_yuv_pf, `qcnn_gpu --strips S --stream`): every strip
 handle reads its own rows of each frame from the anchor / original files and writes its own rows of the reconstruction.
 Checked against the frame-sharded stream (qv_stream_yuv_pf on a whole-frame handle), numpy's SSEs and the C oracle; a frame
-range in the middle of a file, strips split over calls, every refused argument, the CLI against its in-memory and frame-sharded
-modes, and host memory that does not grow with the sequence."""
+range in the middle of a file, strips split over calls, every refused argument, a reconstruction file that cannot be
+written, the CLI against its in-memory and frame-sharded modes, and host memory that does not grow with the sequence."""
 import ctypes as C
 import os
 import re
@@ -52,8 +52,8 @@ def handles():
     """Creates handles and destroys them after the test, so that a failed test leaves no strip registered on a device."""
     made = []
 
-    def make(dev, rows, w, image):
-        n = api.QVRCNN(dev, 1, 1, rows, w)
+    def make(dev, rows, w, image, batch=1):
+        n = api.QVRCNN(dev, batch, 1, rows, w)
         n.load_static_para_mem(image)
         made.append(n)
         return n
@@ -239,6 +239,39 @@ def test_errors(tmp_path, images, handles):
     assert _raw_call(nets, 2, A, O, str(tmp_path / "never.yuv"), 0, 0) == 0
     assert not (tmp_path / "never.yuv").exists()
     assert _raw_call(nets, 2, A, O, R, 0, 0) == 0 and (tmp_path / "recon.yuv").read_bytes() == done
+
+
+@pytest.mark.parametrize("mode", ["frames", "strips"])
+def test_reconstruction_write_failure(tmp_path, images, handles, mode):
+    """A reconstruction file that takes no bytes (/dev/full): the streaming call returns QV_ERR_IO instead of hanging, and the
+    same handles then stream exactly as fresh ones do.  Frames: qv_stream_yuv_pf in chunks of 4 over 11 frames (3 chunks, the
+    last one short); strips: 2 strips on one device, 7 frames."""
+    if not os.path.exists("/dev/full"):
+        pytest.skip("no /dev/full")
+    h, w = 61, 250
+    n = 11 if mode == "frames" else FRAMES
+    _sequence(tmp_path, h, w, n, 0xC0FFEE + 57)
+    A, O = str(tmp_path / "anchor.yuv"), str(tmp_path / "ori.yuv")
+    image = images["qp27"]
+
+    def make():
+        if mode == "frames":
+            nets = [handles(0, h, w, image, batch=4)]
+            return nets, lambda recon: nets[0].stream_yuv_pf(A, O, recon, 0, n)
+        nets = _strips(handles, image, h, w, _bounds(h, 2), [0, 0])
+        return nets, lambda recon: api.strip_stream_yuv_pf(nets, A, O, recon, 0, n)
+    fresh, call = make()
+    want_b, want_a = call(str(tmp_path / "fresh.yuv"))
+    for x in fresh:                                 # strips of one device are driven together: the fresh ones leave
+        x.strip_release()
+    _, call = make()
+    with pytest.raises(api.QVError) as e:
+        call("/dev/full")
+    assert e.value.code == -2, e.value
+    assert "write to the reconstruction file failed" in str(e.value)
+    b, a = call(str(tmp_path / "again.yuv"))
+    assert (tmp_path / "again.yuv").read_bytes() == (tmp_path / "fresh.yuv").read_bytes()
+    assert np.array_equal(b, want_b) and np.array_equal(a, want_a)
 
 
 # ---- the CLI ----------------------------------------------------------------------------------------------------------------
