@@ -33,6 +33,17 @@ struct ModelHost {
 void set_error(const char *fmt, ...);
 const char *get_error();
 
+// In a function returning a QV_* code (CUDA translation units): a failed CUDA call sets the message and returns QV_ERR_CUDA.
+// Variadic so that template arguments may contain commas.
+#define QV_CUDA(...)                                                                        \
+    do {                                                                                    \
+        cudaError_t e__ = (__VA_ARGS__);                                                    \
+        if (e__ != cudaSuccess) {                                                           \
+            set_error("%s failed: %s (%s:%d)", #__VA_ARGS__, cudaGetErrorString(e__), __FILE__, __LINE__); \
+            return QV_ERR_CUDA;                                                             \
+        }                                                                                   \
+    } while (0)
+
 // formats (qv_formats.cpp)
 size_t model_file_size_vect_c();
 size_t model_file_size_hwcn();

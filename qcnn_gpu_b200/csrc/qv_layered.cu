@@ -5,7 +5,9 @@
 // clamp (inference/cnn.cu:507-523) into C4.  Activations live in HBM as NHWC int8.
 // This path is the simple, independently written second CUDA implementation the fused tcgen05
 // kernel is cross-checked against at sizes the CPU oracle cannot reach.
+#include <algorithm>
 #include <cstdint>
+#include <vector>
 #include <cuda_runtime.h>
 
 #include "qv_device.cuh"
@@ -226,7 +228,103 @@ __global__ void __launch_bounds__(256) k_sse(const uint8_t *__restrict__ a, cons
     }
 }
 
-// ---- host launchers ---------------------------------------------------------------------
+// ---- host side --------------------------------------------------------------------------
+struct LayeredLayer {
+    int32_t *d_wpk = nullptr;   // packed weights (layout documented at each kernel)
+    int32_t *d_bias = nullptr;  // int32 bias[cout]
+    QParam q{};
+    int cout = 0;
+};
+
+struct LayeredNet {
+    int batch = 0, H = 0, W = 0;                // the handle's geometry
+    LayeredLayer L[QV_NLAYER];
+    int c4_bias = 0;
+    // C1.v, Conc1.conc, Conc2.conc of the reference (inference/cnn.cu:64,281), NHWC here; the reference also holds 644 B/px
+    // of fp32 `u` tensors which this design never materialises.
+    int8_t *a1 = nullptr, *a2 = nullptr, *a3 = nullptr;
+    int act_frames = 0;
+    uint8_t *rows = nullptr;                    // the window of layered_forward_rows, run as an image of its own
+    size_t rows_bytes = 0;
+    cudaEvent_t ev = nullptr;                   // recorded after the last launch or copy of every call that uses a1..a3 / rows
+};
+
+cudaError_t layered_create(LayeredNet **out, int batch, int H, int W)
+{
+    *out = new LayeredNet{batch, H, W};
+    return cudaEventCreateWithFlags(&(*out)->ev, cudaEventDisableTiming);
+}
+
+static void free_weights(LayeredNet *ln)
+{
+    for (LayeredLayer &D : ln->L) { cudaFree(D.d_wpk); cudaFree(D.d_bias); D = LayeredLayer{}; }
+}
+
+void layered_free(LayeredNet *ln)
+{
+    if (!ln) return;
+    free_weights(ln);
+    cudaFree(ln->a1); cudaFree(ln->a2); cudaFree(ln->a3);
+    cudaFree(ln->rows);
+    if (ln->ev) cudaEventDestroy(ln->ev);
+    delete ln;
+}
+
+static int pack_word(const int8_t *p, int stride, int n)
+{
+    int v = 0;
+    for (int j = 0; j < n; ++j) v |= ((int)(uint8_t)p[j * stride]) << (8 * j);
+    return v;
+}
+
+// Re-pack the plain [K][C][R][S] host weights into the word layouts the kernels above read.
+int layered_load(LayeredNet *ln, const ModelHost &m, cudaStream_t st)
+{
+    free_weights(ln);
+    for (int l = 0; l < QV_NLAYER; ++l) {
+        const LayerShape &s = kLayers[l];
+        const LayerHost &L = m.L[l];
+        std::vector<int32_t> wpk;
+        const int R = s.k;
+        if (l == QV_C1) {                        // [r][k][2]
+            wpk.assign(5 * 64 * 2, 0);
+            for (int r = 0; r < 5; ++r)
+                for (int k = 0; k < 64; ++k) {
+                    const int8_t *row = &L.w[((size_t)k * 5 + r) * 5];
+                    wpk[(r * 64 + k) * 2 + 0] = pack_word(row, 1, 4);
+                    wpk[(r * 64 + k) * 2 + 1] = pack_word(row + 4, 1, 1);
+                }
+        } else if (l == QV_C4) {                 // [tap][c4]
+            wpk.assign(9 * 12, 0);
+            for (int t = 0; t < 9; ++t)
+                for (int c4 = 0; c4 < 12; ++c4)
+                    wpk[t * 12 + c4] = pack_word(&L.w[((size_t)(4 * c4) * 3 + t / 3) * 3 + t % 3], 9, 4);
+        } else {                                 // [group][tap][c4][16]
+            const int C4 = s.cin / 4, G = s.cout / 16;
+            wpk.assign((size_t)G * R * R * C4 * 16, 0);
+            for (int g = 0; g < G; ++g)
+                for (int t = 0; t < R * R; ++t)
+                    for (int c4 = 0; c4 < C4; ++c4)
+                        for (int j = 0; j < 16; ++j) {
+                            const int k = g * 16 + j;
+                            wpk[(((size_t)g * R * R + t) * C4 + c4) * 16 + j] =
+                                pack_word(&L.w[(((size_t)k * s.cin + 4 * c4) * R + t / R) * R + t % R], R * R, 4);
+                        }
+        }
+        LayeredLayer &D = ln->L[l];
+        D.cout = s.cout;
+        D.q.blu = L.blu; D.q.mul = L.mul; D.q.shift = L.shift;
+        D.q.rbias = (1 << (L.shift - 1)) / L.mul;                       // inference/mat.cu:268
+        QV_CUDA(cudaMalloc(&D.d_wpk, wpk.size() * sizeof(int32_t)));
+        QV_CUDA(cudaMalloc(&D.d_bias, L.b.size() * sizeof(int32_t)));
+        QV_CUDA(cudaMemcpyAsync(D.d_wpk, wpk.data(), wpk.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        QV_CUDA(cudaMemcpyAsync(D.d_bias, L.b.data(), L.b.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        QV_CUDA(cudaStreamSynchronize(st));   // wpk is a local
+    }
+    ln->c4_bias = m.L[QV_C4].b[0];
+    return QV_OK;
+}
+
 template <int CIN, int KS>
 static cudaError_t launch_conv(const int8_t *in, int8_t *out, const LayeredLayer &L, int n, int H, int W, int out_ch,
                                int out_coff, cudaStream_t st)
@@ -243,29 +341,90 @@ static cudaError_t launch_conv(const int8_t *in, int8_t *out, const LayeredLayer
     return cudaGetLastError();
 }
 
-cudaError_t layered_forward(const LayeredModel &M, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W,
-                            int8_t *a1, int8_t *a2, int8_t *a3, cudaStream_t st, long long *launches)
+// The scratch is allocated at the first forward; n frames run in chunks of as many frames as it holds.
+int layered_forward(LayeredNet *ln, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W, cudaStream_t st,
+                    long long *launches, const uint8_t *d_ori, int64_t *d_sse)
 {
-    cudaError_t e;
-    dim3 block(TX, TY), grid((W + TX - 1) / TX, (H + TY - 1) / TY, n);
-    k_c1<<<grid, block, 0, st>>>(d_in, a1, M.L[QV_C1].d_wpk, M.L[QV_C1].d_bias, M.L[QV_C1].q, H, W);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    if ((e = launch_conv<64, 3>(a1, a2, M.L[QV_C2_1], n, H, W, 48, 0, st)) != cudaSuccess) return e;
-    if ((e = launch_conv<64, 5>(a1, a2, M.L[QV_C2_2], n, H, W, 48, 32, st)) != cudaSuccess) return e;
-    if ((e = launch_conv<48, 3>(a2, a3, M.L[QV_C3_1], n, H, W, 48, 0, st)) != cudaSuccess) return e;
-    if ((e = launch_conv<48, 1>(a2, a3, M.L[QV_C3_2], n, H, W, 48, 16, st)) != cudaSuccess) return e;
-    k_c4_res<<<grid, block, 0, st>>>(a3, d_in, d_out, M.L[QV_C4].d_wpk, M.c4_bias, M.L[QV_C4].q.mul,
-                                     M.L[QV_C4].q.shift, H, W);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    if (launches) *launches += 6;
-    return cudaSuccess;
+    if (!ln->a1) {
+        const int frames = std::min(ln->batch, 8);
+        const size_t px = (size_t)frames * ln->H * ln->W;
+        QV_CUDA(cudaMalloc(&ln->a1, px * 64));
+        QV_CUDA(cudaMalloc(&ln->a2, px * 48));
+        QV_CUDA(cudaMalloc(&ln->a3, px * 48));
+        ln->act_frames = frames;
+    }
+    const size_t cap_px = (size_t)ln->act_frames * ln->H * ln->W, fpx = (size_t)H * W;
+    if (fpx > cap_px) { set_error("frame of %dx%d exceeds the handle's activation scratch", W, H); return QV_ERR_ARG; }
+    QV_CUDA(cudaStreamWaitEvent(st, ln->ev, 0));
+    const int chunk = (int)std::max<size_t>(1, cap_px / fpx);
+    const LayeredLayer *L = ln->L;
+    int8_t *a1 = ln->a1, *a2 = ln->a2, *a3 = ln->a3;
+    for (int f0 = 0; f0 < n; f0 += chunk) {
+        const int c = std::min(chunk, n - f0);
+        const uint8_t *in = d_in + (size_t)f0 * fpx;
+        const dim3 block(TX, TY), grid((W + TX - 1) / TX, (H + TY - 1) / TY, c);
+        k_c1<<<grid, block, 0, st>>>(in, a1, L[QV_C1].d_wpk, L[QV_C1].d_bias, L[QV_C1].q, H, W);
+        QV_CUDA(cudaGetLastError());
+        QV_CUDA(launch_conv<64, 3>(a1, a2, L[QV_C2_1], c, H, W, 48, 0, st));
+        QV_CUDA(launch_conv<64, 5>(a1, a2, L[QV_C2_2], c, H, W, 48, 32, st));
+        QV_CUDA(launch_conv<48, 3>(a2, a3, L[QV_C3_1], c, H, W, 48, 0, st));
+        QV_CUDA(launch_conv<48, 1>(a2, a3, L[QV_C3_2], c, H, W, 48, 16, st));
+        k_c4_res<<<grid, block, 0, st>>>(a3, in, d_out + (size_t)f0 * fpx, L[QV_C4].d_wpk, ln->c4_bias, L[QV_C4].q.mul,
+                                         L[QV_C4].q.shift, H, W);
+        QV_CUDA(cudaGetLastError());
+        *launches += 6;
+    }
+    if (d_sse) {
+        for (int f = 0; f < n; ++f) {
+            const size_t o = (size_t)f * fpx;
+            QV_CUDA(sse_accumulate(d_in + o, d_ori + o, fpx, d_sse + 2 * f, st));
+            QV_CUDA(sse_accumulate(d_out + o, d_ori + o, fpx, d_sse + 2 * f + 1, st));
+        }
+        *launches += 2 * n;
+    }
+    QV_CUDA(cudaEventRecord(ln->ev, st));
+    return QV_OK;
 }
 
-cudaError_t nhwc_to_planar(const int8_t *d_in, int8_t *d_out, int C, size_t HW, cudaStream_t st)
+int layered_forward_rows(LayeredNet *ln, const uint8_t *d_in, int in_rows, uint8_t *d_out, int out0, int out1, cudaStream_t st,
+                         long long *launches)
 {
-    const size_t n = (size_t)C * HW;
-    k_nhwc_to_planar<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_in, d_out, C, (int)HW);
-    return cudaGetLastError();
+    const size_t W = ln->W, need = (size_t)in_rows * W;
+    if (need > (size_t)ln->batch * ln->H * ln->W) {
+        set_error("qv_forward_rows_device: window larger than the handle's geometry");
+        return QV_ERR_ARG;
+    }
+    if (ln->rows_bytes < need) {
+        QV_CUDA(cudaEventSynchronize(ln->ev));     // the buffer's last user, on whatever stream
+        cudaFree(ln->rows);
+        ln->rows = nullptr; ln->rows_bytes = 0;
+        QV_CUDA(cudaMalloc(&ln->rows, need));
+        ln->rows_bytes = need;
+    }
+    const int rc = layered_forward(ln, d_in, ln->rows, 1, in_rows, ln->W, st, launches, nullptr, nullptr);
+    if (rc) return rc;
+    QV_CUDA(cudaMemcpyAsync(d_out, ln->rows + (size_t)out0 * W, (size_t)(out1 - out0) * W, cudaMemcpyDeviceToDevice, st));
+    QV_CUDA(cudaEventRecord(ln->ev, st));       // again: the next user of the buffer waits for the copy too
+    return QV_OK;
+}
+
+int layered_activation(LayeredNet *ln, int which, int8_t *host_out, cudaStream_t st)
+{
+    if (!ln->a1) { set_error("qv_get_activation: the layered path has not run on this handle"); return QV_ERR_STATE; }
+    const int C = which == 1 ? 64 : 48;
+    const int8_t *src = which == 1 ? ln->a1 : (which == 2 ? ln->a2 : ln->a3);
+    const size_t HW = (size_t)ln->H * ln->W, n = HW * C;
+    int8_t *tmp = nullptr;
+    QV_CUDA(cudaStreamWaitEvent(st, ln->ev, 0));
+    QV_CUDA(cudaMalloc(&tmp, n));
+    k_nhwc_to_planar<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(src, tmp, C, (int)HW);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(host_out, tmp, n, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaEventRecord(ln->ev, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    cudaFree(tmp);
+    QV_CUDA(e);
+    return QV_OK;
 }
 
 cudaError_t sse_accumulate(const uint8_t *a, const uint8_t *b, size_t n, int64_t *d_accum, cudaStream_t st)

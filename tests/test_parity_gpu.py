@@ -346,6 +346,75 @@ def test_device_entry_and_sse(models):
     assert net.launch_count() > 0
 
 
+@pytest.mark.parametrize("entry", ["frames", "frames_sse", "rows"])
+def test_layered_calls_on_several_streams_are_ordered(models, entry):
+    """A layered handle's calls share its activation scratch, whatever stream they run on: two asynchronous calls with
+    different inputs on two streams, then a third on a caller stream directly followed by qv_get_activation (which runs on
+    the handle's own stream), with no synchronisation in between -- every output, SSE and activation is the oracle's."""
+    import torch
+    m = models[27]
+    om = _oracle(m)
+    h, w = 120, 208
+    net = _net(m, 2, h, w, api.IMPL_LAYERED)
+    sse = lambda x, ori: ((x.astype(np.int64) - ori) ** 2).reshape(len(x), -1).sum(axis=1)
+    calls = []
+    for i in range(3):
+        if entry == "rows":
+            # rows [40, 160) of a 200-row image, run as a window; its rows [46, 154) are exact
+            img = synth.make_frames(0xC0FFEE + 50 + i, 1, 200, w)[0]
+            d_in = torch.from_numpy(np.ascontiguousarray(img[0, 40:160])).cuda()
+            d_out = torch.zeros((108, w), dtype=torch.uint8, device="cuda")
+            calls.append(dict(d_in=d_in, d_out=d_out, want=om.forward_blu(img)[0, 46:154], taps=img[0, 40:160]))
+        else:
+            x, ori = synth.make_frames(0xC0FFEE + 50 + i, 2, h, w)
+            want = om.forward_blu(x)
+            calls.append(dict(d_in=torch.from_numpy(x).cuda(), d_ori=torch.from_numpy(ori).cuda(),
+                              d_out=torch.zeros((2, h, w), dtype=torch.uint8, device="cuda"),
+                              d_sse=torch.zeros(4, dtype=torch.int64, device="cuda"), want=want, taps=x[0],
+                              sse=np.stack([sse(x, ori), sse(want, ori)], axis=1).reshape(-1)))
+
+    def run(c, stream):
+        if entry == "rows":
+            net.forward_rows_device(c["d_in"].data_ptr(), 200, 40, 120, c["d_out"].data_ptr(), 46, 154, stream.cuda_stream)
+        elif entry == "frames":
+            net.forward_frames_device(c["d_in"].data_ptr(), c["d_out"].data_ptr(), 2, stream.cuda_stream)
+        else:
+            net.forward_frames_device_sse(c["d_in"].data_ptr(), c["d_ori"].data_ptr(), c["d_out"].data_ptr(), 2,
+                                          c["d_sse"].data_ptr(), stream.cuda_stream)
+
+    torch.cuda.synchronize()                  # the inputs are on the device before any call
+    a, b = torch.cuda.Stream(), torch.cuda.Stream()
+    run(calls[0], a)
+    run(calls[1], b)
+    run(calls[2], a)
+    acts = [net.get_activation(k) for k in (1, 2, 3)]
+    torch.cuda.synchronize()
+    for i, c in enumerate(calls):
+        assert np.array_equal(c["d_out"].cpu().numpy(), c["want"]), (entry, i)
+        if entry == "frames_sse":
+            assert c["d_sse"].cpu().numpy().tolist() == c["sse"].tolist(), i
+    _, a1, a2, a3, _ = om.forward_taps(calls[2]["taps"])
+    for k, want in enumerate((a1, a2, a3)):
+        assert np.array_equal(acts[k], want), (entry, k + 1)
+    assert net.launch_count() == 3 * (10 if entry == "frames_sse" else 6)
+
+
+def test_layered_scratch_errors(models):
+    """qv_get_activation before any layered forward, and a row window of more pixels than batch x H x W."""
+    import torch
+    net = _net(models[27], 1, 40, 64, api.IMPL_LAYERED)
+    with pytest.raises(api.QVError) as e:
+        net.get_activation(1)
+    assert e.value.code == -5
+    assert str(e.value) == "qvrcnn_b200 error -5: qv_get_activation: the layered path has not run on this handle"
+    d_in = torch.zeros((41, 64), dtype=torch.uint8, device="cuda")
+    d_out = torch.zeros_like(d_in)
+    with pytest.raises(api.QVError) as e:
+        net.forward_rows_device(d_in.data_ptr(), 41, 0, 41, d_out.data_ptr(), 0, 41)
+    assert e.value.code == -1
+    assert str(e.value) == "qvrcnn_b200 error -1: qv_forward_rows_device: window larger than the handle's geometry"
+
+
 def test_error_behaviour(models, tmp_path):
     net = api.QVRCNN(0, 1, 1, 16, 16)
     with pytest.raises(api.QVError) as e:           # forward before load
