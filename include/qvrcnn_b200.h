@@ -175,7 +175,9 @@ enum { QV_STRIP_ABOVE = 0, QV_STRIP_BELOW = 1 };
 /* This handle owns image rows [row0, row1) of an img_height x width frame (width = the handle's). */
 QV_API int qv_strip_setup(qv_net *net, int img_height, int row0, int row1);
 QV_API int qv_strip_export(qv_net *net, qv_strip_desc *out);
-/* Maps the neighbour's block.  Fails if the rows are not adjacent, or if the neighbour holds fewer than 6 rows. */
+/* Maps the neighbour's block.  Fails if the rows are not adjacent, or if the neighbour holds fewer than 6 rows.  A descriptor
+   of this process whose strip has since been released (qv_strip_release, qv_destroy or a new qv_strip_setup) is refused
+   with QV_ERR_STATE. */
 QV_API int qv_strip_attach(qv_net *net, int side, const qv_strip_desc *neighbour);
 /* Device pointer of input slot 0 / 1 ((row1-row0) * width bytes) for callers that fill it on the device. */
 QV_API int qv_strip_input(qv_net *net, int slot, void **d_rows);
@@ -215,7 +217,9 @@ QV_API int qv_strip_forward_sse(qv_net *net, int slot, const uint8_t *d_ori_rows
 QV_API int qv_strip_stream_yuv_pf(qv_net *const *nets, int n_nets, const char *anchor_yuv, const char *ori_yuv,
                                   const char *recon_yuv, int first_frame, int n_frames,
                                   int64_t *sse_before_pf, int64_t *sse_after_pf);
-/* Unmaps the neighbours and frees the block (all GPUs must be idle). */
+/* Unmaps the neighbours and frees the block (all GPUs must be idle).  The strips of this process that had this one attached
+   lose it: their forwards return QV_ERR_STATE until a neighbour is attached again.  Strips of other processes are not told
+   (one process cannot revoke another's mapping). */
 QV_API int qv_strip_release(qv_net *net);
 
 /* Explicit device-pointer accessor for drivers that, like the reference's, read the object's

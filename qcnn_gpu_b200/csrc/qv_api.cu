@@ -11,7 +11,6 @@
 #include <cstring>
 #include <functional>
 #include <mutex>
-#include <random>
 #include <thread>
 #include <vector>
 
@@ -23,61 +22,12 @@
 #include "qv_fused.h"
 #include "qv_internal.h"
 #include "qv_layered.h"
+#include "qv_strip.h"
 
 using namespace qv;
 
-// ---- spatial strips over several GPUs (SURVEY 8e-ii) ---------------------------------------------------------
-// One cudaMalloc'ed block per handle: a 256-byte header (published / completed sequence numbers, CTA counter) and two
-// input slots holding this GPU's rows of the frame.  The block is what neighbours map (same process: peer access;
-// other process: CUDA IPC) and read their 6 halo rows from, straight out of this GPU's HBM over NVLink.
-namespace {
-constexpr int STRIP_HALO = 6;                   // receptive-field radius of the net: 2 + 2 + 1 + 1 rows
-constexpr size_t STRIP_HDR = 256, STRIP_PUB = 0, STRIP_DONE = 64, STRIP_CTR = 128;
-constexpr uint32_t STRIP_MAGIC = 0x51565354u;   // "QVST"
-struct StripDescImpl {                          // the content of qv_strip_desc
-    uint32_t magic;
-    int32_t dev, row0, row1, width, img_h;
-    uint64_t nonce;                             // identifies the exporting process
-    uint64_t base, slot_off, slot_stride;
-    uint64_t net;                               // the exporting handle (meaningful inside the exporting process only)
-    cudaIpcMemHandle_t ipc;
-    char pci[16];                               // PCI bus id of the device: device ordinals differ between processes
-};
-static_assert(sizeof(StripDescImpl) <= sizeof(qv_strip_desc), "qv_strip_desc too small");
-struct StripPeer {
-    bool attached = false, ipc = false, same_device = false;
-    uint8_t *base = nullptr;
-    qv_net *net = nullptr;                      // same process only
-    StripDescImpl d{};
-};
-struct StripState {
-    bool on = false;
-    int img_h = 0, row0 = 0, row1 = 0;
-    uint8_t *block = nullptr;
-    size_t slot_stride = 0;
-    uint32_t seq = 0, slot_seq[2] = {0, 0};
-    uint32_t fills[2] = {0, 0}, forwards[2] = {0, 0};   // per slot: how often acquired for filling / consumed (ordering checks between strips that share a GPU)
-    cudaStream_t last_stream = nullptr;
-    bool used = false;
-    StripPeer peer[2];                          // QV_STRIP_ABOVE, QV_STRIP_BELOW
-};
-// Strip-mode handles of this process, per device.  Kernels that wait for one another must never share a GPU (nothing
-// guarantees that two launches on one GPU run at the same time), so strips that live on the SAME device are ordered by
-// the stream they are driven on instead: one stream for all of them, all loads of a frame before its forwards (checked).
-std::mutex g_strip_mu;
-std::vector<qv_net *> g_strip_nets[64];
-uint64_t process_nonce()
-{
-    static const uint64_t n = [] {
-        std::random_device rd;
-        return ((uint64_t)rd() << 32) ^ (uint64_t)rd() ^ ((uint64_t)getpid() << 17);
-    }();
-    return n;
-}
-}  // namespace
-
 struct qv_net {
-    StripState strip;
+    StripNet *strip = nullptr;                     // null: not a strip handle (qv_strip_setup)
     int dev = 0, batch = 0, H = 0, W = 0;
     cudaStream_t st = nullptr;
     cudaStream_t pst[2] = {nullptr, nullptr};      // pipeline slots of qv_forward_frames_host
@@ -93,6 +43,9 @@ struct qv_net {
 };
 
 static int set_device(const qv_net *net) { QV_CUDA(cudaSetDevice(net->dev)); return QV_OK; }
+
+// The stream of an entry point's cuda_stream argument: null names the handle's own.
+static cudaStream_t stream_of(const qv_net *net, void *cuda_stream) { return cuda_stream ? (cudaStream_t)cuda_stream : net->st; }
 
 // Does this handle run the fused kernel?  QV_IMPL_AUTO picks it whenever it is built.
 static bool runs_fused(const qv_net *net) { return net->impl == QV_IMPL_FUSED || (net->impl == QV_IMPL_AUTO && net->fm); }
@@ -318,6 +271,14 @@ static int kernel_report(qv_net *net)
     return QV_ERR_CUDA;
 }
 
+// The end of an entry point that ran on cuda_stream: a null one named the handle's own stream, and the call is synchronous.
+static int finish(qv_net *net, void *cuda_stream)
+{
+    if (cuda_stream) return QV_OK;
+    QV_CUDA(cudaStreamSynchronize(net->st));
+    return kernel_report(net);
+}
+
 // qv_forward_blu, qv_forward_frames_device and, with d_ori / d_sse, qv_forward_frames_device_sse once their arguments are
 // checked.  A null cuda_stream runs on the handle's own stream and synchronises.
 static int forward_frames_device(qv_net *net, const uint8_t *d_in, const uint8_t *d_ori, uint8_t *d_out, int n_frames,
@@ -325,10 +286,8 @@ static int forward_frames_device(qv_net *net, const uint8_t *d_in, const uint8_t
 {
     int rc = set_device(net);
     if (rc) return rc;
-    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : net->st;
-    if (n_frames > 0 && (rc = run_forward(net, d_in, d_out, n_frames, net->H, net->W, st, d_ori, d_sse))) return rc;
-    if (!cuda_stream) { QV_CUDA(cudaStreamSynchronize(st)); return kernel_report(net); }
-    return QV_OK;
+    if (n_frames > 0 && (rc = run_forward(net, d_in, d_out, n_frames, net->H, net->W, stream_of(net, cuda_stream), d_ori, d_sse))) return rc;
+    return finish(net, cuda_stream);
 }
 
 int qv_forward_blu(qv_net *net)
@@ -377,7 +336,7 @@ int qv_forward_rows_device(qv_net *net, const uint8_t *d_in, int img_height, int
     }
     int rc = set_device(net);
     if (rc) return rc;
-    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : net->st;
+    const cudaStream_t st = stream_of(net, cuda_stream);
     if (!net->uploaded || (runs_fused(net) && !net->fm)) { set_error("forward called before a complete model (weights + quant params) was loaded"); return QV_ERR_STATE; }
     if (runs_fused(net)) {
         // the fused kernel takes the window as what it is: rows [in_row0, in_row1) of an img_height-row image, of which it
@@ -388,8 +347,7 @@ int qv_forward_rows_device(qv_net *net, const uint8_t *d_in, int img_height, int
     } else if ((rc = layered_forward_rows(net->ln, d_in, in_rows, d_out, out_row0 - in_row0, out_row1 - in_row0, st, &net->launches))) {
         return rc;
     }
-    if (!cuda_stream) { QV_CUDA(cudaStreamSynchronize(st)); return kernel_report(net); }
-    return QV_OK;
+    return finish(net, cuda_stream);
 }
 
 int qv_synchronize(qv_net *net, void *cuda_stream)
@@ -397,33 +355,30 @@ int qv_synchronize(qv_net *net, void *cuda_stream)
     if (!net) { set_error("qv_synchronize: null handle"); return QV_ERR_ARG; }
     int rc = set_device(net);
     if (rc) return rc;
-    QV_CUDA(cudaStreamSynchronize(cuda_stream ? (cudaStream_t)cuda_stream : net->st));
+    QV_CUDA(cudaStreamSynchronize(stream_of(net, cuda_stream)));
     return kernel_report(net);
 }
 
-// ---- strips: setup / export / attach / load / forward -------------------------------------------------------------
-static void strip_detach(qv_net *net)
+// ---- strips: setup / export / attach / load / forward (qv_strip.cu) -------------------------------------------------
+// Past its argument checks, a strip entry point needs qv_strip_setup and the handle's device.
+static int strip_on(qv_net *net, const char *who)
 {
-    for (StripPeer &p : net->strip.peer) {
-        if (p.attached && p.ipc && p.base) cudaIpcCloseMemHandle(p.base);
-        p = StripPeer{};
-    }
+    if (!net->strip) { set_error("%s: qv_strip_setup has not been called", who); return QV_ERR_STATE; }
+    return set_device(net);
+}
+
+// A strip forward runs the fused kernel, which reads the neighbours' halo rows.
+static int strip_fused(const qv_net *net, const char *who)
+{
+    if (net->uploaded && net->fm && net->impl != QV_IMPL_LAYERED) return QV_OK;
+    set_error("%s: needs a loaded model and the fused path (peer-mapped halo rows are read by the fused kernel)", who);
+    return QV_ERR_STATE;
 }
 
 int qv_strip_release(qv_net *net)
 {
     if (!net) { set_error("qv_strip_release: null handle"); return QV_ERR_ARG; }
-    if (!net->strip.on) return QV_OK;
-    cudaSetDevice(net->dev);
-    cudaStreamSynchronize(net->st);
-    strip_detach(net);
-    cudaFree(net->strip.block);
-    net->strip = StripState{};
-    if (net->dev >= 0 && net->dev < 64) {
-        std::lock_guard<std::mutex> l(g_strip_mu);
-        auto &v = g_strip_nets[net->dev];
-        v.erase(std::remove(v.begin(), v.end(), net), v.end());
-    }
+    if (net->strip) { cudaSetDevice(net->dev); cudaStreamSynchronize(net->st); strip_free(net->strip); net->strip = nullptr; }
     return QV_OK;
 }
 
@@ -431,233 +386,69 @@ int qv_strip_setup(qv_net *net, int img_height, int row0, int row1)
 {
     if (!net) { set_error("qv_strip_setup: null handle"); return QV_ERR_ARG; }
     if (img_height < 1 || row0 < 0 || row1 <= row0 || row1 > img_height) { set_error("qv_strip_setup: rows [%d, %d) of %d", row0, row1, img_height); return QV_ERR_ARG; }
-    int rc = set_device(net);
-    if (rc) return rc;
+    if (int rc = set_device(net)) return rc;
     qv_strip_release(net);
-    StripState &S = net->strip;
-    S.img_h = img_height; S.row0 = row0; S.row1 = row1;
-    S.slot_stride = ((size_t)(row1 - row0) * net->W + 255) / 256 * 256;
-    QV_CUDA(cudaMalloc(&S.block, STRIP_HDR + 2 * S.slot_stride));
-    QV_CUDA(cudaMemset(S.block, 0, STRIP_HDR));
-    QV_CUDA(cudaDeviceSynchronize());
-    S.on = true;
-    if (net->dev >= 0 && net->dev < 64) {
-        std::lock_guard<std::mutex> l(g_strip_mu);
-        g_strip_nets[net->dev].push_back(net);
-    }
-    return QV_OK;
+    return strip_create(&net->strip, net->dev, net->W, img_height, row0, row1);
 }
 
 int qv_strip_export(qv_net *net, qv_strip_desc *out)
 {
     if (!net || !out) { set_error("qv_strip_export: null argument"); return QV_ERR_ARG; }
-    if (!net->strip.on) { set_error("qv_strip_export: qv_strip_setup has not been called"); return QV_ERR_STATE; }
-    int rc = set_device(net);
-    if (rc) return rc;
-    StripDescImpl d{};
-    d.magic = STRIP_MAGIC; d.dev = net->dev; d.row0 = net->strip.row0; d.row1 = net->strip.row1; d.width = net->W; d.img_h = net->strip.img_h;
-    d.nonce = process_nonce();
-    d.base = (uint64_t)(uintptr_t)net->strip.block; d.slot_off = STRIP_HDR; d.slot_stride = net->strip.slot_stride;
-    d.net = (uint64_t)(uintptr_t)net;
-    QV_CUDA(cudaIpcGetMemHandle(&d.ipc, net->strip.block));
-    QV_CUDA(cudaDeviceGetPCIBusId(d.pci, (int)sizeof(d.pci), net->dev));
-    memset(out, 0, sizeof(*out));
-    memcpy(out, &d, sizeof(d));
-    return QV_OK;
+    const int rc = strip_on(net, "qv_strip_export");
+    return rc ? rc : strip_export(net->strip, out);
 }
 
 int qv_strip_attach(qv_net *net, int side, const qv_strip_desc *neighbour)
 {
     if (!net || !neighbour || (side != QV_STRIP_ABOVE && side != QV_STRIP_BELOW)) { set_error("qv_strip_attach: bad argument"); return QV_ERR_ARG; }
-    StripState &S = net->strip;
-    if (!S.on) { set_error("qv_strip_attach: qv_strip_setup has not been called"); return QV_ERR_STATE; }
-    StripDescImpl d;
-    memcpy(&d, neighbour, sizeof(d));
-    if (d.magic != STRIP_MAGIC) { set_error("qv_strip_attach: not a strip descriptor"); return QV_ERR_ARG; }
-    if (d.width != net->W || d.img_h != S.img_h) { set_error("qv_strip_attach: the neighbour's frame is %dx%d, this one %dx%d", d.width, d.img_h, net->W, S.img_h); return QV_ERR_ARG; }
-    if (side == QV_STRIP_ABOVE ? d.row1 != S.row0 : d.row0 != S.row1) {
-        set_error("qv_strip_attach: rows [%d, %d) are not adjacent %s rows [%d, %d)", d.row0, d.row1, side == QV_STRIP_ABOVE ? "above" : "below", S.row0, S.row1);
-        return QV_ERR_ARG;
-    }
-    if (d.row1 - d.row0 < STRIP_HALO) {
-        // the halo would reach into the strip after next, which this protocol does not exchange
-        set_error("qv_strip_attach: the neighbour holds %d rows, fewer than the %d-row halo (use fewer strips)", d.row1 - d.row0, STRIP_HALO);
-        return QV_ERR_ARG;
-    }
-    int rc = set_device(net);
-    if (rc) return rc;
-    StripPeer &P = S.peer[side];
-    if (P.attached && P.ipc && P.base) cudaIpcCloseMemHandle(P.base);
-    P = StripPeer{};
-    if (d.nonce == process_nonce()) {
-        // same process: plain peer access to the neighbour's allocation
-        if (d.dev != net->dev) {
-            int can = 0;
-            QV_CUDA(cudaDeviceCanAccessPeer(&can, net->dev, d.dev));
-            if (!can) { set_error("qv_strip_attach: device %d cannot map memory of device %d (no peer access)", net->dev, d.dev); return QV_ERR_CUDA; }
-            cudaError_t e = cudaDeviceEnablePeerAccess(d.dev, 0);
-            if (e == cudaErrorPeerAccessAlreadyEnabled) { cudaGetLastError(); e = cudaSuccess; }
-            QV_CUDA(e);
-        }
-        P.base = (uint8_t *)(uintptr_t)d.base;
-        P.net = (qv_net *)(uintptr_t)d.net;
-    } else {
-        char my_pci[16] = {0};
-        QV_CUDA(cudaDeviceGetPCIBusId(my_pci, (int)sizeof(my_pci), net->dev));
-        if (strncmp(my_pci, d.pci, sizeof(my_pci)) == 0) {
-            // two processes time-slicing one GPU: a kernel of one that waits for a kernel of the other may never see it run
-            set_error("qv_strip_attach: the neighbour strip belongs to another process on the SAME GPU; strips of different processes must be on different GPUs");
-            return QV_ERR_ARG;
-        }
-        void *p = nullptr;
-        QV_CUDA(cudaIpcOpenMemHandle(&p, d.ipc, cudaIpcMemLazyEnablePeerAccess));
-        P.base = (uint8_t *)p;
-        P.ipc = true;
-    }
-    P.d = d;
-    char my_pci[16] = {0};
-    QV_CUDA(cudaDeviceGetPCIBusId(my_pci, (int)sizeof(my_pci), net->dev));
-    P.same_device = strncmp(my_pci, d.pci, sizeof(my_pci)) == 0;
-    P.attached = true;
-    return QV_OK;
+    const int rc = strip_on(net, "qv_strip_attach");
+    return rc ? rc : strip_attach(net->strip, side, neighbour);
 }
 
 int qv_strip_input(qv_net *net, int slot, void **d_rows)
 {
     if (!net || !d_rows || slot < 0 || slot > 1) { set_error("qv_strip_input: bad argument"); return QV_ERR_ARG; }
-    if (!net->strip.on) { set_error("qv_strip_input: qv_strip_setup has not been called"); return QV_ERR_STATE; }
-    *d_rows = net->strip.block + STRIP_HDR + (size_t)slot * net->strip.slot_stride;
-    return QV_OK;
-}
-
-// Strips that share this handle's GPU (same process) are ordered by the one stream they must all be driven on.
-static int check_shared_device_stream(qv_net *net, cudaStream_t st, const char *who)
-{
-    std::lock_guard<std::mutex> l(g_strip_mu);
-    for (qv_net *o : g_strip_nets[net->dev])
-        if (o != net && o->strip.used && o->strip.last_stream != st) {
-            set_error("%s: several strips live on GPU %d: drive all of them on ONE caller-provided stream (kernels of different launches "
-                      "must not wait for each other on one GPU, so stream order is what orders them)", who, net->dev);
-            return QV_ERR_STATE;
-        }
+    if (!net->strip) { set_error("qv_strip_input: qv_strip_setup has not been called"); return QV_ERR_STATE; }
+    *d_rows = strip_slot(net->strip, slot);
     return QV_OK;
 }
 
 int qv_strip_acquire(qv_net *net, int slot, void *cuda_stream)
 {
     if (!net || slot < 0 || slot > 1) { set_error("qv_strip_acquire: bad argument"); return QV_ERR_ARG; }
-    StripState &S = net->strip;
-    if (!S.on) { set_error("qv_strip_acquire: qv_strip_setup has not been called"); return QV_ERR_STATE; }
-    int rc = set_device(net);
-    if (rc) return rc;
-    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : net->st;
-    if ((rc = check_shared_device_stream(net, st, "qv_strip_acquire"))) return rc;
-    S.last_stream = st; S.used = true;
-    const uint32_t s = S.slot_seq[slot];
-    const uint32_t *w[2] = {nullptr, nullptr};
-    for (int side = 0; side < 2; ++side) {
-        const StripPeer &P = S.peer[side];
-        if (!P.attached || s == 0) continue;
-        if (P.same_device) {
-            // the neighbour's forward that read this slot must already be on the (shared) stream
-            if (P.net->strip.forwards[slot] < S.forwards[slot]) {
-                set_error("qv_strip_acquire: the neighbour strip on the same GPU has not yet consumed slot %d (issue the strips' calls frame by frame)", slot);
-                return QV_ERR_STATE;
-            }
-        } else {
-            w[side] = reinterpret_cast<const uint32_t *>(P.base + STRIP_DONE);      // another GPU: wait for its "completed step s"
-        }
-    }
-    if (net->fm && (w[0] || w[1])) {
-        QV_CUDA(fused_wait_words(net->fm, w[0], s, w[1], s, st));
-        net->launches += 1;
-    }
-    S.fills[slot] += 1;
-    return QV_OK;
+    const int rc = strip_on(net, "qv_strip_acquire");
+    return rc ? rc : strip_acquire(net->strip, slot, net->fm, stream_of(net, cuda_stream), &net->launches);
 }
 
 int qv_strip_load(qv_net *net, int slot, const uint8_t *host_rows, void *cuda_stream)
 {
     if (!host_rows) { set_error("qv_strip_load: null argument"); return QV_ERR_ARG; }
-    int rc = qv_strip_acquire(net, slot, cuda_stream);
-    if (rc) return rc;
-    StripState &S = net->strip;
-    QV_CUDA(cudaMemcpyAsync(S.block + STRIP_HDR + (size_t)slot * S.slot_stride, host_rows, (size_t)(S.row1 - S.row0) * net->W,
-                            cudaMemcpyHostToDevice, cuda_stream ? (cudaStream_t)cuda_stream : net->st));
+    if (int rc = qv_strip_acquire(net, slot, cuda_stream)) return rc;
+    const StripRows R = strip_rows(net->strip);
+    QV_CUDA(cudaMemcpyAsync(strip_slot(net->strip, slot), host_rows, (size_t)(R.row1 - R.row0) * net->W, cudaMemcpyHostToDevice,
+                            stream_of(net, cuda_stream)));
     return QV_OK;
 }
 
-// What every forward of a strip handle needs: qv_strip_setup, a loaded model on the fused path, a neighbour on every interior edge.
-static int strip_ready(const qv_net *net, const char *who)
+static int forward_strip(qv_net *net, int slot, const uint8_t *d_ori, uint8_t *d_out, int64_t *d_sse, void *cuda_stream, const char *who)
 {
-    const StripState &S = net->strip;
-    if (!S.on) { set_error("%s: qv_strip_setup has not been called", who); return QV_ERR_STATE; }
-    if (!net->uploaded || !net->fm || net->impl == QV_IMPL_LAYERED) {
-        set_error("%s: needs a loaded model and the fused path (peer-mapped halo rows are read by the fused kernel)", who);
-        return QV_ERR_STATE;
-    }
-    if ((S.row0 > 0 && !S.peer[QV_STRIP_ABOVE].attached) || (S.row1 < S.img_h && !S.peer[QV_STRIP_BELOW].attached)) {
-        set_error("%s: rows [%d, %d) of %d have an interior edge with no neighbour attached", who, S.row0, S.row1, S.img_h);
-        return QV_ERR_STATE;
-    }
-    return QV_OK;
-}
-
-static int strip_forward(qv_net *net, int slot, const uint8_t *d_ori, uint8_t *d_out, int64_t *d_sse, void *cuda_stream, const char *who)
-{
-    StripState &S = net->strip;
-    int rc = strip_ready(net, who);
-    if (rc) return rc;
-    if (d_sse && S.img_h > FUSED_SSE_MAX_H) { set_error("%s: frame height %d exceeds %d", who, S.img_h, FUSED_SSE_MAX_H); return QV_ERR_ARG; }
-    rc = set_device(net);
-    if (rc) return rc;
-    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : net->st;
-    if ((rc = check_shared_device_stream(net, st, who))) return rc;
-    const size_t W = net->W;
-    FusedRows fr;
-    fr.own0 = fr.out0 = S.row0; fr.own1 = fr.out1 = S.row1;
-    fr.pub = reinterpret_cast<uint32_t *>(S.block + STRIP_PUB);
-    fr.done = reinterpret_cast<uint32_t *>(S.block + STRIP_DONE);
-    fr.done_ctr = reinterpret_cast<uint32_t *>(S.block + STRIP_CTR);
-    for (int side = 0; side < 2; ++side) {
-        if (side == QV_STRIP_ABOVE ? S.row0 == 0 : S.row1 == S.img_h) continue;
-        const StripPeer &P = S.peer[side];
-        const uint8_t *rows = P.base + P.d.slot_off + (size_t)slot * P.d.slot_stride;
-        const uint32_t *flag = reinterpret_cast<const uint32_t *>(P.base + STRIP_PUB);
-        if (P.same_device) {
-            // a neighbour on this very GPU: no kernel may wait for it -- its rows are ordered before this launch by the shared
-            // stream, provided its slot was filled for this frame already (checked here, on the host)
-            if (P.net->strip.fills[slot] == 0) {
-                set_error("%s: the neighbour strip on the same GPU has not filled slot %d yet (strips that share a GPU: all loads of a frame, then its forwards, on one stream)", who, slot);
-                return QV_ERR_STATE;
-            }
-            flag = nullptr;
-        }
-        if (side == QV_STRIP_ABOVE) { fr.top_rows = STRIP_HALO; fr.d_top = rows + (size_t)(P.d.row1 - P.d.row0 - STRIP_HALO) * W; fr.flag_top = flag; }
-        else { fr.bot_rows = STRIP_HALO; fr.d_bot = rows; fr.flag_bot = flag; }
-    }
-    const uint32_t seq = ++S.seq;
-    S.slot_seq[slot] = seq;
-    S.forwards[slot] += 1;
-    S.last_stream = st; S.used = true;
-    fr.seq = seq;
-    const uint8_t *own = S.block + STRIP_HDR + (size_t)slot * S.slot_stride;
-    QV_CUDA(fused_forward(net->fm, own, d_out, 1, S.img_h, net->W, st, &net->launches, &fr, d_ori, d_sse));
-    if (!cuda_stream) { QV_CUDA(cudaStreamSynchronize(st)); return kernel_report(net); }
-    return QV_OK;
+    int rc = strip_on(net, who);
+    if (!rc) rc = strip_fused(net, who);
+    if (!rc) rc = strip_forward(net->strip, slot, net->fm, d_ori, d_out, d_sse, stream_of(net, cuda_stream), &net->launches, who);
+    return rc ? rc : finish(net, cuda_stream);
 }
 
 int qv_strip_forward(qv_net *net, int slot, uint8_t *d_out, void *cuda_stream)
 {
     if (!net || !d_out || slot < 0 || slot > 1) { set_error("qv_strip_forward: bad argument"); return QV_ERR_ARG; }
-    return strip_forward(net, slot, nullptr, d_out, nullptr, cuda_stream, "qv_strip_forward");
+    return forward_strip(net, slot, nullptr, d_out, nullptr, cuda_stream, "qv_strip_forward");
 }
 
 int qv_strip_forward_sse(qv_net *net, int slot, const uint8_t *d_ori_rows, uint8_t *d_out, int64_t *d_sse2, void *cuda_stream)
 {
     // this GPU's share of vrcnn_data::psnr_pf (inference/yuv_data.cpp:98-112) for one frame; the strips' values add up
     if (!net || !d_ori_rows || !d_out || !d_sse2 || slot < 0 || slot > 1) { set_error("qv_strip_forward_sse: bad argument"); return QV_ERR_ARG; }
-    return strip_forward(net, slot, d_ori_rows, d_out, d_sse2, cuda_stream, "qv_strip_forward_sse");
+    return forward_strip(net, slot, d_ori_rows, d_out, d_sse2, cuda_stream, "qv_strip_forward_sse");
 }
 
 int qv_forward_frames_host(qv_net *net, const uint8_t *h_in, uint8_t *h_out, int n_frames)
@@ -1049,26 +840,18 @@ int qv_strip_stream_yuv_pf(qv_net *const *nets, int n_nets, const char *anchor_y
             if (nets[j] == nets[i]) { set_error("%s: handles %d and %d are the same handle", who, j, i); return QV_ERR_ARG; }
     }
     int rc;
+    std::vector<StripNet *> strips(n_nets);
     for (int i = 0; i < n_nets; ++i)
-        if ((rc = strip_ready(nets[i], who))) return rc;
-    const int img_h = nets[0]->strip.img_h, W = nets[0]->W;
+        if ((rc = strip_on(nets[i], who)) || (rc = strip_fused(nets[i], who)) || (rc = strip_ready(strips[i] = nets[i]->strip, who))) return rc;
+    auto rows = [&](int i) { return strip_rows(strips[i]); };
+    const int img_h = rows(0).img_h, W = nets[0]->W;
     for (int i = 1; i < n_nets; ++i)
-        if (nets[i]->W != W || nets[i]->strip.img_h != img_h) {
-            set_error("%s: handle %d holds rows of a %dx%d frame, handle 0 of a %dx%d frame", who, i, nets[i]->W, nets[i]->strip.img_h, W, img_h);
+        if (nets[i]->W != W || rows(i).img_h != img_h) {
+            set_error("%s: handle %d holds rows of a %dx%d frame, handle 0 of a %dx%d frame", who, i, nets[i]->W, rows(i).img_h, W, img_h);
             return QV_ERR_ARG;
         }
     if (ori_yuv && img_h > FUSED_SSE_MAX_H) { set_error("%s: frame height %d exceeds %d", who, img_h, FUSED_SSE_MAX_H); return QV_ERR_ARG; }
-    {
-        // strips that share a GPU are ordered by the one stream they are driven on, so this call must drive all of them
-        std::lock_guard<std::mutex> l(g_strip_mu);
-        for (int i = 0; i < n_nets; ++i)
-            for (qv_net *o : g_strip_nets[nets[i]->dev])
-                if (std::find(nets, nets + n_nets, o) == nets + n_nets) {
-                    set_error("%s: GPU %d also holds a strip handle that is not in this call (strips that share a GPU are driven "
-                              "together, on one stream)", who, nets[i]->dev);
-                    return QV_ERR_STATE;
-                }
-    }
+    if ((rc = strip_claim(strips.data(), n_nets, who))) return rc;
     for (int j = 0; j < n_frames; ++j) {
         if (sse_before_pf) sse_before_pf[j] = 0;
         if (sse_after_pf) sse_after_pf[j] = 0;
@@ -1085,8 +868,8 @@ int qv_strip_stream_yuv_pf(qv_net *const *nets, int n_nets, const char *anchor_y
         auto d = std::find(devices.begin(), devices.end(), nets[i]->dev);
         parts[i].hold = (int)(d - devices.begin());
         if (d == devices.end()) devices.push_back(nets[i]->dev);
-        parts[i].row0 = nets[i]->strip.row0;
-        parts[i].row1 = nets[i]->strip.row1;
+        parts[i].row0 = rows(i).row0;
+        parts[i].row1 = rows(i).row1;
     }
     struct StripDevice {
         std::vector<int> strips;
@@ -1104,11 +887,7 @@ int qv_strip_stream_yuv_pf(qv_net *const *nets, int n_nets, const char *anchor_y
     const size_t sse_bytes = (size_t)n_frames * 2 * sizeof(int64_t);
     auto bytes = [&](int i) { return (size_t)(parts[i].row1 - parts[i].row0) * W; };
     // the handles' streams are this call's from here on; at the end they are idle and free to be driven on any stream again
-    auto unbind = [&]() {
-        std::lock_guard<std::mutex> l(g_strip_mu);
-        for (int i = 0; i < n_nets; ++i) { nets[i]->strip.used = false; nets[i]->strip.last_stream = nullptr; }
-    };
-    unbind();
+    strip_unbind(strips.data(), n_nets);
     for (size_t d = 0; d < devices.size(); ++d) {
         hold[d].dev = devices[d];
         // the strips' earlier work, on whatever stream, is complete before this call moves them onto its own streams
@@ -1164,7 +943,7 @@ int qv_strip_stream_yuv_pf(qv_net *const *nets, int n_nets, const char *anchor_y
             for (size_t x = 0; rc == QV_OK && x < sum.size(); ++x) sum[x] += h_sse[x];
         }
     }
-    unbind();
+    strip_unbind(strips.data(), n_nets);
     // every handle's fused-kernel report is taken (and cleared) now that its streams are idle; the first failure's message stands
     for (int i = 0; i < n_nets; ++i) {
         if (rc == QV_OK) rc = kernel_report(nets[i]);

@@ -163,7 +163,42 @@ def test_strip_api_refuses_what_it_cannot_do(models):
     e.strip_load(0, x[0], st.cuda_stream)
     e.strip_forward(0, oo.data_ptr(), st.cuda_stream)
     e.synchronize(st.cuda_stream)
-    assert np.array_equal(oo.cpu().numpy(), e.forward_frames_host(x)[0])
+    want = e.forward_frames_host(x)[0]
+    assert np.array_equal(oo.cpu().numpy(), want)
+    # a descriptor outlives its strip: once the strip is released, attaching its descriptor is refused
+    a.strip_setup(h, 0, 20)
+    b.strip_setup(h, 20, 40)
+    old = b.strip_export()
+    b.strip_release()
+    with pytest.raises(api.QVError, match="neighbour strip was released"):
+        a.strip_attach(api.STRIP_BELOW, old)
+    # releasing a strip unlinks it from the strips that had it attached, also once it is set up again, until re-attached
+    b.strip_setup(h, 20, 40)
+    a.strip_attach(api.STRIP_BELOW, b.strip_export())
+    b.strip_attach(api.STRIP_ABOVE, a.strip_export())
+    a.strip_release()
+    with pytest.raises(api.QVError, match="no neighbour attached"):
+        b.strip_forward(0, o.data_ptr())
+    a.strip_setup(h, 0, 20)
+    with pytest.raises(api.QVError, match="no neighbour attached"):
+        b.strip_forward(0, o.data_ptr())
+    b.strip_attach(api.STRIP_ABOVE, a.strip_export())
+    a.strip_attach(api.STRIP_BELOW, b.strip_export())
+    ob = torch.empty((20, w), dtype=torch.uint8, device="cuda")
+    a.strip_load(0, x[0][:20], st.cuda_stream)
+    b.strip_load(0, x[0][20:], st.cuda_stream)
+    a.strip_forward(0, o.data_ptr(), st.cuda_stream)
+    b.strip_forward(0, ob.data_ptr(), st.cuda_stream)
+    b.synchronize(st.cuda_stream)
+    assert np.array_equal(np.vstack([o.cpu().numpy(), ob.cpu().numpy()]), want)
+    # a second strip_setup of a live strip, and qv_destroy, unlink it the same way
+    b.strip_setup(h, 20, 40)
+    with pytest.raises(api.QVError, match="no neighbour attached"):
+        a.strip_forward(0, o.data_ptr(), st.cuda_stream)
+    a.strip_attach(api.STRIP_BELOW, b.strip_export())
+    b.close()
+    with pytest.raises(api.QVError, match="no neighbour attached"):
+        a.strip_forward(0, o.data_ptr(), st.cuda_stream)
 
 
 @pytest.mark.parametrize("strips,gpus", [(3, 1), (2, 2), (4, 2), (8, 8)])

@@ -6,6 +6,6 @@ NV="/usr/local/cuda/bin/nvcc -gencode arch=compute_100a,code=sm_100a -O3 -linein
 for spec in "$@"; do
   name=${spec%%:*}; flags=${spec#*:}
   $NV $flags -c qv_fused.cu -o /tmp/qv_fused_$name.o
-  $NV -shared -o ../../tools/bin/lib_$name.so qv_formats.o qv_api.o qv_layered.o /tmp/qv_fused_$name.o -cudart static
+  $NV -shared -o ../../tools/bin/lib_$name.so qv_formats.o qv_api.o qv_strip.o qv_layered.o /tmp/qv_fused_$name.o -cudart static
   echo built lib_$name.so "($flags)"
 done
