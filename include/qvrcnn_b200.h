@@ -137,6 +137,32 @@ QV_API int qv_forward_frames_device(qv_net *net, const uint8_t *d_in, uint8_t *d
    (QV_ERR_ARG), the layered path takes any height. */
 QV_API int qv_forward_frames_device_sse(qv_net *net, const uint8_t *d_in, const uint8_t *d_ori, uint8_t *d_out,
                                         int n_frames, int64_t *d_sse, void *cuda_stream);
+/* One frame of a frame list: planar luma in device memory of the handle's GPU, rows packed (pitch = width). */
+typedef struct {
+    const uint8_t *d_in;      /* height*width bytes of planar luma */
+    uint8_t       *d_out;     /* height*width bytes; must not overlap any d_in of the list (documented, not checked) */
+    const uint8_t *d_ori;     /* original luma of the same frame, or NULL */
+    int height, width;
+} qv_frame_desc;
+/* Frames the fused path takes in one launch: the frame table travels in the kernel's parameter block, whose size is
+   limited.  Longer lists are split into several launches (qv_launch_count counts each). */
+#define QV_FRAME_LIST_LAUNCH_MAX 256
+/* Enhances n_frames frames of any sizes, each with its own pointers, as one batch: one model, per-frame geometry.  The
+   handle's own height x width is not used, so one handle serves every resolution; each frame's output is byte-identical
+   to qv_forward_frames_device on a handle of that frame's geometry.  The fused path deals the rows of all frames out to
+   the SMs together (a tick of small frames fills the GPU as one large batch does); the layered path runs the frames one
+   after another, growing its activation scratch to the largest frame.
+   Asynchronous on cuda_stream (NULL = the handle's own stream, synchronous), like qv_forward_frames_device; failures a
+   kernel reports later come from qv_synchronize.  With d_sse != NULL every descriptor must carry d_ori, and for frame j
+   the SSE of the anchor / of the reconstruction against the original is ADDED to d_sse[2j] / d_sse[2j+1] (device
+   int64), as in qv_forward_frames_device_sse.  The descriptor array is read before the call returns and may be reused at
+   once.  Validated before anything is launched: QV_ERR_ARG for a null net, a null `frames` with n_frames > 0, a
+   negative n_frames, a null d_in or d_out, a height or width below 1, a d_sse while some d_ori is NULL, a d_ori while
+   d_sse is NULL, and on the fused path, with d_sse, a height above 66051, or frames of one launch (QV_FRAME_LIST_LAUNCH_MAX)
+   whose strip columns add up to more than 2^30 rows; QV_ERR_STATE without a complete model.
+   n_frames == 0: QV_OK, nothing launched. */
+QV_API int qv_forward_frame_list_device(qv_net *net, const qv_frame_desc *frames, int n_frames, int64_t *d_sse,
+                                        void *cuda_stream);
 /* Spatially partitioned pass for one very large frame (multi-GPU strips): the frame has
    img_height x width pixels (width = the handle's); d_in points at image row `in_row0` and holds
    `in_rows` rows (the strip plus up to 6 halo rows each side); rows [out_row0, out_row1) are
@@ -239,7 +265,9 @@ QV_API int qv_get_impl(const qv_net *net);
 QV_API long long qv_launch_count(const qv_net *net);
 /* Debug taps of the LAYERED path, valid after qv_forward_blu: copies frame 0's activations to
    host as planar int8 [C][H][W] (a1: 64, a2: 48, a3: 48 channels) -- the contents of C1.v,
-   Conc1.conc, Conc2.conc in the reference (inference/qvrcnn.cu:183,202,218). */
+   Conc1.conc, Conc2.conc in the reference (inference/qvrcnn.cu:183,202,218).  After a layered
+   qv_forward_frame_list_device the scratch holds a list frame's activations, not the handle's
+   geometry: QV_ERR_STATE until the next forward of the handle's own frames. */
 QV_API int qv_get_activation(qv_net *net, int which /*1,2,3*/, int8_t *host_out);
 
 /* Test hook, needs no GPU: what the host builds for the fused kernel from a static model image (Appendix B format) --
@@ -256,6 +284,10 @@ QV_API int qv_debug_fused_tables(const void *model_image, size_t len, uint8_t *w
    tests/test_fused_units.py checks that every (frame, column, row) is covered exactly once and the load is balanced. */
 QV_API int qv_debug_fused_units(int sm_count, int n_frames, int height, int width, int row0, int row1, int row_window, int allow_line,
                                 int32_t *units, size_t *n_units, int *grid);
+/* Test hook, needs no GPU: the same for ONE launch of qv_forward_frame_list_device over n_frames (1 ..
+   QV_FRAME_LIST_LAUNCH_MAX) frames of heights[j] x widths[j]; the frame of a unit is its index in the list. */
+QV_API int qv_debug_fused_list_units(int sm_count, int n_frames, const int *heights, const int *widths, int32_t *units,
+                                     size_t *n_units, int *grid);
 
 /* ---- model-file converters (SURVEY 8f1) ------------------------------------------------- */
 /* model_qfp_HWCN2NCHW_VECT_C   inference/qvrcnn.cu:558-585 */

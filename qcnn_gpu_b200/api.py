@@ -26,12 +26,12 @@ ABI_SYMBOLS = (
     "qv_last_error", "qv_version", "qv_create", "qv_destroy", "qv_load_static_para",
     "qv_load_static_para_mem", "qv_load_static_para_hwcn", "qv_load_quant_params", "qv_read_quant_params",
     "qv_set_weights", "qv_get_quant_params", "qv_load_data", "qv_forward_blu", "qv_get_recon",
-    "qv_forward_frames_host", "qv_stream_yuv", "qv_stream_yuv_pf", "qv_forward_frames_device", "qv_forward_frames_device_sse", "qv_forward_rows_device", "qv_device_buffers",
+    "qv_forward_frames_host", "qv_stream_yuv", "qv_stream_yuv_pf", "qv_forward_frames_device", "qv_forward_frames_device_sse", "qv_forward_frame_list_device", "qv_forward_rows_device", "qv_device_buffers",
     "qv_sse_device", "qv_host_alloc", "qv_host_free",
     "qv_set_impl", "qv_get_impl", "qv_launch_count", "qv_get_activation",
     "qv_convert_model_hwcn_to_vect_c", "qv_yuv_read_luma", "qv_yuv_read_frame", "qv_yuv_write_recon",
     "qv_psnr", "qv_psnr_from_sse", "qv_solve_quant_params", "qv_write_quant_params_cpp", "qv_quantize_layer",
-    "qv_debug_fused_tables", "qv_debug_fused_units", "qv_synchronize",
+    "qv_debug_fused_tables", "qv_debug_fused_units", "qv_debug_fused_list_units", "qv_synchronize",
     "qv_strip_setup", "qv_strip_export", "qv_strip_attach", "qv_strip_input", "qv_strip_acquire", "qv_strip_load",
     "qv_strip_forward", "qv_strip_forward_sse", "qv_strip_stream_yuv_pf", "qv_strip_release",
 )
@@ -39,6 +39,12 @@ ABI_SYMBOLS = (
 CUDA_STREAM_LEGACY = 1      # cudaStreamLegacy: names the legacy default stream explicitly (NULL = "the handle's own stream")
 STRIP_ABOVE, STRIP_BELOW = 0, 1
 STRIP_DESC_BYTES = 192
+FRAME_LIST_LAUNCH_MAX = 256   # QV_FRAME_LIST_LAUNCH_MAX: frames the fused path takes in one launch of a frame list
+
+
+class FrameDesc(C.Structure):
+    """qv_frame_desc: one frame of qv_forward_frame_list_device."""
+    _fields_ = [("d_in", C.c_void_p), ("d_out", C.c_void_p), ("d_ori", C.c_void_p), ("height", C.c_int), ("width", C.c_int)]
 
 
 def stream_arg(stream: int):
@@ -88,6 +94,8 @@ def lib():
         L.qv_host_free.restype = None
         L.qv_stream_yuv.argtypes = [vp, cp, cp, cp, i32, i32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         L.qv_stream_yuv_pf.argtypes = [vp, cp, cp, cp, i32, i32, vp, vp]
+        L.qv_forward_frame_list_device.argtypes = [vp, C.POINTER(FrameDesc), i32, vp, vp]
+        L.qv_debug_fused_list_units.argtypes = [i32, i32, vp, vp, vp, C.POINTER(C.c_size_t), C.POINTER(i32)]
         L.qv_forward_rows_device.argtypes = [vp, vp, i32, i32, i32, vp, i32, i32, vp]
         L.qv_sse_device.argtypes = [vp, vp, C.c_size_t, vp, vp]
         L.qv_set_impl.argtypes = [vp, i32]
@@ -135,7 +143,7 @@ class QVRCNN:
 
     def __init__(self, gpu_num: int, batch: int, channel: int, height: int, width: int):
         self._h = C.c_void_p()
-        self.batch, self.channel, self.height, self.width = batch, channel, height, width
+        self.gpu_num, self.batch, self.channel, self.height, self.width = gpu_num, batch, channel, height, width
         _check(lib().qv_create(gpu_num, batch, channel, height, width, C.byref(self._h)))
 
     def close(self) -> None:
@@ -227,6 +235,29 @@ class QVRCNN:
         pair d_sse[2f], d_sse[2f + 1]."""
         _check(lib().qv_forward_frames_device_sse(self._h, d_in, d_ori, d_out, n, d_sse, stream or None))
 
+    def forward_frame_list_device(self, frames, d_sse=None, stream: int = 0) -> None:
+        """qv_forward_frame_list_device: `frames` is a sequence of (input, output) or (input, output, original) tuples of
+        contiguous 2-D uint8 tensors of one frame each (height x width, any size per frame) on the handle's GPU; with
+        `d_sse`, an int64 tensor of [len(frames)][2] on that GPU, the SSEs of frame j against its original are ADDED to
+        d_sse[j].  `stream` as in forward_frames_device (0 = the handle's own stream, synchronous)."""
+        def on_gpu(t):
+            return t.is_cuda and t.device.index == self.gpu_num
+
+        descs = (FrameDesc * max(1, len(frames)))()
+        for j, fr in enumerate(frames):
+            x, y = fr[0], fr[1]
+            ori = fr[2] if len(fr) > 2 else None
+            for t in (x, y) + ((ori,) if ori is not None else ()):
+                if t.dim() != 2 or not t.is_contiguous() or t.shape != x.shape or str(t.dtype) != "torch.uint8" or not on_gpu(t):
+                    raise ValueError("frame %d: every tensor must be one contiguous uint8 height x width frame of one shape on "
+                                     "cuda:%d" % (j, self.gpu_num))
+            descs[j] = FrameDesc(x.data_ptr(), y.data_ptr(), ori.data_ptr() if ori is not None else None, x.shape[0], x.shape[1])
+        if d_sse is not None and (str(d_sse.dtype) != "torch.int64" or not d_sse.is_contiguous() or d_sse.numel() < 2 * len(frames)
+                                  or not on_gpu(d_sse)):
+            raise ValueError("d_sse must be a contiguous int64 tensor of at least [len(frames)][2] on cuda:%d" % self.gpu_num)
+        _check(lib().qv_forward_frame_list_device(self._h, descs, len(frames), d_sse.data_ptr() if d_sse is not None else None,
+                                                  stream or None))
+
     def forward_rows_device(self, d_in: int, img_height: int, in_row0: int, in_rows: int, d_out: int,
                             out_row0: int, out_row1: int, stream: int = 0) -> None:
         _check(lib().qv_forward_rows_device(self._h, d_in, img_height, in_row0, in_rows, d_out, out_row0,
@@ -302,6 +333,21 @@ def strip_stream_yuv_pf(nets, anchor_yuv: str, ori_yuv: Optional[str], recon_yuv
     _check(lib().qv_strip_stream_yuv_pf(handles, len(nets), enc(anchor_yuv), enc(ori_yuv), enc(recon_yuv), first_frame, n_frames,
                                         before.ctypes.data if ori_yuv else None, after.ctypes.data if ori_yuv else None))
     return before, after
+
+
+def fused_list_units(sm_count: int, heights, widths):
+    """qv_debug_fused_list_units (no GPU): the work units of one frame-list launch, an int32 array of rows (cta, frame,
+    strip column, y0, y1), and the grid."""
+    L = lib()
+    h = np.ascontiguousarray(heights, np.int32)
+    w = np.ascontiguousarray(widths, np.int32)
+    if h.shape != w.shape or h.ndim != 1:
+        raise ValueError("heights and widths must be two 1-D sequences of one length")
+    cnt, grid = C.c_size_t(0), C.c_int(0)
+    _check(L.qv_debug_fused_list_units(sm_count, len(h), h.ctypes.data, w.ctypes.data, None, C.byref(cnt), C.byref(grid)))
+    u = np.zeros((cnt.value, 5), np.int32)
+    _check(L.qv_debug_fused_list_units(sm_count, len(h), h.ctypes.data, w.ctypes.data, u.ctypes.data, C.byref(cnt), C.byref(grid)))
+    return u, grid.value
 
 
 def sse_device(d_a: int, d_b: int, n: int, d_accum: int, stream: int = 0) -> None:

@@ -193,6 +193,21 @@ int qv_debug_fused_units(int sm_count, int n_frames, int height, int width, int 
     return QV_OK;
 }
 
+int qv_debug_fused_list_units(int sm_count, int n_frames, const int *heights, const int *widths, int32_t *units, size_t *n_units, int *grid)
+{
+    if (!n_units || !grid || !heights || !widths) { set_error("qv_debug_fused_list_units: null argument"); return QV_ERR_ARG; }
+    std::vector<int> u;
+    int g = 0;
+    if (fused_debug_list_units(sm_count, n_frames, heights, widths, u, g)) {
+        set_error("qv_debug_fused_list_units: bad list");
+        return QV_ERR_ARG;
+    }
+    if (units && *n_units >= u.size() / 5) memcpy(units, u.data(), u.size() * sizeof(int));
+    *n_units = u.size() / 5;
+    *grid = g;
+    return QV_OK;
+}
+
 int qv_load_static_para(qv_net *net, const char *filename)
 {
     if (!net) { set_error("qv_load_static_para: null handle"); return QV_ERR_ARG; }
@@ -319,6 +334,37 @@ int qv_forward_frames_device_sse(qv_net *net, const uint8_t *d_in, const uint8_t
     // per-frame form of vrcnn_data::psnr_pf (inference/yuv_data.cpp:98-112): exact integer SSEs, incremented
     if (!net || !d_in || !d_ori || !d_out || !d_sse || n_frames < 0) { set_error("qv_forward_frames_device_sse: bad argument"); return QV_ERR_ARG; }
     return forward_frames_device(net, d_in, d_ori, d_out, n_frames, d_sse, cuda_stream);
+}
+
+int qv_forward_frame_list_device(qv_net *net, const qv_frame_desc *frames, int n_frames, int64_t *d_sse, void *cuda_stream)
+{
+    if (!net || n_frames < 0 || (n_frames > 0 && !frames)) { set_error("qv_forward_frame_list_device: bad argument"); return QV_ERR_ARG; }
+    for (int j = 0; j < n_frames; ++j) {
+        const qv_frame_desc &f = frames[j];
+        if (!f.d_in || !f.d_out || f.height < 1 || f.width < 1) {
+            set_error("qv_forward_frame_list_device: frame %d: null pointer or bad geometry %dx%d", j, f.width, f.height);
+            return QV_ERR_ARG;
+        }
+        if (!f.d_ori != !d_sse) {
+            set_error("qv_forward_frame_list_device: frame %d: %s", j, d_sse ? "d_sse given but no d_ori" : "d_ori given but no d_sse");
+            return QV_ERR_ARG;
+        }
+    }
+    if (n_frames == 0) return QV_OK;
+    if (!net->uploaded || (runs_fused(net) && !net->fm)) { set_error("forward called before a complete model (weights + quant params) was loaded"); return QV_ERR_STATE; }
+    const bool fused = runs_fused(net);
+    for (int j = 0; fused && d_sse && j < n_frames; ++j)
+        if (frames[j].height > FUSED_SSE_MAX_H) { set_error("per-frame SSE: frame %d height %d exceeds %d", j, frames[j].height, FUSED_SSE_MAX_H); return QV_ERR_ARG; }
+    if (fused && !fused_list_ok(net->fm, frames, n_frames, d_sse != nullptr)) {
+        set_error("qv_forward_frame_list_device: the frames of one launch exceed 2^30 strip-column rows");
+        return QV_ERR_ARG;
+    }
+    int rc = set_device(net);
+    if (rc) return rc;
+    const cudaStream_t st = stream_of(net, cuda_stream);
+    if (fused) QV_CUDA(fused_forward_list(net->fm, frames, n_frames, d_sse, st, &net->launches));
+    else if ((rc = layered_forward_list(net->ln, frames, n_frames, d_sse, st, &net->launches))) return rc;
+    return finish(net, cuda_stream);
 }
 
 int qv_forward_rows_device(qv_net *net, const uint8_t *d_in, int img_height, int in_row0, int in_rows, uint8_t *d_out,

@@ -55,6 +55,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <type_traits>
 #include <vector>
@@ -168,6 +169,23 @@ struct alignas(64) FusedParams {
     unsigned long long *sse;
 };
 
+// Frame lists (k_enh_list): the frame table of one launch, passed by value behind FusedParams in the kernel parameters, so
+// that it needs no device copy and no lifetime rule.  The units are cut from one row line over every (frame, strip column)
+// column, column c of frame f being H_f rows long: line0 / col0 are the line position and the index of the frame's first
+// column, and the entry behind the last frame holds the line length and the column count.
+struct ListFrame {
+    const uint8_t *in;
+    uint8_t *out;
+    const uint8_t *ori;
+    int H, W, line0, col0;
+};
+struct alignas(64) FusedListParams {
+    FusedParams p;                     // first member: the body's P is this, at the offsets every other kernel uses
+    ListFrame fr[QV_FRAME_LIST_LAUNCH_MAX + 1];
+};
+static_assert(sizeof(FusedListParams) <= 32764, "exceeds the kernel-parameter limit: lower QV_FRAME_LIST_LAUNCH_MAX");
+static_assert(std::is_standard_layout<FusedListParams>::value, "list_of() reads the table through a FusedParams reference");
+
 // Operands of the 27 MMAs of one row iteration, for each of the 12 phases R1 mod 12 (the ring rotations have periods 2,
 // 3, 4 and 6).  PhaseBases / FixedBases are the host-side description (what rotates, what does not); PhaseOps is its
 // expansion into ready-made descriptors in constant memory, so that the MMA warp needs uniform-datapath loads only:
@@ -263,6 +281,68 @@ __host__ __device__ __forceinline__ UnitGeo unit_geo(const FusedParams &P, int u
     return g;
 }
 
+// The frame table of a k_enh_list launch, from the FusedParams at its start.
+__host__ __device__ __forceinline__ const FusedListParams &list_of(const FusedParams &P)
+{
+    return reinterpret_cast<const FusedListParams &>(P);
+}
+
+// The last frame of the list whose first column starts at or before line position (by_col: column index) v.  A binary
+// search over the table's prefix sums, once per unit.
+__host__ __device__ __forceinline__ int list_find(const FusedListParams &L, int v, bool by_col)
+{
+    int lo = 0, hi = L.p.n_frames - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if ((by_col ? L.fr[mid].col0 : L.fr[mid].line0) <= v) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// Frame lists: CTA b takes [b * chunk, (b + 1) * chunk) of the row line, and unit b + j * grid is the part of it in the j-th
+// column it touches, as in the whole-frame line but without the column permutation (unit_geo): g.f is the frame's index in
+// the launch.
+__host__ __device__ __forceinline__ UnitGeo list_unit_geo(const FusedListParams &L, int unit, int grid)
+{
+    const int n = L.p.n_frames, b = unit % grid, j = unit / grid;
+    const int lo = b * L.p.seg_rows, hi = min(L.fr[n].line0, lo + L.p.seg_rows);
+    UnitGeo g{0, 0, 0, 0, false};
+    if (lo >= hi) return g;
+    int f = list_find(L, lo, false);
+    const int col = L.fr[f].col0 + (lo - L.fr[f].line0) / L.fr[f].H + j;
+    if (col >= L.fr[n].col0) return g;
+    if (j > 0) f = list_find(L, col, true);
+    const ListFrame &F = L.fr[f];
+    g.f = f;
+    g.strip = col - F.col0;
+    const int c0 = F.line0 + g.strip * F.H;          // line position of the column's first row
+    const int start = max(lo, c0), end = min(hi, c0 + F.H);
+    g.y0 = start - c0;
+    g.y1 = end - c0;
+    g.ok = start < end;
+    return g;
+}
+
+// What the kernel body calls: the unit's geometry, and H / W of the frame it belongs to.  The if constexpr keeps the frame
+// table out of every other kernel's code, and H / W of those stay the values the body read from P once at its start
+// (reading P.H again per unit, behind the loops' asm volatile memory clobbers, changes their instruction streams).
+template <bool ROWS, bool LIST>
+__device__ __forceinline__ UnitGeo unit_at(const FusedParams &P, int unit, int H, int grid)
+{
+    if constexpr (LIST) return list_unit_geo(list_of(P), unit, grid);
+    else return unit_geo<ROWS>(P, unit, H, grid);
+}
+template <bool LIST> __device__ __forceinline__ int frame_h(const FusedParams &P, int f, int H)
+{
+    if constexpr (LIST) return list_of(P).fr[f].H;
+    else return H;
+}
+template <bool LIST> __device__ __forceinline__ int frame_w(const FusedParams &P, int f, int W)
+{
+    if constexpr (LIST) return list_of(P).fr[f].W;
+    else return W;
+}
+
 // workers / C4 warps -> MMA warp, event ev: every lane arrives on named barrier 2 + ev mod 3, the MMA warp blocks in
 // bar.sync on the same id.  A warp blocked there issues nothing (a warp polling an mbarrier does, and on the MMA warp's SM
 // sub-partition that is measurable: DESIGN.md section 7) and is released ~40 cycles after the last arrival.  Three ids are
@@ -336,7 +416,7 @@ __device__ __forceinline__ void c4_taps(const uint4 (&v)[3], const FusedParams &
 template <bool FAST, bool PROF, bool ROWS, bool TMA = false>
 __global__ void __launch_bounds__(NTHREADS, 1) k_fused(const __grid_constant__ FusedParams P)
 {
-    constexpr bool SSE = false;
+    constexpr bool SSE = false, LIST = false;
 #include "qv_fused_body.inc"
 }
 
@@ -348,7 +428,18 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_fused(const __grid_constant__ F
 template <bool FAST, bool ROWS>
 __global__ void __launch_bounds__(NTHREADS, 1) k_enh_sse(const __grid_constant__ FusedParams P)
 {
-    constexpr bool SSE = true, PROF = false, TMA = false;
+    constexpr bool SSE = true, PROF = false, TMA = false, LIST = false;
+#include "qv_fused_body.inc"
+}
+
+// Frames of different sizes in one launch (qv_forward_frame_list_device), with (SSE) or without the per-frame SSEs: every
+// unit reads its frame's pointers and geometry from the frame table behind P.  Its own name, so that the k_fused /
+// k_enh_sse builds stay what they are.
+template <bool FAST, bool SSE>
+__global__ void __launch_bounds__(NTHREADS, 1) k_enh_list(const __grid_constant__ FusedListParams PL)
+{
+    constexpr bool PROF = false, ROWS = false, TMA = false, LIST = true;
+    const FusedParams &P = PL.p;
 #include "qv_fused_body.inc"
 }
 
@@ -608,6 +699,10 @@ FusedModel *fused_upload(const ModelHost &m, cudaStream_t st)
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_sse<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_sse<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_sse<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_list<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_list<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_list<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_list<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k_bases, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
     int dev = 0, sms = 148;
     if (e == cudaSuccess) e = cudaGetDevice(&dev);
@@ -772,6 +867,101 @@ int fused_debug_units(int sm_count, int n_frames, int H, int W, int row0, int ro
         units.insert(units.end(), v, v + 5);
     }
     return 0;
+}
+
+// The plan of one frame-list launch: fills the frame table and the geometry fields of L.p that list_unit_geo reads and returns
+// the grid.  The row line over all (frame, strip column) columns is cut into one equal chunk per SM, as plan_units' line;
+// a chunk pays PIPE iterations of pipeline fill per column it touches.
+static cudaError_t plan_list(FusedListParams &L, const qv_frame_desc *frames, int n, int sm_count, int &grid)
+{
+    if (n < 1 || n > QV_FRAME_LIST_LAUNCH_MAX || sm_count < 1) return cudaErrorInvalidValue;
+    long long line = 0, cols = 0;
+    for (int f = 0; f < n; ++f) {
+        const qv_frame_desc &fr = frames[f];
+        if (fr.height < 1 || fr.width < 1) return cudaErrorInvalidValue;
+        L.fr[f] = ListFrame{fr.d_in, fr.d_out, fr.d_ori, fr.height, fr.width, (int)line, (int)cols};
+        const long long nstrips = (fr.width + WT - 1) / WT;
+        line += nstrips * fr.height;
+        cols += nstrips;
+        if (line > 0x3fffffffll) return cudaErrorInvalidValue;
+    }
+    L.fr[n] = ListFrame{nullptr, nullptr, nullptr, 0, 0, (int)line, (int)cols};
+    FusedParams &P = L.p;
+    P.n_frames = n;
+    grid = (int)std::max<long long>(1, std::min<long long>(sm_count, line / 32));
+    const int chunk = (int)((line + grid - 1) / grid);
+    grid = (int)((line + chunk - 1) / chunk);
+    // units per CTA: the columns its chunk touches, at most
+    int pieces = 1;
+    for (int b = 0; b < grid; ++b) {
+        const int lo = b * chunk, last = (int)std::min<long long>(line, (long long)lo + chunk) - 1;
+        auto col_at = [&](int v) { const int f = list_find(L, v, false); return L.fr[f].col0 + (v - L.fr[f].line0) / L.fr[f].H; };
+        pieces = std::max(pieces, col_at(last) - col_at(lo) + 1);
+    }
+    if ((long long)grid * pieces > 0x7fffffffll) return cudaErrorInvalidValue;
+    P.seg_rows = chunk;
+    P.n_units = grid * pieces;
+    P.nseg = 1;
+    P.linear = 1;
+    return cudaSuccess;
+}
+
+int fused_debug_list_units(int sm_count, int n_frames, const int *H, const int *W, std::vector<int> &units, int &grid)
+{
+    if (n_frames < 1 || n_frames > QV_FRAME_LIST_LAUNCH_MAX) return -1;
+    std::vector<qv_frame_desc> fr(n_frames);
+    for (int f = 0; f < n_frames; ++f) fr[f] = qv_frame_desc{nullptr, nullptr, nullptr, H[f], W[f]};
+    std::unique_ptr<FusedListParams> L(new FusedListParams{});
+    if (plan_list(*L, fr.data(), n_frames, sm_count, grid) != cudaSuccess) return -1;
+    units.clear();
+    for (int u = 0; u < L->p.n_units; ++u) {
+        const UnitGeo g = list_unit_geo(*L, u, grid);
+        if (!g.ok) continue;
+        const int v[5] = {u % grid, g.f, g.strip, g.y0, g.y1};
+        units.insert(units.end(), v, v + 5);
+    }
+    return 0;
+}
+
+bool fused_list_ok(const FusedModel *fm, const qv_frame_desc *frames, int n, bool sse)
+{
+    for (int f = 0; f < n; ++f)
+        if (sse ? !frames[f].d_ori || frames[f].height > FUSED_SSE_MAX_H : frames[f].d_ori != nullptr) return false;
+    std::unique_ptr<FusedListParams> L(new FusedListParams{});      // 12 KB: not on the stack
+    int grid = 1;
+    for (int f0 = 0; f0 < n; f0 += QV_FRAME_LIST_LAUNCH_MAX)
+        if (plan_list(*L, frames + f0, std::min(QV_FRAME_LIST_LAUNCH_MAX, n - f0), fm->sm_count, grid) != cudaSuccess) return false;
+    return true;
+}
+
+cudaError_t fused_forward_list(const FusedModel *fm, const qv_frame_desc *frames, int n, int64_t *d_sse, cudaStream_t st, long long *launches)
+{
+    if (!fused_list_ok(fm, frames, n, d_sse != nullptr)) return cudaErrorInvalidValue;      // every launch's plan, before the first
+    std::unique_ptr<FusedListParams> L(new FusedListParams{});
+    for (int f0 = 0; f0 < n; f0 += QV_FRAME_LIST_LAUNCH_MAX) {
+        const int c = std::min(QV_FRAME_LIST_LAUNCH_MAX, n - f0);
+        FusedParams &P = L->p;
+        P = fm->proto;
+        P.in = nullptr; P.out = nullptr; P.ori = nullptr;
+        P.sse = d_sse ? reinterpret_cast<unsigned long long *>(d_sse + 2 * (size_t)f0) : nullptr;
+        P.H = P.W = 0;
+        P.frame_stride = 0;
+        P.ys = P.ye = P.own0 = P.own1 = P.rlo = P.rhi = 0;
+        P.in_top = P.in_bot = nullptr; P.flag_top = P.flag_bot = nullptr;
+        P.pub = P.done = P.done_ctr = nullptr; P.seq = 0;
+        P.dbg = nullptr;
+        P.dbg_flags = 0;
+        if (fm->env_test_fail) P.sbase16 ^= 1u;
+        int grid = 1;
+        if (const cudaError_t e = plan_list(*L, frames + f0, c, fm->sm_count, grid)) return e;
+        if (d_sse && fm->fast) k_enh_list<true, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(*L);
+        else if (d_sse) k_enh_list<false, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(*L);
+        else if (fm->fast) k_enh_list<true, false><<<grid, NTHREADS, SMEM_BYTES, st>>>(*L);
+        else k_enh_list<false, false><<<grid, NTHREADS, SMEM_BYTES, st>>>(*L);
+        if (launches) *launches += 1;
+        if (const cudaError_t e = cudaGetLastError()) return e;
+    }
+    return cudaSuccess;
 }
 
 cudaError_t fused_forward(const FusedModel *fm, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W, cudaStream_t st,

@@ -34,6 +34,15 @@ constexpr int FUSED_SSE_MAX_H = 66051;     // per-thread column sums are 32-bit:
 cudaError_t fused_forward(const FusedModel *fm, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W,
                           cudaStream_t st, long long *launches, const FusedRows *rows = nullptr,
                           const uint8_t *d_ori = nullptr, int64_t *d_sse = nullptr);
+// Frames of any sizes, one model (qv_forward_frame_list_device): k_enh_list, one launch per QV_FRAME_LIST_LAUNCH_MAX frames,
+// each adding 1 to *launches.  With d_sse every frame carries d_ori and height <= FUSED_SSE_MAX_H, and the SSE pair of frame j is
+// ADDED to d_sse[2j], d_sse[2j + 1]; without it no frame carries d_ori.  Otherwise (fused_list_ok) cudaErrorInvalidValue
+// before any launch.
+// Whether fused_forward_list takes the list: the d_ori / d_sse rule above, and every launch's row line fits the planner
+// (at most 2^30 row iterations).
+bool fused_list_ok(const FusedModel *fm, const qv_frame_desc *frames, int n, bool sse);
+cudaError_t fused_forward_list(const FusedModel *fm, const qv_frame_desc *frames, int n, int64_t *d_sse, cudaStream_t st,
+                               long long *launches);
 // Stream-ordered helper of the strip protocol: spin (bounded) until *a >= va and *b >= vb (either pointer may be null; the
 // words live on OTHER GPUs), reporting a timeout through the model's failure word (code 3).
 cudaError_t fused_wait_words(const FusedModel *fm, const uint32_t *a, uint32_t va, const uint32_t *b, uint32_t vb, cudaStream_t st);
@@ -46,5 +55,7 @@ int fused_take_failure(const FusedModel *fm);
 void fused_debug_tables(const ModelHost &m, std::vector<uint8_t> &wimg, std::vector<uint32_t> &ops, std::vector<int32_t> &consts);
 // test hook: how a launch is dealt out to the persistent CTAs (5 ints per unit: cta, frame, strip column, y0, y1); no GPU needed
 int fused_debug_units(int sm_count, int n_frames, int H, int W, int row0, int row1, bool rows_mode, bool allow_linear, std::vector<int> &units, int &grid);
+// test hook: the same for one frame-list launch (the frame of a unit is its index in the list)
+int fused_debug_list_units(int sm_count, int n_frames, const int *H, const int *W, std::vector<int> &units, int &grid);
 
 }  // namespace qv

@@ -244,6 +244,9 @@ struct LayeredNet {
     // of fp32 `u` tensors which this design never materialises.
     int8_t *a1 = nullptr, *a2 = nullptr, *a3 = nullptr;
     int act_frames = 0;
+    bool act_list = false;                      // a1..a3 hold a frame list's last frame (layered_activation refuses)
+    size_t act_px = 0;                          // pixels a1..a3 hold (0: not allocated): act_frames x H x W, or more once a
+                                                // frame list grew them
     uint8_t *rows = nullptr;                    // the window of layered_forward_rows, run as an image of its own
     size_t rows_bytes = 0;
     cudaEvent_t ev = nullptr;                   // recorded after the last launch or copy of every call that uses a1..a3 / rows
@@ -341,20 +344,37 @@ static cudaError_t launch_conv(const int8_t *in, int8_t *out, const LayeredLayer
     return cudaGetLastError();
 }
 
-// The scratch is allocated at the first forward; n frames run in chunks of as many frames as it holds.
+// Activation scratch of at least px pixels (and of min(batch, 8) frames of the handle's geometry at the least).  Growing it
+// waits for its last user, on whatever stream.
+static int ensure_scratch(LayeredNet *ln, size_t px)
+{
+    const int frames = std::min(ln->batch, 8);
+    px = std::max(px, (size_t)frames * ln->H * ln->W);
+    if (ln->act_px && px <= ln->act_px) return QV_OK;
+    QV_CUDA(cudaEventSynchronize(ln->ev));
+    cudaFree(ln->a1); cudaFree(ln->a2); cudaFree(ln->a3);
+    ln->a1 = ln->a2 = ln->a3 = nullptr;
+    ln->act_px = 0;
+    QV_CUDA(cudaMalloc(&ln->a1, px * 64));
+    QV_CUDA(cudaMalloc(&ln->a2, px * 48));
+    QV_CUDA(cudaMalloc(&ln->a3, px * 48));
+    ln->act_frames = frames;
+    ln->act_px = px;
+    return QV_OK;
+}
+
+// The scratch is allocated at the first forward; n frames run in chunks of as many frames of the handle's geometry as it
+// was made for.
 int layered_forward(LayeredNet *ln, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W, cudaStream_t st,
                     long long *launches, const uint8_t *d_ori, int64_t *d_sse)
 {
-    if (!ln->a1) {
-        const int frames = std::min(ln->batch, 8);
-        const size_t px = (size_t)frames * ln->H * ln->W;
-        QV_CUDA(cudaMalloc(&ln->a1, px * 64));
-        QV_CUDA(cudaMalloc(&ln->a2, px * 48));
-        QV_CUDA(cudaMalloc(&ln->a3, px * 48));
-        ln->act_frames = frames;
+    if (!ln->act_px) {
+        const int rc = ensure_scratch(ln, 0);
+        if (rc) return rc;
     }
+    ln->act_list = false;
     const size_t cap_px = (size_t)ln->act_frames * ln->H * ln->W, fpx = (size_t)H * W;
-    if (fpx > cap_px) { set_error("frame of %dx%d exceeds the handle's activation scratch", W, H); return QV_ERR_ARG; }
+    if (fpx > ln->act_px) { set_error("frame of %dx%d exceeds the handle's activation scratch", W, H); return QV_ERR_ARG; }
     QV_CUDA(cudaStreamWaitEvent(st, ln->ev, 0));
     const int chunk = (int)std::max<size_t>(1, cap_px / fpx);
     const LayeredLayer *L = ln->L;
@@ -386,6 +406,19 @@ int layered_forward(LayeredNet *ln, const uint8_t *d_in, uint8_t *d_out, int n, 
     return QV_OK;
 }
 
+int layered_forward_list(LayeredNet *ln, const qv_frame_desc *frames, int n, int64_t *d_sse, cudaStream_t st, long long *launches)
+{
+    size_t px = 0;
+    for (int j = 0; j < n; ++j) px = std::max(px, (size_t)frames[j].height * frames[j].width);
+    int rc = ensure_scratch(ln, px);
+    for (int j = 0; j < n && !rc; ++j) {
+        const qv_frame_desc &f = frames[j];
+        rc = layered_forward(ln, f.d_in, f.d_out, 1, f.height, f.width, st, launches, d_sse ? f.d_ori : nullptr, d_sse ? d_sse + 2 * (size_t)j : nullptr);
+    }
+    ln->act_list = true;
+    return rc;
+}
+
 int layered_forward_rows(LayeredNet *ln, const uint8_t *d_in, int in_rows, uint8_t *d_out, int out0, int out1, cudaStream_t st,
                          long long *launches)
 {
@@ -410,7 +443,8 @@ int layered_forward_rows(LayeredNet *ln, const uint8_t *d_in, int in_rows, uint8
 
 int layered_activation(LayeredNet *ln, int which, int8_t *host_out, cudaStream_t st)
 {
-    if (!ln->a1) { set_error("qv_get_activation: the layered path has not run on this handle"); return QV_ERR_STATE; }
+    if (!ln->act_px) { set_error("qv_get_activation: the layered path has not run on this handle"); return QV_ERR_STATE; }
+    if (ln->act_list) { set_error("qv_get_activation: the last layered forward was a frame list, not the handle's geometry"); return QV_ERR_STATE; }
     const int C = which == 1 ? 64 : 48;
     const int8_t *src = which == 1 ? ln->a1 : (which == 2 ? ln->a2 : ln->a3);
     const size_t HW = (size_t)ln->H * ln->W, n = HW * C;
