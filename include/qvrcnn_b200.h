@@ -47,7 +47,7 @@ enum {
 
 /* Kernel implementation selector (qv_set_impl). */
 enum {
-    QV_IMPL_AUTO = 0,     /* fused tcgen05 path when available, else per-layer */
+    QV_IMPL_AUTO = 0,     /* the fused tcgen05 path; qv_get_impl reports QV_IMPL_LAYERED until a model is loaded */
     QV_IMPL_LAYERED = 1,  /* per-layer CUDA-core dp4a kernels, activations in HBM */
     QV_IMPL_FUSED = 2     /* whole net fused per strip, tcgen05.mma kind::i8 + TMEM */
 };
@@ -70,7 +70,9 @@ QV_API int qv_destroy(qv_net *net);
    inference/cnn.cu:90-112.  Reads the 60 028-byte NCHW_VECT_C static model file.
    Returns QV_ERR_RANGE if some output channel has 128*sum|w| + |b| >= 2^24: beyond that the
    reference's fp32 materialisation of u (inference/mat.cuh:69-70) stops being exact integer
-   arithmetic and this integer implementation would not be bit-identical. */
+   arithmetic and this integer implementation would not be bit-identical.  Every load call that completes the model
+   builds the device images of both implementations; QV_ERR_CUDA if that fails, and the handle then holds no model
+   (forwards return QV_ERR_STATE until a load succeeds). */
 QV_API int qv_load_static_para(qv_net *net, const char *filename);
 /* Same record stream from memory (for callers that hold the model image already). */
 QV_API int qv_load_static_para_mem(qv_net *net, const void *image, size_t len);

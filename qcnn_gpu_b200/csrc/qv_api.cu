@@ -47,8 +47,8 @@ static int set_device(const qv_net *net) { QV_CUDA(cudaSetDevice(net->dev)); ret
 // The stream of an entry point's cuda_stream argument: null names the handle's own.
 static cudaStream_t stream_of(const qv_net *net, void *cuda_stream) { return cuda_stream ? (cudaStream_t)cuda_stream : net->st; }
 
-// Does this handle run the fused kernel?  QV_IMPL_AUTO picks it whenever it is built.
-static bool runs_fused(const qv_net *net) { return net->impl == QV_IMPL_FUSED || (net->impl == QV_IMPL_AUTO && net->fm); }
+// Does this handle run the fused kernel?  QV_IMPL_AUTO picks it once a model is loaded.
+static bool runs_fused(const qv_net *net) { return net->impl == QV_IMPL_FUSED || (net->impl == QV_IMPL_AUTO && net->uploaded); }
 
 static int validate_qparams(const ModelHost &m)
 {
@@ -66,7 +66,8 @@ static int validate_qparams(const ModelHost &m)
     return QV_OK;
 }
 
-// Called whenever the host model changed; (re)builds device images once the model is complete.
+// Called whenever the host model changed; (re)builds device images once the model is complete.  If one cannot be built the
+// handle holds no model (uploaded = false); fm is replaced only by a new one, so once set it is never null again.
 static int sync_model(qv_net *net)
 {
     net->uploaded = false;
@@ -77,8 +78,10 @@ static int sync_model(qv_net *net)
     if (rc) return rc;
     if ((rc = set_device(net))) return rc;
     if ((rc = layered_load(net->ln, net->model, net->st))) return rc;
-    if (net->fm) { fused_free(net->fm); net->fm = nullptr; }
-    net->fm = fused_upload(net->model, net->st);     // may be null when the fused path is not built
+    FusedModel *fm = nullptr;
+    if ((rc = fused_upload(net->model, net->st, &fm))) return rc;
+    fused_free(net->fm);
+    net->fm = fm;
     net->uploaded = true;
     return QV_OK;
 }
@@ -94,10 +97,7 @@ static int run_forward(qv_net *net, const uint8_t *d_in, uint8_t *d_out, int n, 
         return QV_ERR_STATE;
     }
     if (!runs_fused(net)) return layered_forward(net->ln, d_in, d_out, n, H, W, st, &net->launches, d_ori, d_sse);
-    if (!net->fm) { set_error("fused tcgen05 path is not available in this build"); return QV_ERR_STATE; }
-    if (d_sse && H > FUSED_SSE_MAX_H) { set_error("per-frame SSE: frame height %d exceeds %d", H, FUSED_SSE_MAX_H); return QV_ERR_ARG; }
-    QV_CUDA(fused_forward(net->fm, d_in, d_out, n, H, W, st, &net->launches, nullptr, d_ori, d_sse));
-    return QV_OK;
+    return fused_forward(net->fm, d_in, d_out, n, H, W, st, &net->launches, nullptr, d_ori, d_sse);
 }
 
 extern "C" {
@@ -138,7 +138,7 @@ int qv_destroy(qv_net *net)
     if (net->st) cudaStreamSynchronize(net->st);
     qv_strip_release(net);
     layered_free(net->ln);
-    if (net->fm) fused_free(net->fm);
+    fused_free(net->fm);
     cudaFree(net->d_x); cudaFree(net->d_rec);
     for (int i = 0; i < 2; ++i) {
         cudaFree(net->d_slot_in[i]); cudaFree(net->d_slot_out[i]);
@@ -278,7 +278,7 @@ int qv_load_data(qv_net *net, const uint8_t *host_luma)
 // After a synchronisation: did a CTA of the fused kernel report a failure?  (Never a silent wrong answer.)
 static int kernel_report(qv_net *net)
 {
-    const int f = net->fm ? fused_take_failure(net->fm) : 0;
+    const int f = fused_take_failure(net->fm);
     if (!f) return QV_OK;
     set_error(f == 2 ? "fused kernel: a CTA saw other shared-memory / TMEM bases than the operand table was built for"
               : f == 3 ? "strip mode: a neighbour GPU's rows were never published (the frame data of this call is not valid)"
@@ -351,20 +351,13 @@ int qv_forward_frame_list_device(qv_net *net, const qv_frame_desc *frames, int n
         }
     }
     if (n_frames == 0) return QV_OK;
-    if (!net->uploaded || (runs_fused(net) && !net->fm)) { set_error("forward called before a complete model (weights + quant params) was loaded"); return QV_ERR_STATE; }
-    const bool fused = runs_fused(net);
-    for (int j = 0; fused && d_sse && j < n_frames; ++j)
-        if (frames[j].height > FUSED_SSE_MAX_H) { set_error("per-frame SSE: frame %d height %d exceeds %d", j, frames[j].height, FUSED_SSE_MAX_H); return QV_ERR_ARG; }
-    if (fused && !fused_list_ok(net->fm, frames, n_frames, d_sse != nullptr)) {
-        set_error("qv_forward_frame_list_device: the frames of one launch exceed 2^30 strip-column rows");
-        return QV_ERR_ARG;
-    }
+    if (!net->uploaded) { set_error("forward called before a complete model (weights + quant params) was loaded"); return QV_ERR_STATE; }
     int rc = set_device(net);
     if (rc) return rc;
     const cudaStream_t st = stream_of(net, cuda_stream);
-    if (fused) QV_CUDA(fused_forward_list(net->fm, frames, n_frames, d_sse, st, &net->launches));
-    else if ((rc = layered_forward_list(net->ln, frames, n_frames, d_sse, st, &net->launches))) return rc;
-    return finish(net, cuda_stream);
+    rc = runs_fused(net) ? fused_forward_list(net->fm, frames, n_frames, d_sse, st, &net->launches)
+                         : layered_forward_list(net->ln, frames, n_frames, d_sse, st, &net->launches);
+    return rc ? rc : finish(net, cuda_stream);
 }
 
 int qv_forward_rows_device(qv_net *net, const uint8_t *d_in, int img_height, int in_row0, int in_rows, uint8_t *d_out,
@@ -383,17 +376,17 @@ int qv_forward_rows_device(qv_net *net, const uint8_t *d_in, int img_height, int
     int rc = set_device(net);
     if (rc) return rc;
     const cudaStream_t st = stream_of(net, cuda_stream);
-    if (!net->uploaded || (runs_fused(net) && !net->fm)) { set_error("forward called before a complete model (weights + quant params) was loaded"); return QV_ERR_STATE; }
+    if (!net->uploaded) { set_error("forward called before a complete model (weights + quant params) was loaded"); return QV_ERR_STATE; }
     if (runs_fused(net)) {
         // the fused kernel takes the window as what it is: rows [in_row0, in_row1) of an img_height-row image, of which it
         // computes and writes exactly [out_row0, out_row1) -- no scratch frame, no copy
         FusedRows fr;
         fr.own0 = in_row0; fr.own1 = in_row1; fr.out0 = out_row0; fr.out1 = out_row1;
-        QV_CUDA(fused_forward(net->fm, d_in, d_out, 1, img_height, net->W, st, &net->launches, &fr));
-    } else if ((rc = layered_forward_rows(net->ln, d_in, in_rows, d_out, out_row0 - in_row0, out_row1 - in_row0, st, &net->launches))) {
-        return rc;
+        rc = fused_forward(net->fm, d_in, d_out, 1, img_height, net->W, st, &net->launches, &fr);
+    } else {
+        rc = layered_forward_rows(net->ln, d_in, in_rows, d_out, out_row0 - in_row0, out_row1 - in_row0, st, &net->launches);
     }
-    return finish(net, cuda_stream);
+    return rc ? rc : finish(net, cuda_stream);
 }
 
 int qv_synchronize(qv_net *net, void *cuda_stream)
@@ -416,7 +409,7 @@ static int strip_on(qv_net *net, const char *who)
 // A strip forward runs the fused kernel, which reads the neighbours' halo rows.
 static int strip_fused(const qv_net *net, const char *who)
 {
-    if (net->uploaded && net->fm && net->impl != QV_IMPL_LAYERED) return QV_OK;
+    if (net->uploaded && runs_fused(net)) return QV_OK;
     set_error("%s: needs a loaded model and the fused path (peer-mapped halo rows are read by the fused kernel)", who);
     return QV_ERR_STATE;
 }
@@ -993,7 +986,7 @@ int qv_strip_stream_yuv_pf(qv_net *const *nets, int n_nets, const char *anchor_y
     // every handle's fused-kernel report is taken (and cleared) now that its streams are idle; the first failure's message stands
     for (int i = 0; i < n_nets; ++i) {
         if (rc == QV_OK) rc = kernel_report(nets[i]);
-        else if (nets[i]->fm) fused_take_failure(nets[i]->fm);
+        else fused_take_failure(nets[i]->fm);
     }
     if (rc != QV_OK) return rc;
     for (int j = 0; with_ori && j < n_frames; ++j) {

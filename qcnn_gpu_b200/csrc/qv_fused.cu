@@ -55,6 +55,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <memory>
 #include <mutex>
 #include <type_traits>
@@ -533,7 +534,7 @@ void build_mma_ops(const PhaseBases *pb, const FixedBases &fb, PhaseOps *ops)
 struct FusedModel {
     int *h_fail = nullptr;             // cudaHostAlloc'ed, mapped: kernel failure report
     uint8_t *d_wimg = nullptr;
-    FusedParams proto{};
+    FusedParams proto{};               // the model's constants; every per-launch field stays zero (launch_params)
     bool fast = true;
     int sm_count = 148;
     // environment switches, read once at upload (never on the per-launch path)
@@ -542,12 +543,59 @@ struct FusedModel {
     void *encode_tiled = nullptr;      // cuTensorMapEncodeTiled (driver entry point; the library does not link libcuda)
 };
 
+// Every kernel build the host launches, with the dynamic shared memory it runs with: fused_upload raises each one's limit,
+// build_of picks the one a launch runs.  The first twelve come in pairs, generic requantiser first, so that entry + fast
+// is the build for a model.
+struct KernelBuild { const void *fn; int smem; };
+const KernelBuild k_builds[] = {
+    {(const void *)k_fused<false, false, false>, SMEM_BYTES}, {(const void *)k_fused<true, false, false>, SMEM_BYTES},
+    {(const void *)k_fused<false, false, true>, SMEM_BYTES},  {(const void *)k_fused<true, false, true>, SMEM_BYTES},
+    {(const void *)k_enh_sse<false, false>, SMEM_BYTES},      {(const void *)k_enh_sse<true, false>, SMEM_BYTES},
+    {(const void *)k_enh_sse<false, true>, SMEM_BYTES},       {(const void *)k_enh_sse<true, true>, SMEM_BYTES},
+    {(const void *)k_enh_list<false, false>, SMEM_BYTES},     {(const void *)k_enh_list<true, false>, SMEM_BYTES},
+    {(const void *)k_enh_list<false, true>, SMEM_BYTES},      {(const void *)k_enh_list<true, true>, SMEM_BYTES},
+    {(const void *)k_fused<true, true, false>, SMEM_BYTES},
+    {(const void *)k_fused<true, false, false, true>, SMEM_BYTES_T},
+    {(const void *)k_bases, SMEM_BYTES},
+};
+enum { B_WHOLE = 0, B_ROWS = 2, B_SSE = 4, B_SSE_ROWS = 6, B_LIST = 8, B_LIST_SSE = 10, B_PROFILE = 12, B_TMA = 13, B_BASES = 14 };
+static_assert(sizeof(k_builds) / sizeof(k_builds[0]) == B_BASES + 1, "one entry per build");
+
+// The build a launch runs: a frame list, the SSE form and a row window have their own; whole frames of a fast model run the
+// profiling build with QV_FUSED_PROFILE, else the TMA input ring with `tma` (QV_FUSED_TMA and an input a tensor map can
+// describe), else the plain kernel.
+static int build_of(bool fast, bool list, bool sse, bool rows, bool profile, bool tma)
+{
+    if (list) return (sse ? B_LIST_SSE : B_LIST) + fast;
+    if (sse) return (rows ? B_SSE_ROWS : B_SSE) + fast;
+    if (rows) return B_ROWS + fast;
+    if (fast && profile) return B_PROFILE;
+    if (fast && tma) return B_TMA;
+    return B_WHOLE + fast;
+}
+
+// One launch of build b (not k_bases) on `grid` CTAs; params points at its FusedParams (FusedListParams for a frame list).
+static int launch(int b, int grid, void *params, cudaStream_t st, long long *launches)
+{
+    if (launches) *launches += 1;
+    QV_CUDA(cudaLaunchKernel(k_builds[b].fn, grid, NTHREADS, &params, k_builds[b].smem, st));   // &params: the one argument
+    return QV_OK;
+}
+
+// The parameters every launch starts from: the model's constants, with QV_FUSED_TEST_FAIL applied.
+static FusedParams launch_params(const FusedModel *fm)
+{
+    FusedParams P = fm->proto;
+    if (fm->env_test_fail) P.sbase16 ^= 1u;
+    return P;
+}
+
 // The operand table lives in constant memory: one copy per device, and its content depends only on the shared-memory
 // window / TMEM bases a CTA of this launch shape gets -- the same for every model.  It is written once per device, under
 // a lock, so that distinct handles can load models from distinct threads (include/qvrcnn_b200.h).
+struct OpsBases { uint32_t sbase16, tmem_base; };
 static std::mutex g_ops_mu;
-struct OpsRecord { bool done = false; uint32_t sbase16 = 0, tmem_base = 0; };
-static OpsRecord g_ops_done[64];
+static std::map<int, OpsBases> g_ops;   // device -> the bases its table was built for
 
 // Writes 16 K-bytes of row n, K-chunk j, of a B block laid out [2][NR][16].
 static void put_chunk(uint8_t *blk, int NR, int j, int n, const int8_t *src16) { memcpy(blk + ((size_t)j * NR + n) * 16, src16, 16); }
@@ -680,67 +728,48 @@ void fused_debug_tables(const ModelHost &m, std::vector<uint8_t> &wimg, std::vec
     consts.insert(consts.end(), P.c4_w, P.c4_w + 108);
 }
 
-FusedModel *fused_upload(const ModelHost &m, cudaStream_t st)
+// Writes the operand table of device dev (the current one) on its first model; P takes the bases it was built for.  Under g_ops_mu.
+static int operand_table(int dev, cudaStream_t st, FusedParams &P)
 {
-    std::vector<uint8_t> img;
-    FusedModel *fm = new FusedModel();
+    auto it = g_ops.find(dev);
+    if (it == g_ops.end()) {
+        uint32_t *d_b = nullptr, h_b[2] = {0, 0};
+        QV_CUDA(cudaMalloc(&d_b, 8));
+        k_bases<<<1, 32, k_builds[B_BASES].smem, st>>>(d_b);
+        cudaError_t e = cudaMemcpyAsync(h_b, d_b, 8, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        cudaFree(d_b);
+        QV_CUDA(e);
+        PhaseBases pb[N_PHASE];
+        FixedBases fb;
+        build_mma_bases(h_b[0] >> 4, h_b[1], pb, fb);
+        std::vector<PhaseOps> ops(N_PHASE);      // outlives the copy: synchronised below
+        build_mma_ops(pb, fb, ops.data());
+        QV_CUDA(cudaMemcpyToSymbolAsync(c_ops, ops.data(), sizeof(PhaseOps) * N_PHASE, 0, cudaMemcpyHostToDevice, st));
+        QV_CUDA(cudaStreamSynchronize(st));
+        it = g_ops.emplace(dev, OpsBases{h_b[0] >> 4, h_b[1]}).first;
+    }
+    P.sbase16 = it->second.sbase16; P.tmem_base = it->second.tmem_base;
+    return QV_OK;
+}
+
+int fused_upload(const ModelHost &m, cudaStream_t st, FusedModel **out)
+{
+    std::unique_ptr<FusedModel, void (*)(FusedModel *)> fm(new FusedModel(), fused_free);   // freed on every failure
     FusedParams &P = fm->proto;
+    std::vector<uint8_t> img;
     fm->fast = build_host_image(m, img, P);
-    cudaError_t e = cudaMalloc(&fm->d_wimg, WIMG_BYTES);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(fm->d_wimg, img.data(), WIMG_BYTES, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_fused<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_fused<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_fused<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_fused<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_fused<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_fused<true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES_T);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_sse<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_sse<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_sse<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_sse<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_list<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_list<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_list<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_enh_list<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k_bases, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    int dev = 0, sms = 148;
-    if (e == cudaSuccess) e = cudaGetDevice(&dev);
-    if (e == cudaSuccess && (dev < 0 || dev >= 64)) e = cudaErrorInvalidDevice;
-    if (e == cudaSuccess) {
-        // descriptor table in constant memory, for the shared-memory / TMEM bases a CTA of this launch shape gets
+    QV_CUDA(cudaMalloc(&fm->d_wimg, WIMG_BYTES));
+    QV_CUDA(cudaMemcpyAsync(fm->d_wimg, img.data(), WIMG_BYTES, cudaMemcpyHostToDevice, st));
+    QV_CUDA(cudaStreamSynchronize(st));
+    for (const KernelBuild &k : k_builds) QV_CUDA(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, k.smem));
+    int dev = 0;
+    QV_CUDA(cudaGetDevice(&dev));
+    {
         std::lock_guard<std::mutex> lock(g_ops_mu);
-        OpsRecord &rec = g_ops_done[dev];
-        if (!rec.done) {
-            uint32_t *d_b = nullptr, h_b[2] = {0, 0};
-            e = cudaMalloc(&d_b, 8);
-            if (e == cudaSuccess) {
-                k_bases<<<1, 32, SMEM_BYTES, st>>>(d_b);
-                e = cudaMemcpyAsync(h_b, d_b, 8, cudaMemcpyDeviceToHost, st);
-                if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-                cudaFree(d_b);
-            }
-            if (e == cudaSuccess) {
-                PhaseBases pb[N_PHASE];
-                FixedBases fb;
-                build_mma_bases(h_b[0] >> 4, h_b[1], pb, fb);
-                std::vector<PhaseOps> ops(N_PHASE);      // outlives the copy: synchronised below
-                build_mma_ops(pb, fb, ops.data());
-                e = cudaMemcpyToSymbolAsync(c_ops, ops.data(), sizeof(PhaseOps) * N_PHASE, 0, cudaMemcpyHostToDevice, st);
-                if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-                if (e == cudaSuccess) { rec.done = true; rec.sbase16 = h_b[0] >> 4; rec.tmem_base = h_b[1]; }
-            }
-        }
-        P.sbase16 = rec.sbase16; P.tmem_base = rec.tmem_base;
+        if (int rc = operand_table(dev, st, P)) return rc;
     }
-    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (e != cudaSuccess) {
-        set_error("fused_upload: %s", cudaGetErrorString(e));
-        cudaFree(fm->d_wimg);
-        delete fm;
-        return nullptr;
-    }
-    fm->sm_count = sms;
+    QV_CUDA(cudaDeviceGetAttribute(&fm->sm_count, cudaDevAttrMultiProcessorCount, dev));
     fm->env_profile = getenv("QV_FUSED_PROFILE") != nullptr;
     fm->env_experiment = getenv("QV_FUSED_EXPERIMENT") ? atoi(getenv("QV_FUSED_EXPERIMENT")) : 0;
     fm->env_test_fail = getenv("QV_FUSED_TEST_FAIL") != nullptr;     // tests only: make every CTA report a base mismatch
@@ -752,19 +781,11 @@ FusedModel *fused_upload(const ModelHost &m, cudaStream_t st)
         cudaGetLastError();
     }
     P.wimg = fm->d_wimg;
-    P.fail_flag = nullptr;
-    if (cudaHostAlloc(&fm->h_fail, sizeof(int), cudaHostAllocMapped) == cudaSuccess) {
-        *fm->h_fail = 0;
-        if (cudaHostGetDevicePointer(&P.fail_flag, fm->h_fail, 0) != cudaSuccess) P.fail_flag = nullptr;
-    }
-    if (!P.fail_flag) {
-        set_error("fused_upload: no mapped host memory for the failure report");
-        if (fm->h_fail) cudaFreeHost(fm->h_fail);
-        cudaFree(fm->d_wimg);
-        delete fm;
-        return nullptr;
-    }
-    return fm;
+    QV_CUDA(cudaHostAlloc(&fm->h_fail, sizeof(int), cudaHostAllocMapped));
+    *fm->h_fail = 0;
+    QV_CUDA(cudaHostGetDevicePointer(&P.fail_flag, fm->h_fail, 0));
+    *out = fm.release();
+    return QV_OK;
 }
 
 cudaError_t fused_wait_words(const FusedModel *fm, const uint32_t *a, uint32_t va, const uint32_t *b, uint32_t vb, cudaStream_t st)
@@ -784,7 +805,7 @@ void fused_free(FusedModel *fm)
 
 int fused_take_failure(const FusedModel *fm)
 {
-    if (!fm || !fm->h_fail) return 0;
+    if (!fm) return 0;
     const int f = *reinterpret_cast<volatile int *>(fm->h_fail);
     if (f) *fm->h_fail = 0;
     return f;
@@ -923,74 +944,105 @@ int fused_debug_list_units(int sm_count, int n_frames, const int *H, const int *
     return 0;
 }
 
-bool fused_list_ok(const FusedModel *fm, const qv_frame_desc *frames, int n, bool sse)
+int fused_forward_list(const FusedModel *fm, const qv_frame_desc *frames, int n, int64_t *d_sse, cudaStream_t st, long long *launches)
 {
-    for (int f = 0; f < n; ++f)
-        if (sse ? !frames[f].d_ori || frames[f].height > FUSED_SSE_MAX_H : frames[f].d_ori != nullptr) return false;
+    for (int f = 0; f < n; ++f) {
+        if (!frames[f].d_ori != !d_sse) { set_error("fused_forward_list: frame %d: d_ori and d_sse go together", f); return QV_ERR_ARG; }
+        if (d_sse && frames[f].height > FUSED_SSE_MAX_H) {      // the C4 threads' 32-bit column sums
+            set_error("fused_forward_list: per-frame SSE: frame %d height %d exceeds %d", f, frames[f].height, FUSED_SSE_MAX_H);
+            return QV_ERR_ARG;
+        }
+    }
     std::unique_ptr<FusedListParams> L(new FusedListParams{});      // 12 KB: not on the stack
     int grid = 1;
-    for (int f0 = 0; f0 < n; f0 += QV_FRAME_LIST_LAUNCH_MAX)
-        if (plan_list(*L, frames + f0, std::min(QV_FRAME_LIST_LAUNCH_MAX, n - f0), fm->sm_count, grid) != cudaSuccess) return false;
-    return true;
-}
-
-cudaError_t fused_forward_list(const FusedModel *fm, const qv_frame_desc *frames, int n, int64_t *d_sse, cudaStream_t st, long long *launches)
-{
-    if (!fused_list_ok(fm, frames, n, d_sse != nullptr)) return cudaErrorInvalidValue;      // every launch's plan, before the first
-    std::unique_ptr<FusedListParams> L(new FusedListParams{});
+    auto plan = [&](int f0) {
+        L->p = launch_params(fm);
+        return plan_list(*L, frames + f0, std::min(QV_FRAME_LIST_LAUNCH_MAX, n - f0), fm->sm_count, grid) == cudaSuccess;
+    };
+    for (int f0 = 0; f0 < n; f0 += QV_FRAME_LIST_LAUNCH_MAX)        // every launch's plan, before the first launch
+        if (!plan(f0)) {
+            set_error("fused_forward_list: the frames of one launch exceed 2^30 strip-column rows");
+            return QV_ERR_ARG;
+        }
     for (int f0 = 0; f0 < n; f0 += QV_FRAME_LIST_LAUNCH_MAX) {
-        const int c = std::min(QV_FRAME_LIST_LAUNCH_MAX, n - f0);
-        FusedParams &P = L->p;
-        P = fm->proto;
-        P.in = nullptr; P.out = nullptr; P.ori = nullptr;
-        P.sse = d_sse ? reinterpret_cast<unsigned long long *>(d_sse + 2 * (size_t)f0) : nullptr;
-        P.H = P.W = 0;
-        P.frame_stride = 0;
-        P.ys = P.ye = P.own0 = P.own1 = P.rlo = P.rhi = 0;
-        P.in_top = P.in_bot = nullptr; P.flag_top = P.flag_bot = nullptr;
-        P.pub = P.done = P.done_ctr = nullptr; P.seq = 0;
-        P.dbg = nullptr;
-        P.dbg_flags = 0;
-        if (fm->env_test_fail) P.sbase16 ^= 1u;
-        int grid = 1;
-        if (const cudaError_t e = plan_list(*L, frames + f0, c, fm->sm_count, grid)) return e;
-        if (d_sse && fm->fast) k_enh_list<true, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(*L);
-        else if (d_sse) k_enh_list<false, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(*L);
-        else if (fm->fast) k_enh_list<true, false><<<grid, NTHREADS, SMEM_BYTES, st>>>(*L);
-        else k_enh_list<false, false><<<grid, NTHREADS, SMEM_BYTES, st>>>(*L);
-        if (launches) *launches += 1;
-        if (const cudaError_t e = cudaGetLastError()) return e;
+        plan(f0);
+        L->p.sse = d_sse ? reinterpret_cast<unsigned long long *>(d_sse + 2 * (size_t)f0) : nullptr;
+        if (int rc = launch(build_of(fm->fast, true, d_sse != nullptr, false, false, false), grid, L.get(), st, launches)) return rc;
     }
-    return cudaSuccess;
+    return QV_OK;
 }
 
-cudaError_t fused_forward(const FusedModel *fm, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W, cudaStream_t st,
-                          long long *launches, const FusedRows *rows, const uint8_t *d_ori, int64_t *d_sse)
+// The profiling build (QV_FUSED_PROFILE=1): one launch with per-block phase timers; once it has finished, their averages
+// and the timeline of block 0 go to stderr.
+static int launch_profiled(const FusedModel *fm, FusedParams &P, int grid, cudaStream_t st, long long *launches)
 {
-    if (n <= 0) return cudaSuccess;
+    std::vector<long long> h((size_t)grid * 16 + TR_N * 48);
+    const size_t bytes = h.size() * sizeof(long long);
+    QV_CUDA(cudaMalloc(&P.dbg, bytes));
+    const std::unique_ptr<long long, cudaError_t (*)(void *)> hold(P.dbg, cudaFree);
+    P.dbg_flags = fm->env_experiment;
+    QV_CUDA(cudaMemsetAsync(P.dbg, 0, bytes, st));
+    if (int rc = launch(B_PROFILE, grid, &P, st, launches)) return rc;
+    QV_CUDA(cudaStreamSynchronize(st));
+    QV_CUDA(cudaMemcpy(h.data(), P.dbg, bytes, cudaMemcpyDeviceToHost));
+    double a[16] = {0};
+    for (int b = 0; b < grid; ++b) for (int k = 0; k < 16; ++k) a[k] += (double)h[(size_t)b * 16 + k] / grid;
+    const double iters = P.linear ? (double)P.seg_rows + PIPE * (P.n_units / grid - 1) : (double)P.n_units / grid * (P.seg_rows + PIPE);
+    fprintf(stderr, "[qv fused profile] units=%d grid=%d iters/block~%.0f | cycles per iteration: MMA warp wait=%.0f issue=%.0f | "
+            "worker w0: wait_mma=%.0f drain=%.0f (of which tcgen05.ld+wait %.0f) fence+arrive=%.0f bar=%.0f | "
+            "second traced worker (thread NWORKER/2): wait_mma=%.0f drain=%.0f (tcgen05.ld+wait %.0f) fence+arrive=%.0f bar=%.0f\n",
+            P.n_units, grid, iters, a[0] / iters, a[1] / iters, a[2] / iters, a[3] / iters, a[14] / iters, a[4] / iters, a[5] / iters,
+            a[8] / iters, a[9] / iters, a[15] / iters, a[10] / iters, a[11] / iters);
+    // timeline of block 0: per traced iteration, cycles relative to the first issue start
+    const long long *tr = h.data() + (size_t)grid * 16, t0 = tr[0];
+    if (t0)
+        for (int k = 0; k < TR_N; ++k, tr += 16)
+            fprintf(stderr, "[qv fused trace] it %d | mma: start %lld end %lld | w0: commit %lld drained %lld arrived %lld bar %lld | "
+                    "w2: commit %lld drained %lld arrived %lld bar %lld\n", TR_ITER0 + k, tr[0] - t0, tr[1] - t0, tr[2] - t0, tr[3] - t0,
+                    tr[4] - t0, tr[5] - t0, tr[6] - t0, tr[7] - t0, tr[8] - t0, tr[9] - t0);
+    tr = h.data() + (size_t)grid * 16;
+    if (t0)
+        for (int k = 0; k < TR_N; ++k, tr += 16)
+            fprintf(stderr, "[qv fused mma-side] it %d | loop top %lld  wait done %lld  fence done %lld  (issue start %lld)  commit issued %lld  end %lld\n",
+                    TR_ITER0 + k, tr[10] - t0, tr[11] - t0, tr[12] - t0, tr[0] - t0, tr[13] - t0, tr[1] - t0);
+    if (t0)
+        for (int k = 0; k < TR_N; ++k) {
+            const long long *sp = h.data() + (size_t)grid * 16 + TR_N * 16 + k * 32, s0 = h[(size_t)grid * 16 + k * 16];
+            fprintf(stderr, "[qv fused stamps] it %d:", TR_ITER0 + k);
+            for (int j = 0; j < 27; ++j) fprintf(stderr, " %lld", sp[j] - (j ? sp[j - 1] : s0));
+            fprintf(stderr, "\n");
+        }
+    return QV_OK;
+}
+
+int fused_forward(const FusedModel *fm, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W, cudaStream_t st,
+                  long long *launches, const FusedRows *rows, const uint8_t *d_ori, int64_t *d_sse)
+{
+    if (n <= 0) return QV_OK;
     const bool sse = d_ori && d_sse;
-    if ((d_ori || d_sse) && !sse) return cudaErrorInvalidValue;
-    if (sse && H > FUSED_SSE_MAX_H) return cudaErrorInvalidValue;      // the C4 threads' 32-bit column sums
-    FusedParams P = fm->proto;
+    if ((d_ori || d_sse) && !sse) { set_error("fused_forward: d_ori and d_sse go together"); return QV_ERR_ARG; }
+    if (sse && H > FUSED_SSE_MAX_H) {      // the C4 threads' 32-bit column sums
+        set_error("fused_forward: per-frame SSE: frame height %d exceeds %d", H, FUSED_SSE_MAX_H);
+        return QV_ERR_ARG;
+    }
+    FusedParams P = launch_params(fm);
     P.ori = d_ori;
     P.sse = reinterpret_cast<unsigned long long *>(d_sse);
     P.n_frames = n; P.H = H; P.W = W;
     P.frame_stride = (size_t)H * W;
     P.in = d_in; P.out = d_out;
-    P.ys = P.own0 = P.rlo = 0; P.ye = P.own1 = P.rhi = H;
-    P.in_top = P.in_bot = nullptr; P.flag_top = P.flag_bot = nullptr;
-    P.pub = P.done = P.done_ctr = nullptr; P.seq = 0;
+    P.ye = P.own1 = P.rhi = H;
     if (rows) {
         // one frame, a row window of it: H is the height of the IMAGE (each layer's zero padding applies at the image
         // edges only, inference/cnn.cu:44-49), the buffers hold the rows the launch description names
+        const char *bad = "fused_forward: inconsistent row window";
         if (n != 1 || rows->own0 < 0 || rows->own1 > H || rows->own0 >= rows->own1 || rows->out0 < rows->own0 || rows->out1 > rows->own1 ||
-            rows->out0 > rows->out1 || rows->top_rows < 0 || rows->bot_rows < 0)
-            return cudaErrorInvalidValue;
-        if (rows->out0 == rows->out1) return cudaSuccess;
+            rows->out0 > rows->out1 || rows->top_rows < 0 || rows->bot_rows < 0) { set_error("%s", bad); return QV_ERR_ARG; }
+        if (rows->out0 == rows->out1) return QV_OK;
         P.own0 = rows->own0; P.own1 = rows->own1; P.ys = rows->out0; P.ye = rows->out1;
         P.rlo = rows->d_top ? rows->own0 - rows->top_rows : rows->own0;
         P.rhi = rows->d_bot ? rows->own1 + rows->bot_rows : rows->own1;
-        if (P.rlo < 0 || P.rhi > H) return cudaErrorInvalidValue;
+        if (P.rlo < 0 || P.rhi > H) { set_error("%s", bad); return QV_ERR_ARG; }
         P.in = d_in - (ptrdiff_t)rows->own0 * W;
         P.out = d_out - (ptrdiff_t)rows->out0 * W;
         if (sse) P.ori = d_ori - (ptrdiff_t)rows->out0 * W;
@@ -1001,74 +1053,25 @@ cudaError_t fused_forward(const FusedModel *fm, const uint8_t *d_in, uint8_t *d_
         P.pub = rows->pub; P.done = rows->done; P.done_ctr = rows->done_ctr; P.seq = rows->seq;
     }
     int grid = 1;
-    if (const cudaError_t e = plan_units(P, fm->sm_count, true, rows != nullptr, grid)) return e;
-    const bool prof = fm->env_profile;
-    P.dbg = nullptr;
-    P.dbg_flags = fm->env_experiment;
-    if (fm->env_test_fail) P.sbase16 ^= 1u;
-    const size_t dbg_n = (size_t)grid * 16 + TR_N * 48;
-    if (prof && !rows && !sse && cudaMalloc(&P.dbg, dbg_n * sizeof(long long)) != cudaSuccess) P.dbg = nullptr;
-    if (P.dbg) cudaMemsetAsync(P.dbg, 0, dbg_n * sizeof(long long), st);
-    // TMA input ring (opt-in, QV_FUSED_TMA=1): whole-frame launches of the fast instantiation whose input can be described
-    // by a tensor map (16-byte aligned base and row pitch); the SSE kernel has no TMA form
-    bool tma = false;
-    if (fm->env_tma && fm->encode_tiled && !rows && !sse && fm->fast && !P.dbg && W % 16 == 0 && W >= IN_BOX && ((uintptr_t)d_in & 15) == 0) {
+    if (plan_units(P, fm->sm_count, true, rows != nullptr, grid) != cudaSuccess) {
+        set_error("fused_forward: %d frames of %dx%d are more work units than one launch takes", n, W, H);
+        return QV_ERR_ARG;
+    }
+    // TMA input ring (opt-in, QV_FUSED_TMA=1): input a tensor map can describe (16-byte aligned base and row pitch)
+    const bool tma = fm->env_tma && fm->encode_tiled && W % 16 == 0 && W >= IN_BOX && ((uintptr_t)d_in & 15) == 0;
+    int b = build_of(fm->fast, false, sse, rows != nullptr, fm->env_profile, tma);
+    if (b == B_PROFILE) return launch_profiled(fm, P, grid, st, launches);
+    if (b == B_TMA) {
         using EncodeFn = CUresult (*)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
                                       const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
         const cuuint64_t dims[2] = {(cuuint64_t)W, (cuuint64_t)n * (cuuint64_t)H}, strides[1] = {(cuuint64_t)W};
         const cuuint32_t box[2] = {(cuuint32_t)IN_BOX, 1}, estr[2] = {1, 1};
-        tma = reinterpret_cast<EncodeFn>(fm->encode_tiled)(&P.tmap_in, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<uint8_t *>(d_in), dims, strides, box, estr,
-                                                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                                            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+        if (reinterpret_cast<EncodeFn>(fm->encode_tiled)(&P.tmap_in, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<uint8_t *>(d_in), dims, strides, box, estr,
+                                                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                                                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+            b = B_WHOLE + fm->fast;                                     // no tensor map: the plain input ring
     }
-    if (sse && rows) {
-        if (fm->fast) k_enh_sse<true, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(P);
-        else k_enh_sse<false, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(P);
-    } else if (sse) {
-        if (fm->fast) k_enh_sse<true, false><<<grid, NTHREADS, SMEM_BYTES, st>>>(P);
-        else k_enh_sse<false, false><<<grid, NTHREADS, SMEM_BYTES, st>>>(P);
-    } else if (tma) k_fused<true, false, false, true><<<grid, NTHREADS, SMEM_BYTES_T, st>>>(P);
-    else if (rows && fm->fast) k_fused<true, false, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(P);
-    else if (rows) k_fused<false, false, true><<<grid, NTHREADS, SMEM_BYTES, st>>>(P);
-    else if (fm->fast && P.dbg) k_fused<true, true, false><<<grid, NTHREADS, SMEM_BYTES, st>>>(P);
-    else if (fm->fast) k_fused<true, false, false><<<grid, NTHREADS, SMEM_BYTES, st>>>(P);
-    else k_fused<false, false, false><<<grid, NTHREADS, SMEM_BYTES, st>>>(P);
-    if (launches) *launches += 1;
-    cudaError_t e = cudaGetLastError();
-    if (P.dbg) {
-        std::vector<long long> h(dbg_n);
-        cudaStreamSynchronize(st);
-        cudaMemcpy(h.data(), P.dbg, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-        cudaFree(P.dbg);
-        double a[16] = {0};
-        for (int b = 0; b < grid; ++b) for (int k = 0; k < 16; ++k) a[k] += (double)h[(size_t)b * 16 + k] / grid;
-        const double iters = P.linear ? (double)P.seg_rows + PIPE * (P.n_units / grid - 1) : (double)P.n_units / grid * (P.seg_rows + PIPE);
-        fprintf(stderr, "[qv fused profile] units=%d grid=%d iters/block~%.0f | cycles per iteration: MMA warp wait=%.0f issue=%.0f | "
-                "worker w0: wait_mma=%.0f drain=%.0f (of which tcgen05.ld+wait %.0f) fence+arrive=%.0f bar=%.0f | "
-                "second traced worker (thread NWORKER/2): wait_mma=%.0f drain=%.0f (tcgen05.ld+wait %.0f) fence+arrive=%.0f bar=%.0f\n",
-                P.n_units, grid, iters, a[0] / iters, a[1] / iters, a[2] / iters, a[3] / iters, a[14] / iters, a[4] / iters, a[5] / iters,
-                a[8] / iters, a[9] / iters, a[15] / iters, a[10] / iters, a[11] / iters);
-        // timeline of block 0: per traced iteration, cycles relative to the first issue start
-        const long long *tr = h.data() + (size_t)grid * 16, t0 = tr[0];
-        if (t0)
-            for (int k = 0; k < TR_N; ++k, tr += 16)
-                fprintf(stderr, "[qv fused trace] it %d | mma: start %lld end %lld | w0: commit %lld drained %lld arrived %lld bar %lld | "
-                        "w2: commit %lld drained %lld arrived %lld bar %lld\n", TR_ITER0 + k, tr[0] - t0, tr[1] - t0, tr[2] - t0, tr[3] - t0,
-                        tr[4] - t0, tr[5] - t0, tr[6] - t0, tr[7] - t0, tr[8] - t0, tr[9] - t0);
-        tr = h.data() + (size_t)grid * 16;
-        if (t0)
-            for (int k = 0; k < TR_N; ++k, tr += 16)
-                fprintf(stderr, "[qv fused mma-side] it %d | loop top %lld  wait done %lld  fence done %lld  (issue start %lld)  commit issued %lld  end %lld\n",
-                        TR_ITER0 + k, tr[10] - t0, tr[11] - t0, tr[12] - t0, tr[0] - t0, tr[13] - t0, tr[1] - t0);
-        if (t0)
-            for (int k = 0; k < TR_N; ++k) {
-                const long long *sp = h.data() + (size_t)grid * 16 + TR_N * 16 + k * 32, s0 = h[(size_t)grid * 16 + k * 16];
-                fprintf(stderr, "[qv fused stamps] it %d:", TR_ITER0 + k);
-                for (int j = 0; j < 27; ++j) fprintf(stderr, " %lld", sp[j] - (j ? sp[j - 1] : s0));
-                fprintf(stderr, "\n");
-            }
-    }
-    return e;
+    return launch(b, grid, &P, st, launches);
 }
 
 }  // namespace qv

@@ -1,4 +1,5 @@
-// Host-visible interface of the fused tcgen05 path (qv_fused.cu).
+// Host-visible interface of the fused tcgen05 path (qv_fused.cu).  fused_upload, fused_forward and fused_forward_list
+// return a QV_* code and set the message.
 #pragma once
 #include <cstdint>
 #include <vector>
@@ -10,8 +11,8 @@ namespace qv {
 
 struct FusedModel;   // device-resident weights / descriptors in the layout the fused kernel wants
 
-// Builds the device image of the model for the fused kernel. Returns nullptr + error on failure.
-FusedModel *fused_upload(const ModelHost &m, cudaStream_t st);
+// Builds the device image of the model for the fused kernel into *out (untouched on failure).
+int fused_upload(const ModelHost &m, cudaStream_t st, FusedModel **out);
 void fused_free(FusedModel *fm);
 // A row window of ONE frame (spatial partition over several GPUs): the launch produces image rows [out0, out1) into d_out
 // (first row = out0) from d_in, which holds image rows [own0, own1); up to 6 rows above / below come from d_top (first row
@@ -29,26 +30,22 @@ struct FusedRows {
 // launch the exact sum (anchor - ori)^2 is ADDED to d_sse[2f] and sum (out - ori)^2 to d_sse[2f + 1] (device int64; the
 // integer core of vrcnn_data::psnr_pf, inference/yuv_data.cpp:98-112).  d_ori holds the same pixels as d_out (with `rows`:
 // rows [out0, out1)).  There is no SSE form of the profiling build or of the opt-in TMA input ring: with QV_FUSED_TMA=1 an
-// SSE launch runs the kernel without TMA.  H > FUSED_SSE_MAX_H is refused (cudaErrorInvalidValue).
+// SSE launch runs the kernel without TMA.  H > FUSED_SSE_MAX_H is refused (QV_ERR_ARG).
 constexpr int FUSED_SSE_MAX_H = 66051;     // per-thread column sums are 32-bit: 255^2 * H < 2^32
-cudaError_t fused_forward(const FusedModel *fm, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W,
-                          cudaStream_t st, long long *launches, const FusedRows *rows = nullptr,
-                          const uint8_t *d_ori = nullptr, int64_t *d_sse = nullptr);
+int fused_forward(const FusedModel *fm, const uint8_t *d_in, uint8_t *d_out, int n, int H, int W, cudaStream_t st,
+                  long long *launches, const FusedRows *rows = nullptr, const uint8_t *d_ori = nullptr, int64_t *d_sse = nullptr);
 // Frames of any sizes, one model (qv_forward_frame_list_device): k_enh_list, one launch per QV_FRAME_LIST_LAUNCH_MAX frames,
 // each adding 1 to *launches.  With d_sse every frame carries d_ori and height <= FUSED_SSE_MAX_H, and the SSE pair of frame j is
-// ADDED to d_sse[2j], d_sse[2j + 1]; without it no frame carries d_ori.  Otherwise (fused_list_ok) cudaErrorInvalidValue
-// before any launch.
-// Whether fused_forward_list takes the list: the d_ori / d_sse rule above, and every launch's row line fits the planner
-// (at most 2^30 row iterations).
-bool fused_list_ok(const FusedModel *fm, const qv_frame_desc *frames, int n, bool sse);
-cudaError_t fused_forward_list(const FusedModel *fm, const qv_frame_desc *frames, int n, int64_t *d_sse, cudaStream_t st,
-                               long long *launches);
+// ADDED to d_sse[2j], d_sse[2j + 1]; without it no frame carries d_ori.  Every launch's row line must fit the planner (at most
+// 2^30 row iterations).  A list that breaks a rule is refused (QV_ERR_ARG) before any launch.
+int fused_forward_list(const FusedModel *fm, const qv_frame_desc *frames, int n, int64_t *d_sse, cudaStream_t st,
+                       long long *launches);
 // Stream-ordered helper of the strip protocol: spin (bounded) until *a >= va and *b >= vb (either pointer may be null; the
 // words live on OTHER GPUs), reporting a timeout through the model's failure word (code 3).
 cudaError_t fused_wait_words(const FusedModel *fm, const uint32_t *a, uint32_t va, const uint32_t *b, uint32_t vb, cudaStream_t st);
 // After the stream the kernel ran on has been synchronised: 0, or what a CTA reported (1 = an mbarrier wait timed
 // out, 2 = shared-memory / TMEM bases other than the operand table was built for, 3 = a neighbour GPU's rows never
-// arrived); the report is cleared.
+// arrived); the report is cleared.  0 for a null fm (no model uploaded yet).
 int fused_take_failure(const FusedModel *fm);
 
 // Test hook (no GPU): weight image, per-phase MMA operand table (bases 0) and constants as the host builds them.

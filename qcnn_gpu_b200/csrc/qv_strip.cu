@@ -185,7 +185,7 @@ int strip_acquire(StripNet *s, int slot, const FusedModel *fm, cudaStream_t st, 
             }
         }
     }
-    if (fm && (w[0] || w[1])) {   // outside the lock: a launch may block while the launch queue is full
+    if (w[0] || w[1]) {   // seq != 0: forwarded before, so fm is set.  Outside the lock: a launch may block on a full queue
         QV_CUDA(fused_wait_words(fm, w[0], seq, w[1], seq, st));
         *launches += 1;
     }
@@ -228,8 +228,7 @@ int strip_forward(StripNet *s, int slot, const FusedModel *fm, const uint8_t *d_
         s->forwards[slot] += 1;
         s->last_stream = st;
     }
-    QV_CUDA(fused_forward(fm, strip_slot(s, slot), d_out, 1, s->img_h, s->W, st, launches, &fr, d_ori, d_sse));
-    return QV_OK;
+    return fused_forward(fm, strip_slot(s, slot), d_out, 1, s->img_h, s->W, st, launches, &fr, d_ori, d_sse);
 }
 
 int strip_claim(StripNet *const *s, int n, const char *who)

@@ -28,19 +28,6 @@ def _net(model, batch, h, w, impl, tmp_path=None):
     return net
 
 
-def _fused_or_skip(net, impl):
-    if impl == api.IMPL_FUSED:
-        try:
-            net.set_impl(api.IMPL_FUSED)
-            x = np.zeros((net.batch, net.height, net.width), np.uint8)
-            net.load_data(x)
-            net.forward_blu()
-        except api.QVError as e:
-            if "not available" in str(e):
-                pytest.skip("fused path not built")
-            raise
-
-
 @pytest.mark.parametrize("impl", IMPLS, ids=lambda i: IMPL_NAME[i])
 @pytest.mark.parametrize("qp", [22, 27, 32, 37])
 def test_config1_416x240_bit_exact(models, qp, impl, tmp_path):
@@ -52,7 +39,6 @@ def test_config1_416x240_bit_exact(models, qp, impl, tmp_path):
     path.write_bytes(formats.write_model_vect_c(m))
     net = api.QVRCNN(0, 1, 1, 240, 416)
     net.load_static_para(str(path))
-    _fused_or_skip(net, impl)
     net.set_impl(impl)
     net.load_data(anchor)
     net.forward_blu()
@@ -93,7 +79,6 @@ def test_ragged_and_tiny_frames(models, impl, shape):
     h, w = shape
     x = synth.make_uniform_frames(17, 2, h, w)
     net = _net(m, 2, h, w, api.IMPL_LAYERED)
-    _fused_or_skip(net, impl)
     net.set_impl(impl)
     net.load_data(x)
     net.forward_blu()
@@ -106,7 +91,6 @@ def test_constant_frames(models, impl, value):
     m = models[27]
     x = np.full((1, 40, 72), value, np.uint8)
     net = _net(m, 1, 40, 72, api.IMPL_LAYERED)
-    _fused_or_skip(net, impl)
     net.set_impl(impl)
     net.load_data(x)
     net.forward_blu()
@@ -121,7 +105,6 @@ def test_config2_8x832x480_all_qps(models, impl):
     for qp in (22, 27, 32, 37):
         m = models[qp]
         net = _net(m, 8, 480, 832, api.IMPL_LAYERED)
-        _fused_or_skip(net, impl)
         net.set_impl(impl)
         out = net.forward_frames_host(anchor)
         om = _oracle(m)
@@ -142,7 +125,6 @@ def test_fused_equals_layered_1080p(models):
     anchor, _ = synth.make_frames(0xC0FFEE + 4, 6, 1080, 1920)
     a = _net(m, 6, 1080, 1920, api.IMPL_LAYERED)
     out_l = a.forward_frames_host(anchor)
-    _fused_or_skip(a, api.IMPL_FUSED)
     a.set_impl(api.IMPL_FUSED)
     out_f = a.forward_frames_host(anchor)
     assert np.array_equal(out_l, out_f)
@@ -156,7 +138,6 @@ def test_config3_all_64_distinct_frames(models):
     anchor, _ = synth.make_frames(0xC0FFEE + 40, 64, 1080, 1920)
     net = _net(m, 8, 1080, 1920, api.IMPL_LAYERED)
     out_l = net.forward_frames_host(anchor)
-    _fused_or_skip(net, api.IMPL_FUSED)
     net.set_impl(api.IMPL_FUSED)
     out_f = net.forward_frames_host(anchor)
     assert np.array_equal(out_l, out_f)
@@ -268,7 +249,6 @@ def test_full_size_properties_4k_and_8k(models):
     anchor, _ = synth.make_frames(0xC0FFEE + 9, 3, h, w)
     net = _net(m4, 3, h, w, api.IMPL_LAYERED)
     out_l = net.forward_frames_host(anchor)
-    _fused_or_skip(net, api.IMPL_FUSED)
     net.set_impl(api.IMPL_FUSED)
     out_f = net.forward_frames_host(anchor)
     assert np.array_equal(out_l, out_f)
@@ -305,7 +285,6 @@ def test_rows_mode_strips_equal_whole_frame(models, impl):
     h, w = 150, 200
     anchor, _ = synth.make_frames(0xC0FFEE + 5, 1, h, w)
     net = _net(m, 1, h, w, api.IMPL_LAYERED)
-    _fused_or_skip(net, impl)
     net.set_impl(impl)
     net.load_data(anchor)
     net.forward_blu()
@@ -443,7 +422,6 @@ def test_kernel_failure_is_reported(models, monkeypatch):
     is uploaded, not on the launch path.)"""
     image = formats.write_model_vect_c(models[32])
     net = _net(models[32], 1, 64, 250, api.IMPL_LAYERED)
-    _fused_or_skip(net, api.IMPL_FUSED)
     net.set_impl(api.IMPL_FUSED)
     x = np.full((1, 64, 250), 77, np.uint8)
     net.load_data(x)
@@ -476,7 +454,6 @@ def test_tma_input_ring_is_bit_identical(models, monkeypatch, shape):
     x, _ = synth.make_frames(0xC0FFEE + 44, n, h, w)
     a = api.QVRCNN(0, n, 1, h, w)
     a.load_static_para_mem(image)
-    _fused_or_skip(a, api.IMPL_FUSED)
     a.set_impl(api.IMPL_FUSED)
     want = a.forward_frames_host(x)
     monkeypatch.setenv("QV_FUSED_TMA", "1")
@@ -523,7 +500,6 @@ def test_generic_requant_parameters(models, impl, case):
     m.qparams = [tuple(t) for t in q]
     anchor, _ = synth.make_frames(0xC0FFEE + 9, 2, 70, 131)
     net = _net(m, 2, 70, 131, api.IMPL_LAYERED)
-    _fused_or_skip(net, impl)
     net.set_impl(impl)
     net.load_data(anchor)
     net.forward_blu()
