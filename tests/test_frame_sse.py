@@ -101,13 +101,13 @@ def test_fused_sse_matches_numpy(models, qp, shape):
     assert np.array_equal(sse[:, 1], _np_sse(out, ori))
 
 
-def _units(n, h, w, line):
+def _units(sm, n, h, w, line):
     L = api.lib()
     L.qv_debug_fused_units.argtypes = [C.c_int] * 8 + [C.c_void_p, C.POINTER(C.c_size_t), C.POINTER(C.c_int)]
     cnt, grid = C.c_size_t(0), C.c_int(0)
-    assert L.qv_debug_fused_units(148, n, h, w, 0, h, 0, line, None, C.byref(cnt), C.byref(grid)) == 0
+    assert L.qv_debug_fused_units(sm, n, h, w, 0, h, 0, line, None, C.byref(cnt), C.byref(grid)) == 0
     u = np.zeros((cnt.value, 5), np.int32)
-    assert L.qv_debug_fused_units(148, n, h, w, 0, h, 0, line, u.ctypes.data, C.byref(cnt), C.byref(grid)) == 0
+    assert L.qv_debug_fused_units(sm, n, h, w, 0, h, 0, line, u.ctypes.data, C.byref(cnt), C.byref(grid)) == 0
     return u
 
 
@@ -115,11 +115,12 @@ def _units(n, h, w, line):
 def test_row_line_plan_across_frames_and_layered_cross_check(models):
     """A geometry dealt out by the row line (P.linear) in which one CTA's pieces belong to different frames: the per-frame
     flush must go to the right frame.  The layered path gives the same numbers; calls add up; asynchronous calls report
-    after a synchronize."""
+    after a synchronize.  The plan is read at the device's SM count, the one the launch is planned with."""
     import torch
     n, h, w = 26, 56, 250
-    u = _units(n, h, w, 1)
-    assert not np.array_equal(u, _units(n, h, w, 0)), "expected the row-line plan"
+    sm = torch.cuda.get_device_properties(0).multi_processor_count
+    u = _units(sm, n, h, w, 1)
+    assert not np.array_equal(u, _units(sm, n, h, w, 0)), "expected the row-line plan"
     assert any(len(set(u[u[:, 0] == c][:, 1])) > 1 for c in set(u[:, 0])), "expected a CTA that spans frames"
     anchor, ori = synth.make_frames(0xC0FFEE + 41, n, h, w)
     net = _net(models[27], 8, h, w)
